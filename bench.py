@@ -16,6 +16,7 @@ below half the per-sample model (predict, K1: V is half L2-resident) report thei
 
     python bench.py --gpus N --steps K --warmup W            # engine arm
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU implementation
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also save what the timed path computed, DIR/<name>.npy
 
 For N > 1 launch with torchrun (one rank per GPU); see DESIGN.md section "Multi-GPU".
 """
@@ -144,6 +145,26 @@ def parse_profile(txt):
     return agg
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def fixed_sample(n, m, seed):
+    """sorted indices of a seeded sample of m out of n (all n when m >= n): the same for every run with the same n"""
+    if m >= n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, m, replace=False))
+
+
+def write_outputs(path, arrays):
+    """--dump-outputs: each array as <path>/<name>.npy in float64, so two builds can be compared output for output"""
+    arrays = {name: np.asarray(a, np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, "outputs to dump take %d bytes, over the %d-byte limit" % (total, DUMP_LIMIT)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def dist_env():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -231,6 +252,14 @@ def run_engine(args):
     ms_train = ctx.timer_stop_ms()
     l1 = ctx.launches()
     train_sps = epoch * args.steps / (ms_train * 1e-3)
+    dump = {}
+    if args.dump_outputs:
+        # the model the last timed step returns (w0, w, V); w and V as fixed samples of their rows (16 MB of V at any k)
+        w0_t, w_t, v_t = model.get()
+        w_rows = fixed_sample(p, 1 << 20, 1)
+        v_rows = fixed_sample(p, (16 << 20) // (8 * max(k, 1)), 2)
+        dump.update(w0=np.array([w0_t]), w_sample=w_t[w_rows], w_sample_rows=w_rows, v_sample=v_t[v_rows], v_sample_rows=v_rows)
+        del v_t
     # timed region B: the same K steps with a CUDA-event pair around every kernel launch -> per-kernel durations for the roofline
     prof_train, ms_train_prof = profiled(L, lib, ctx, lambda: L.train_dev(ctx, model, data, sc), args.steps)
 
@@ -241,6 +270,11 @@ def run_engine(args):
     for _ in range(args.steps):
         L.predict_dev(ctx, model, data, L.LINK_LOGISTIC)
     ms_pred = ctx.timer_stop_ms()
+    if args.dump_outputs:
+        # predict.FM's probabilities from its last timed step, a fixed sample of the rows
+        pred_rows = fixed_sample(n, 1 << 20, 3)
+        dump.update(predict_sample=L.predict_fetch(ctx, data)[pred_rows], predict_sample_rows=pred_rows)
+        write_outputs(args.dump_outputs, dump)
     prof_pred, _ = profiled(L, lib, ctx, lambda: L.predict_dev(ctx, model, data, L.LINK_LOGISTIC), args.steps)
     clk = clocks.stop()
     pred_rps = n * args.steps / (ms_pred * 1e-3)
@@ -349,7 +383,7 @@ def run_other_solvers(L, lib, ctx, data, args, peak, n, F, p, k, B, info, kp):
     configs[3] (MovieLens-shaped 20M ratings, 3 one-hot fields).  Minibatch fractions are against the compulsory bytes of the
     epoch (forward + update, see k1_/k2_compulsory_bytes); SURVEY 8(d)'s per-sample model is given without a fraction."""
     out = {}
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
 
     def timed(fn):
         for _ in range(3):
@@ -554,7 +588,7 @@ def run_e2e(L, lib, ctx, data, mcfg, sc, n, p, k, args):
     val_bytes = val64.nbytes // 2 if host_narrow else val64.nbytes
     h2d = row_size.nbytes + col_i.nbytes + val_bytes + y64.nbytes + w.nbytes + v.nbytes + 8
     d2h = w.nbytes + v.nbytes + 8
-    steps = max(1, min(args.steps, args.e2e_steps))
+    steps = args.steps
 
     def one():
         L.check(lib.fmwr_train(C.byref(mcfg), C.byref(sc), C.c_int64(n), C.c_int64(p), C.c_int64(col_i.size), L.ptr(row_size),
@@ -1046,7 +1080,10 @@ def run_engine_multi(args, rank, world, local):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of the headline FTRL epoch and predict.FM, of the SGD / TDAP / ALS / MCMC lines and of e2e; the "
+                         "exact-mode (one run per solver), batch-sweep (two epochs per batch size) and configs[0] (2, 2, 5 and 3 runs) "
+                         "lines time fixed counts, and the secondary lines of a multi-GPU run at most 5")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="engine", choices=["engine", "reference"])
     ap.add_argument("--rows", type=int, default=10_000_000)
@@ -1063,10 +1100,16 @@ def main():
     ap.add_argument("--parity-rows", type=int, default=200_000)
     ap.add_argument("--c5-rows", type=int, default=100_000_000)
     ap.add_argument("--c5-features", type=int, default=50_000_000)
-    ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
     ap.add_argument("--ref-step-seconds", type=float, default=4.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the model after the last timed training step and the last timed predict.FM output (fixed samples of "
+                         "the large arrays) to DIR/<name>.npy; single-GPU engine runs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "engine" or dist_env()[1] > 1):
+        ap.error("--dump-outputs is for single-GPU engine runs")
     if args.warmup < 3 and args.impl == "engine":
         args.warmup = max(args.warmup, 3) if os.environ.get("FMWR_BENCH_STRICT", "1") == "1" else args.warmup
     if args.impl == "reference":
