@@ -263,7 +263,6 @@ bool model_alloc_state(fmwr_model* m, int n_state, int solver, bool warm)
 }
 
 fmwr_data* data_create_f64(fmwr_ctx*, int64_t, int64_t, int64_t, const int32_t*, const int32_t*, const double*, const double*, bool defer_values);
-void data_wait_values(fmwr_data* d);
 fmwr_data* data_create_csr32(fmwr_ctx*, int64_t, int64_t, int64_t, const uint32_t*, const uint32_t*, const float*, const float*);
 
 static void fetch_pred(fmwr_ctx* ctx, fmwr_data* d, double* out)
@@ -833,20 +832,18 @@ int fmwr_train(const fmwr_model_cfg* cfg, const fmwr_solver_cfg* s, int64_t n, i
     PhaseTimer pt;
     FMWR_REQUIRE(value || nnz == 0, FMWR_ERR_ARG, "null argument");
     // minibatch path: the f64 values (60 % of the bytes) keep uploading on the copy stream while the compute stream
-    // builds the per-batch CSC keys; every reader of the values waits for the upload's event
-    const bool mb = s->mode == FMWR_MODE_MINIBATCH && s->solver >= FMWR_SGD && s->solver <= FMWR_TDAP;
+    // builds the per-batch CSC keys; each batch waits for its own chunks
+    const bool stream = minibatch_streams_values(s);
     // the model goes up first: once the value chunks are queued on the copy engine nothing else gets through until they are done
     if (fmwr_model_create(ctx, cfg, p, s->precision, &mg.m)) throw Error(FMWR_ERR_ARG, g_last_error);
     model_set_host(mg.m, *w0, w, v);
     pt.lap("model create + set");
-    // (not with the tracker: its mid-epoch scoring pass reads every row's values)
-    dg.d = data_create_f64(ctx, n, p, nnz, row_size, col_idx, value, labels, mb && !pt.on && s->step_size <= 0);
+    dg.d = data_create_f64(ctx, n, p, nnz, row_size, col_idx, value, labels, stream && !pt.on);
     pt.lap("data_create (H2D + narrow)");
-    if (mb) {
+    if (stream) {
       minibatch_build(dg.d, (s->compat & FMWR_COMPAT_SKIP_ROW0) ? 1 : 0, s->batch_size);
       pt.lap("per-batch CSC build");
     }
-    if (!dg.d->mb_vals_pending) data_wait_values(dg.d);
     train_dispatch(ctx, mg.m, dg.d, s, trace);
     pt.lap("train");
     model_get_host(mg.m, w0, w, v);
@@ -930,7 +927,7 @@ int fmwr_data_minibatch_info(fmwr_data* d, int32_t batch_size, int32_t compat, i
     const int64_t nb = (int64_t)d->mb_batch_seg.size() - 1;
     if (n_batches) *n_batches = nb;
     if (n_segments) *n_segments = nb >= 0 ? d->mb_batch_seg[nb] : 0;
-    if (n_entries) *n_entries = d->mb_batch_ent.empty() ? 0 : d->mb_batch_ent.back();
+    if (n_entries) *n_entries = minibatch_entries(d);
   });
 }
 

@@ -171,31 +171,30 @@ struct fmwr_data {
   fmwr::DBuf<uint32_t> mb_ent_row;   // [nnz'] global row index
   fmwr::DBuf<float> mb_ent_val;      // [nnz']
   std::vector<int64_t> mb_batch_seg;  // [n_batches+1] segment offsets per batch (host)
-  // one-shot training path: the value stream may still be uploading on the copy stream while the compute stream already
-  // sorts the (batch, feature) keys; val_ready marks its end (data.cu: data_wait_values)
+  // The upload (data.cu).  A background thread converts the caller's f64 values chunk by chunk (val_chunk entries) into the
+  // context's pinned staging ring and uploads them as f32 -- half the PCIe bytes of the value stream; up_issued = chunks whose copy
+  // and event have been queued (an event must be recorded before anybody waits on it), val_ev[c] = chunk c has arrived, val_ready =
+  // all of them.  From a page-locked caller buffer every third chunk goes up raw into val64 instead (val_dev[c]) and is narrowed on
+  // the device by its first reader.  data_create_f64 waits for all of it unless the values are deferred, and deferred values go only
+  // to the minibatch trainer (minibatch_streams_values), which makes each batch's values ready through minibatch_batch_values.
   cudaEvent_t val_ready = nullptr;
-  std::vector<cudaEvent_t> val_ev;     // one per uploaded chunk of val_chunk entries (deferred upload only)
-  std::vector<char> val_dev;           // chunk c crossed PCIe as raw f64 into val64 and is narrowed on the device (mixed upload, data.cu)
-  int64_t val_waited = 0;              // chunks whose events the compute stream already waits for (train_minibatch.cu)
-  // one-shot training path: the column ids cross PCIe in chunks on the copy stream too (col_ev[c] = chunk c of col_chunk entries
-  // has arrived), so the per-batch CSC of the first row groups is built while the later ones are still uploading
-  // (data.cu: minibatch_build_grouped); everything else waits for all of them first (data_wait_cols)
-  std::vector<cudaEvent_t> col_ev;
-  int64_t col_chunk = 0;
-  bool cols_pending = false;           // uploads queued, CSR not validated yet
+  std::vector<cudaEvent_t> val_ev;
+  std::vector<char> val_dev;
+  int64_t val_waited = 0;              // chunks whose events the compute stream already waits for (per-batch value fill)
   int64_t val_chunk = 0;
-  fmwr::DBuf<double> val_stage[2];
-  fmwr::DBuf<double> val64;            // deferred upload: the raw f64 values; narrowed into `val` range by range on the compute stream
+  fmwr::DBuf<double> val64;
   bool val_all_narrowed = true;
-  // host-side narrowing (default): a background thread converts the caller's f64 values chunk by chunk into the context's pinned
-  // staging ring and uploads them as f32 -- half the PCIe bytes of the value stream; up_issued = chunks whose copy and event have
-  // been queued (an event must be recorded before anybody waits on it)
   std::thread up_thread;
   std::atomic<int64_t> up_issued{0};
   int64_t up_chunks = 0;
-  bool upload_in_flight() const { return up_chunks > 0 && up_issued.load(std::memory_order_acquire) <= up_chunks; }
+  // one-shot training path (values deferred): the column ids cross PCIe in chunks on the copy stream too (col_ev[c] = chunk c of
+  // col_chunk entries has arrived), so the per-batch CSC of the first row groups is built while the later ones are still uploading
+  // (data.cu: minibatch_build); everything else waits for all of them first (data_wait_cols)
+  std::vector<cudaEvent_t> col_ev;
+  int64_t col_chunk = 0;
+  bool cols_pending = false;           // uploads queued, CSR not validated yet
   // per-batch CSC built while the values were still in flight: ent_val / seg_rec.w of batch b are filled right before
-  // batch b trains, as soon as the value chunks covering its rows have arrived (train_minibatch.cu)
+  // batch b trains, as soon as the value chunks covering its rows have arrived (data.cu: minibatch_batch_values)
   bool mb_vals_pending = false;
   fmwr::DBuf<uint32_t> mb_perm;        // sorted position -> original entry (relative to mb_e0)
   uint32_t mb_e0 = 0;
@@ -431,6 +430,10 @@ void sort_pairs_u32(fmwr_ctx* ctx, const uint32_t* key_in, uint32_t* key_out, co
 void sort_pairs_u64(fmwr_ctx* ctx, const uint64_t* key_in, uint64_t* key_out, const uint32_t* val_in, uint32_t* val_out, int64_t n, int bits);
 void phases_build(fmwr_data* d);
 void minibatch_build(fmwr_data* d, int64_t row0, int64_t batch);
+void minibatch_batch_values(fmwr_data* d, int64_t b);   // batch b's values ready on the compute stream (per-batch CSC built while they upload)
+void minibatch_all_values(fmwr_data* d);                // every value ready (a first epoch that stopped early)
+int64_t minibatch_entries(const fmwr_data* d);          // entries of the per-batch CSC
+bool minibatch_streams_values(const fmwr_solver_cfg* s);   // train_minibatch may start on data whose values are still uploading
 void train_exact(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr);
 void train_minibatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr);
 void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr);
@@ -448,7 +451,6 @@ void data_synth(fmwr_ctx* ctx, int64_t n, int64_t row_begin, int32_t n_fields, c
                 int32_t value_mode, int32_t label_mode, double noise, uint64_t seed, fmwr_data** out);
 void model_init_random(fmwr_model* m, double mean, double sd, uint64_t seed);
 fmwr_data* data_slice_columns(fmwr_data* src, int64_t c0, int64_t c1);
-void data_wait_cols(fmwr_data* d);        // one-shot path: every column chunk uploaded and the CSR validated (data.cu)
 fmwr_data* data_concat_rows(fmwr_data* const* parts, int n_parts);
 fmwr_data* data_gather_rows(fmwr_data* src, const uint32_t* order_dev, int64_t m);
 std::vector<uint32_t> visit_order_host(const fmwr_data* d, const fmwr_solver_cfg* s);

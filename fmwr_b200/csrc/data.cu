@@ -13,8 +13,6 @@
 
 namespace fmwr {
 
-void data_wait_values(fmwr_data* d);
-
 // ------------------------------------------------------------------------------------------ scan
 // exclusive prefix sum of u32 (reduce-then-scan, 3 phases, recursive on the block sums)
 constexpr int SCAN_THREADS = 256;
@@ -186,17 +184,11 @@ static void set_labels_f64(fmwr_data* d, const double* labels)
   d->min_y = mn; d->max_y = mx;
 }
 
-// the compute stream waits for a deferred value upload (no-op otherwise)
-void data_narrow_values(fmwr_data* d, int64_t lo, int64_t hi)
+// entries [lo, hi) of `val` on the compute stream: only the chunks of a mixed upload that came up as raw f64 have anything to
+// narrow (the caller has made the stream wait for their events)
+static void data_narrow_values(fmwr_data* d, int64_t lo, int64_t hi)
 {
   if (!d->val64.p || hi <= lo) return;
-  if (d->val_dev.empty()) {
-    f64_to_f32<<<ceil_div(hi - lo, 256), 256, 0, d->ctx->stream>>>(d->val64.p + lo, d->val.p + lo, hi - lo);
-    d->ctx->launches++;
-    FMWR_CUDA(cudaGetLastError());
-    return;
-  }
-  // mixed upload: only the chunks that came up as raw f64 have anything to narrow
   for (int64_t c = lo / d->val_chunk; c * d->val_chunk < hi && c < (int64_t)d->val_dev.size(); ++c) {
     if (!d->val_dev[c]) continue;
     const int64_t a = std::max(lo, c * d->val_chunk), b = std::min(hi, std::min(d->nnz, (c + 1) * d->val_chunk));
@@ -208,13 +200,13 @@ void data_narrow_values(fmwr_data* d, int64_t lo, int64_t hi)
 }
 
 // host wait until the uploader has QUEUED chunk ci (its copy and its event): only then may a stream wait on the event
-void data_wait_chunk_issued(fmwr_data* d, int64_t ci)
+static void data_wait_chunk_issued(fmwr_data* d, int64_t ci)
 {
   while (d->up_chunks > 0 && d->up_issued.load(std::memory_order_acquire) <= ci) std::this_thread::yield();
 }
 
-// every column chunk in, CSR validated: what any reader of `col` other than the grouped build calls first
-void data_wait_cols(fmwr_data* d)
+// every column chunk in, CSR validated: what any reader of `col` other than the per-batch CSC build calls first
+static void data_wait_cols(fmwr_data* d)
 {
   if (!d->cols_pending) return;
   for (cudaEvent_t e : d->col_ev) FMWR_CUDA(cudaStreamWaitEvent(d->ctx->stream, e, 0));
@@ -222,7 +214,8 @@ void data_wait_cols(fmwr_data* d)
   finish_create(d);
 }
 
-void data_wait_values(fmwr_data* d)
+// every value in `val` for the compute stream: what any reader of `val` other than the per-batch value fill calls first
+static void data_wait_values(fmwr_data* d)
 {
   if (d->up_thread.joinable()) d->up_thread.join();
   if (d->val_ready) FMWR_CUDA(cudaStreamWaitEvent(d->ctx->stream, d->val_ready, 0));
@@ -264,10 +257,7 @@ static void start_value_upload(fmwr_data* d, const double* value, int64_t chunk)
   d->val_chunk = chunk;
   d->up_chunks = n_chunks;
   d->up_issued.store(0, std::memory_order_release);
-  static const int n_workers = [] {
-    int t = getenv("FMWR_HOST_THREADS") ? atoi(getenv("FMWR_HOST_THREADS")) : (int)std::thread::hardware_concurrency();
-    return std::max(1, std::min(t, 32));
-  }();
+  static const int n_workers = std::max(1, std::min((int)std::thread::hardware_concurrency(), 32));
   const int dev = ctx->device;
   cudaStream_t vs = ctx->copy_stream;
   float* stage[2] = {ctx->h_stage[0].p, ctx->h_stage[1].p};
@@ -277,23 +267,21 @@ static void start_value_upload(fmwr_data* d, const double* value, int64_t chunk)
   // while the host narrows the two chunks before it: PCIe carries 2 x 4 + 8 bytes per three values in the time the host
   // narrows two -- both ~4.7 ms per three 16M-value chunks.  Raw chunks are narrowed on the device by their first reader
   // (data_narrow_values).  Only when the caller's buffer is pinned: a pageable source would be staged by the driver.
-  static const bool mix_env = !(getenv("FMWR_MIX_UPLOAD") && atoi(getenv("FMWR_MIX_UPLOAD")) == 0);
-  static const int period = std::max(2, std::min(8, getenv("FMWR_MIX_PERIOD") ? atoi(getenv("FMWR_MIX_PERIOD")) : 3));     // one raw chunk per `period`
+  constexpr int P = 3;                       // one raw chunk per P
   bool mix = false;
-  if (mix_env && n_chunks >= 3) {
+  if (n_chunks >= P) {
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, value) == cudaSuccess && at.type == cudaMemoryTypeHost) mix = true;
     cudaGetLastError();
   }
   d->val_dev.assign(n_chunks, 0);
   if (mix) {
-    for (int64_t c = period - 1; c < n_chunks; c += period) d->val_dev[c] = 1;
+    for (int64_t c = P - 1; c < n_chunks; c += P) d->val_dev[c] = 1;
     d->val64.alloc(nnz);
     d->val_all_narrowed = false;
   }
   d->val_waited = 0;
-  const int P = period;
-  d->up_thread = std::thread([d, value, chunk, nnz, n_chunks, dev, vs, stage, P] {
+  d->up_thread = std::thread([d, value, chunk, nnz, n_chunks, dev, vs, stage] {
     cudaSetDevice(dev);
     int64_t last_use[2] = {-1, -1};            // the chunk whose copy last read each staging buffer
     int hcount = 0;
@@ -366,93 +354,42 @@ fmwr_data* data_create_f64(fmwr_ctx* ctx, int64_t n, int64_t p, int64_t nnz, con
       FMWR_CUDA(cudaMemcpy(&total, d->rowptr.p + n, sizeof(uint32_t), cudaMemcpyDeviceToHost));
       FMWR_REQUIRE((int64_t)total == nnz, FMWR_ERR_SHAPE, "the length of input's row_size is not correct...");
     }
-    static const bool host_narrow0 = !(getenv("FMWR_HOST_NARROW") && atoi(getenv("FMWR_HOST_NARROW")) == 0);
-    static const bool col_chunks = !(getenv("FMWR_COL_CHUNKS") && atoi(getenv("FMWR_COL_CHUNKS")) == 0);
-    const bool stream_cols = nnz > 0 && defer_values && host_narrow0 && col_chunks;
-    bool labels_done = false;
-    if (stream_cols && labels) {
-      // the labels first: a copy queued behind the column chunks would sit on the copy engine (and the host in its sync) until
-      // all of them are through
-      set_labels_f64(d, labels);
-      labels_done = true;
-    }
-    if (stream_cols) {
-      // one-shot training: the column ids go up in chunks on the copy stream, one event each, and nobody waits here -- the
-      // per-batch CSC of a row group is built as soon as its chunks are in (minibatch_build_grouped)
-      const int64_t cchunk_env = getenv("FMWR_VAL_CHUNK") ? atoll(getenv("FMWR_VAL_CHUNK")) : 0;      // read per call: tests shrink it
-      const int64_t cchunk = cchunk_env > 0 ? cchunk_env : (16ll << 20);
-      for (int64_t off = 0; off < nnz; off += cchunk) {
-        const int64_t mm = std::min(cchunk, nnz - off);
-        FMWR_CUDA(cudaMemcpyAsync(d->col.p + off, col_idx + off, sizeof(int32_t) * mm, cudaMemcpyHostToDevice, ctx->copy_stream));
-        cudaEvent_t ce = nullptr;
-        FMWR_CUDA(cudaEventCreateWithFlags(&ce, cudaEventDisableTiming));
-        FMWR_CUDA(cudaEventRecord(ce, ctx->copy_stream));
-        d->col_ev.push_back(ce);
-      }
-      d->col_chunk = cchunk;
-      d->cols_pending = true;
-    }
+    // the labels first: a copy queued behind the column chunks would sit on the copy engine (and the host in its sync) until
+    // all of them are through
+    if (labels) set_labels_f64(d, labels);
     if (nnz > 0) {
-      if (!stream_cols) FMWR_CUDA(cudaMemcpyAsync(d->col.p, col_idx, sizeof(int32_t) * nnz, cudaMemcpyHostToDevice, ctx->stream));
-      // f64 -> f32 narrowing on the device, chunked through two staging buffers.  defer_values: the chunks travel on the
-      // copy stream and nobody waits here -- the one-shot training path sorts the (batch, feature) keys (which need only
-      // rowptr and col) while the 8-byte values are still crossing PCIe, and waits for val_ready before it reads them.
-      const int64_t chunk_env = getenv("FMWR_VAL_CHUNK") ? atoll(getenv("FMWR_VAL_CHUNK")) : 0;
+      const int64_t chunk_env = getenv("FMWR_VAL_CHUNK") ? atoll(getenv("FMWR_VAL_CHUNK")) : 0;      // read per call: tests shrink it
       const int64_t chunk = chunk_env > 0 ? chunk_env : (16ll << 20);
-      static const bool host_narrow = !(getenv("FMWR_HOST_NARROW") && atoi(getenv("FMWR_HOST_NARROW")) == 0);
-      if (host_narrow) {
-        FMWR_CUDA(cudaEventRecord(ctx->ev_copy[0], ctx->stream));        // the column ids go first: the key sort needs all of them
-        FMWR_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy[0], 0));
-        start_value_upload(d, value, chunk);
-        if (!defer_values) { data_wait_values(d); FMWR_CUDA(cudaStreamSynchronize(ctx->stream)); }
-      } else if (defer_values) {
-        // the copy stream carries nothing but copies (a narrowing kernel between two chunks would stall the upload whenever it
-        // has to wait for SM slots behind the compute stream's sort): raw f64 into a full-size staging buffer, one event per chunk;
-        // the compute stream narrows exactly the range a batch needs once that batch's chunk has arrived
-        cudaStream_t vs = ctx->copy_stream;
-        FMWR_CUDA(cudaEventRecord(ctx->ev_copy[0], ctx->stream));        // the column ids go first: the key sort needs all of them
-        FMWR_CUDA(cudaStreamWaitEvent(vs, ctx->ev_copy[0], 0));
-        d->val64.alloc(nnz);
+      if (defer_values) {
+        // one-shot training: the column ids go up in chunks on the copy stream, one event each, and nobody waits here -- the
+        // per-batch CSC of a row group is built as soon as its chunks are in (minibatch_build)
         for (int64_t off = 0; off < nnz; off += chunk) {
-          const int64_t m = std::min(chunk, nnz - off);
-          FMWR_CUDA(cudaMemcpyAsync(d->val64.p + off, value + off, sizeof(double) * m, cudaMemcpyHostToDevice, vs));
+          const int64_t mm = std::min(chunk, nnz - off);
+          FMWR_CUDA(cudaMemcpyAsync(d->col.p + off, col_idx + off, sizeof(int32_t) * mm, cudaMemcpyHostToDevice, ctx->copy_stream));
           cudaEvent_t ce = nullptr;
           FMWR_CUDA(cudaEventCreateWithFlags(&ce, cudaEventDisableTiming));
-          FMWR_CUDA(cudaEventRecord(ce, vs));
-          d->val_ev.push_back(ce);
+          FMWR_CUDA(cudaEventRecord(ce, ctx->copy_stream));
+          d->col_ev.push_back(ce);
         }
-        d->val_chunk = chunk;
-        d->val_all_narrowed = false;
-        FMWR_CUDA(cudaEventCreateWithFlags(&d->val_ready, cudaEventDisableTiming));
-        FMWR_CUDA(cudaEventRecord(d->val_ready, vs));
+        d->col_chunk = chunk;
+        d->cols_pending = true;
       } else {
-        d->val_stage[0].alloc(std::min(chunk, nnz));
-        d->val_stage[1].alloc(nnz > chunk ? std::min(chunk, nnz - chunk) : 1);
-        cudaEvent_t free_ev[2] = {nullptr, nullptr};
-        int ci = 0;
-        for (int64_t off = 0; off < nnz; off += chunk, ci ^= 1) {
-          const int64_t m = std::min(chunk, nnz - off);
-          if (free_ev[ci]) FMWR_CUDA(cudaStreamWaitEvent(ctx->stream, free_ev[ci], 0));
-          FMWR_CUDA(cudaMemcpyAsync(d->val_stage[ci].p, value + off, sizeof(double) * m, cudaMemcpyHostToDevice, ctx->stream));
-          f64_to_f32<<<ceil_div(m, 256), 256, 0, ctx->stream>>>(d->val_stage[ci].p, d->val.p + off, m);
-          ctx->launches++;
-          FMWR_CUDA(cudaGetLastError());
-          if (!free_ev[ci]) FMWR_CUDA(cudaEventCreateWithFlags(&free_ev[ci], cudaEventDisableTiming));
-          FMWR_CUDA(cudaEventRecord(free_ev[ci], ctx->stream));
-        }
-        for (int i = 0; i < 2; ++i) if (free_ev[i]) cudaEventDestroy(free_ev[i]);
-        FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
-        d->val_stage[0].release(); d->val_stage[1].release();
+        FMWR_CUDA(cudaMemcpyAsync(d->col.p, col_idx, sizeof(int32_t) * nnz, cudaMemcpyHostToDevice, ctx->stream));
       }
+      // defer_values: nobody waits for the values here -- the one-shot training path sorts the (batch, feature) keys (which need
+      // only rowptr and col) while the values are still crossing PCIe, and each batch waits for its own chunks before it reads them
+      FMWR_CUDA(cudaEventRecord(ctx->ev_copy[0], ctx->stream));        // the column ids go first: the key sort needs all of them
+      FMWR_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_copy[0], 0));
+      start_value_upload(d, value, chunk);
+      if (!defer_values) { data_wait_values(d); FMWR_CUDA(cudaStreamSynchronize(ctx->stream)); }
     }
-    if (labels && !labels_done) set_labels_f64(d, labels);
     {
-      int64_t vbytes = (d->up_chunks > 0 ? 4 : 8) * nnz;                  // values cross as f32 when narrowed on the host
+      int64_t vbytes = 4 * nnz;                                            // values cross as f32, narrowed on the host ...
       for (size_t c = 0; c < d->val_dev.size(); ++c)                       // ... except the chunks of a mixed upload that go up raw
         if (d->val_dev[c]) vbytes += 4 * std::min<int64_t>(d->val_chunk, nnz - (int64_t)c * d->val_chunk);
       ctx->h2d_bytes += 4 * n + 4 * nnz + vbytes + (labels ? 8 * n : 0);
     }
-    if (!d->cols_pending) finish_create(d);            // (chunked columns: validated group by group, or by data_wait_cols)
+    if (!d->cols_pending) finish_create(d);            // (chunked columns: validated by the per-batch CSC build, or by data_wait_cols)
   } catch (...) { delete d; throw; }
   return d;
 }
@@ -598,17 +535,22 @@ void phases_build(fmwr_data* d)
 }
 
 // ------------------------------------------------------------------------------------------ per-batch CSC
+// Entries of rows [row0, n) regrouped by (batch, feature, row): the "sorted-key segmented reduction" layout of the minibatch update
+// kernels (one segment = one touched coordinate).  It is built ROW GROUP BY ROW GROUP: a group is a run of whole batches whose
+// entries are sorted on (batch inside the group, feature) and emitted into the global arrays at the group's entry / segment
+// offsets.  Resident data is one group.  While the column ids are still uploading (one-shot training path) a group holds ~32M
+// entries and is built as soon as its column chunks are in -- fewer key bits, one radix pass less than the whole-matrix sort.
 template <class K>
-__global__ void mb_keys(const uint32_t* __restrict__ rowptr, const uint32_t* __restrict__ col, int64_t row0, int64_t n,
-                        uint32_t batch, int colbits, K* __restrict__ keys, uint32_t* __restrict__ erow)
+__global__ void mbg_keys(const uint32_t* __restrict__ rowptr, const uint32_t* __restrict__ col, int64_t r0, int64_t r1, int64_t row0,
+                         uint32_t batch, uint32_t b0, int colbits, uint32_t eg0, K* __restrict__ keys, uint32_t* __restrict__ erow)
 {
-  const int64_t row = row0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-  if (row >= n) return;
-  const uint32_t b = rowptr[row], e = rowptr[row + 1], e0 = rowptr[row0];
-  const uint64_t bid = (uint64_t)((row - row0) / batch);
+  const int64_t row = r0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+  if (row >= r1) return;
+  const uint32_t b = rowptr[row], e = rowptr[row + 1];
+  const uint64_t bid = (uint64_t)((row - row0) / batch) - b0;
   for (uint32_t j = b + (threadIdx.x & 31); j < e; j += 32) {
-    keys[j - e0] = (K)((bid << colbits) | (uint64_t)col[j]);
-    erow[j - e0] = (uint32_t)row;
+    keys[j - eg0] = (K)((bid << colbits) | (uint64_t)col[j]);
+    erow[j - eg0] = (uint32_t)row;
   }
 }
 
@@ -621,27 +563,34 @@ __global__ void mb_heads(const K* __restrict__ keys, int64_t m, uint32_t* __rest
   head[i] = (i == 0 || keys[i] != keys[i - 1]) ? 1u : 0u;
 }
 
+// val: the group's values go into ent_val and the segment records.  val == nullptr (values still uploading): the permutation goes
+// into perm_global instead, for mb_fill_values to write the values batch by batch once they have arrived.
 template <class K>
-__global__ void mb_emit(const K* __restrict__ keys, const uint32_t* __restrict__ head, const uint32_t* __restrict__ segid,
-                        const uint32_t* __restrict__ perm, const uint32_t* __restrict__ erow, const float* __restrict__ val,
-                        uint32_t e0, int64_t m, int colbits, uint32_t* __restrict__ seg_ptr, uint4* __restrict__ seg_rec,
-                        uint32_t* __restrict__ ent_row, float* __restrict__ ent_val, uint32_t n_seg)
+__global__ void mbg_emit(const K* __restrict__ keys, const uint32_t* __restrict__ head, const uint32_t* __restrict__ segid,
+                         const uint32_t* __restrict__ perm_local, const uint32_t* __restrict__ erow, const float* __restrict__ val,
+                         int64_t mg, int colbits, uint32_t eg0, uint32_t eoff, uint32_t seg_base, uint32_t n_seg_g,
+                         uint32_t* __restrict__ seg_ptr, uint4* __restrict__ seg_rec, uint32_t* __restrict__ ent_row,
+                         float* __restrict__ ent_val, uint32_t* __restrict__ perm_global)
 {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= m) return;
-  const uint32_t e = perm[i];
+  if (i >= mg) return;
+  // every load before the first store: a segment head's loads then share the entry's round trip
+  const uint32_t e = perm_local[i];
+  const bool h = head[i] != 0;
   const uint32_t r = erow[e];
-  const float x = val ? val[e0 + e] : 0.f;           // deferred upload: filled per batch by mb_fill_values
-  ent_row[i] = r;
-  ent_val[i] = x;
-  if (head[i]) {
+  const float x = val ? val[eg0 + e] : 0.f;
+  const uint32_t s = h ? seg_base + segid[i] : 0u;
+  const uint32_t c = h ? (uint32_t)((uint64_t)keys[i] & ((1ull << colbits) - 1ull)) : 0u;
+  ent_row[eoff + i] = r;
+  if (val) ent_val[eoff + i] = x;
+  else perm_global[eoff + i] = e + eoff;             // relative to the first entry of the whole structure
+  if (h) {
     // segment record: {feature, length (filled by mb_seg_len), first row, first value} -- one 16-byte load gives
     // the update kernel everything it needs for the common single-entry segment
-    const uint32_t s = segid[i];
-    seg_ptr[s] = (uint32_t)i;
-    seg_rec[s] = make_uint4((uint32_t)((uint64_t)keys[i] & ((1ull << colbits) - 1ull)), 0u, r, __float_as_uint(x));
+    seg_ptr[s] = eoff + (uint32_t)i;
+    seg_rec[s] = make_uint4(c, 0u, r, __float_as_uint(x));
   }
-  if (i == m - 1) seg_ptr[n_seg] = (uint32_t)m;
+  if (i == mg - 1) seg_ptr[seg_base + n_seg_g] = eoff + (uint32_t)mg;
 }
 
 // values of the segments [seg_lo, seg_hi) (one batch) once their upload has arrived: ent_val and the record's first value
@@ -669,12 +618,6 @@ __global__ void peek2_u32(const uint32_t* __restrict__ a, const uint32_t* __rest
   if (threadIdx.x == 0 && blockIdx.x == 0) { host_dst[0] = *a; host_dst[1] = *b; }
 }
 
-__global__ void fill_u32(uint32_t* __restrict__ a, int64_t n, uint32_t v)
-{
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) a[i] = v;
-}
-
 // out[b] = rowptr[min(row0 + b * batch, n)]: the first entry of batch b
 __global__ void batch_row_ptr(const uint32_t* __restrict__ rowptr, int64_t row0, int64_t batch, int64_t n, int64_t count, uint32_t* __restrict__ out)
 {
@@ -684,165 +627,14 @@ __global__ void batch_row_ptr(const uint32_t* __restrict__ rowptr, int64_t row0,
   out[b] = rowptr[r < n ? r : n];
 }
 
-void minibatch_fill_values(fmwr_data* d, uint32_t seg_lo, uint32_t seg_hi)
-{
-  if (seg_hi <= seg_lo) return;
-  FMWR_LAUNCH(d->ctx, mb_fill_values, ceil_div((int64_t)seg_hi - seg_lo, 256), 256, 0, d->mb_seg_ptr.p, d->mb_seg_rec.p, d->mb_perm.p, d->val.p,
-              d->mb_e0, seg_lo, seg_hi, d->mb_ent_val.p);
-}
-
 __global__ void mb_seg_len(const uint32_t* __restrict__ seg_ptr, uint4* __restrict__ seg_rec, uint32_t n_seg)
 {
   const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
   if (s < n_seg) seg_rec[s].y = seg_ptr[s + 1] - seg_ptr[s];
 }
 
-// first segment of each batch: batch_seg[b] = #segments with batch id < b
-template <class K>
-__global__ void mb_batch_bounds(const K* __restrict__ keys, const uint32_t* __restrict__ head,
-                                const uint32_t* __restrict__ segid, int64_t m, int colbits, int64_t n_batches,
-                                uint32_t n_seg, uint32_t* __restrict__ batch_seg)
-{
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= m) return;
-  if (!head[i]) return;
-  const uint64_t bid = (uint64_t)keys[i] >> colbits;
-  const uint64_t pb = (i == 0) ? (uint64_t)-1 : ((uint64_t)keys[i - 1] >> colbits);
-  if (i == 0 || pb != bid) {
-    // batches (pb, bid] start at this segment (empty batches in between share the offset)
-    const uint64_t from = (i == 0) ? 0 : pb + 1;
-    for (uint64_t b = from; b <= bid; ++b) batch_seg[b] = segid[i];
-  }
-  (void)n_batches; (void)n_seg;
-}
-
-// batch_seg[b] = segment of the first sorted entry of batch b (n_seg past the end; an empty batch shares the next one's)
-__global__ void mb_batch_first_seg(const uint32_t* __restrict__ batch_ent, uint32_t e0, const uint32_t* __restrict__ segid, uint32_t m, uint32_t n_seg,
-                                   int64_t count, uint32_t* __restrict__ batch_seg)
-{
-  const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (b >= count) return;
-  const uint32_t i = batch_ent[b] - e0;
-  batch_seg[b] = i < m ? segid[i] : n_seg;
-}
-
-// Entries of rows [row0, n) regrouped by (batch, feature, row): the "sorted-key segmented
-// reduction" layout of the minibatch update kernels (one segment = one touched coordinate).
-template <class K>
-static void minibatch_build_t(fmwr_data* d, int64_t row0, int64_t batch)
-{
-  fmwr_ctx* ctx = d->ctx;
-  FMWR_REQUIRE(batch > 0, FMWR_ERR_ARG, "batch_size must be positive");
-  const int64_t rows = d->n - row0;
-  const int64_t n_batches = rows > 0 ? ceil_div64(rows, batch) : 0;
-  d->mb_batch_seg.assign(n_batches + 1, 0);
-  if (rows <= 0) { d->mb_batch = batch; d->mb_row0 = row0; return; }
-  // small device -> host reads are zero-copy stores of a kernel into pinned memory: a cudaMemcpy of 4 bytes would queue behind
-  // the upload chunks on the copy engine (measured: the build then ends when the upload ends)
-  ctx->h_u32.ensure(2 * (size_t)n_batches + 32);
-  uint32_t* hp = ctx->h_u32.p;
-  FMWR_LAUNCH(ctx, peek2_u32, 1, 32, 0, d->rowptr.p + row0, d->rowptr.p + d->n, hp);
-  FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
-  const uint32_t e0 = hp[0], e1 = hp[1];
-  DBuf<uint32_t> bp;
-  {
-    // entries before each batch (rows of a batch are consecutive, so this is also the batch's offset in the sorted arrays);
-    // used by the deferred-value path of the one-shot trainer
-    bp.alloc(n_batches + 1);
-    FMWR_LAUNCH(ctx, batch_row_ptr, ceil_div(n_batches + 1, 256), 256, 0, d->rowptr.p, row0, batch, d->n, n_batches + 1, bp.p);
-    FMWR_LAUNCH(ctx, peek_u32, ceil_div(n_batches + 1, 256), 256, 0, bp.p, n_batches + 1, hp + 8);
-    FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
-    d->mb_batch_ent.resize(n_batches + 1);
-    for (int64_t b = 0; b <= n_batches; ++b) d->mb_batch_ent[b] = (int64_t)hp[8 + b] - (int64_t)e0;
-  }
-  const int64_t m = (int64_t)e1 - e0;
-  const int colbits = bits_for((uint64_t)(d->p > 0 ? d->p - 1 : 0));
-  const int batchbits = bits_for((uint64_t)(n_batches > 0 ? n_batches - 1 : 0));
-  d->mb_ent_row.alloc(m + 8); d->mb_ent_val.alloc(m + 8);      // +8: the dense update kernel stages 16-byte-rounded ranges (update_tma.cuh)
-  if (m == 0) {
-    d->mb_seg_ptr.alloc(1); d->mb_seg_rec.alloc(1);
-    FMWR_CUDA(cudaMemsetAsync(d->mb_seg_ptr.p, 0, 4, ctx->stream));
-    d->mb_batch = batch; d->mb_row0 = row0;
-    return;
-  }
-  DBuf<K> keys_in, keys_out;
-  DBuf<uint32_t> erow, idx_out, head, segid;
-  // values still uploading (one-shot training path): build the structure from rowptr / col alone and keep the permutation
-  const bool deferred = d->val_ready != nullptr && !d->val_ev.empty() &&
-                        (d->up_chunks > 0 ? d->upload_in_flight() || cudaEventQuery(d->val_ready) != cudaSuccess : cudaEventQuery(d->val_ready) != cudaSuccess);
-  keys_in.alloc(m); keys_out.alloc(m); erow.alloc(m); head.alloc(m); segid.alloc(m);
-  if (deferred) d->mb_perm.alloc(m); else idx_out.alloc(m);
-  uint32_t* perm_p = deferred ? d->mb_perm.p : idx_out.p;
-  FMWR_LAUNCH(ctx, mb_keys<K>, ceil_div(rows * 32, 256), 256, 0, d->rowptr.p, d->col.p, row0, d->n, (uint32_t)batch, colbits,
-              keys_in.p, erow.p);
-  if (sizeof(K) == 4) sort_pairs_u32(ctx, (const uint32_t*)keys_in.p, (uint32_t*)keys_out.p, nullptr, perm_p, m, colbits + batchbits);
-  else sort_pairs_u64(ctx, (const uint64_t*)keys_in.p, (uint64_t*)keys_out.p, nullptr, perm_p, m, colbits + batchbits);
-  FMWR_LAUNCH(ctx, mb_heads<K>, ceil_div(m, 256), 256, 0, keys_out.p, m, head.p);
-  exclusive_scan_u32(ctx, head.p, segid.p, m);
-  FMWR_LAUNCH(ctx, peek2_u32, 1, 32, 0, segid.p + (m - 1), head.p + (m - 1), hp);
-  FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
-  const uint32_t n_seg = hp[0] + hp[1];
-  d->mb_seg_ptr.alloc((size_t)n_seg + 1 + 8); d->mb_seg_rec.alloc(n_seg);
-  if (!deferred) data_wait_values(d);
-  FMWR_LAUNCH(ctx, mb_emit<K>, ceil_div(m, 256), 256, 0, keys_out.p, head.p, segid.p, perm_p, erow.p, deferred ? (const float*)nullptr : d->val.p, e0, m,
-              colbits, d->mb_seg_ptr.p, d->mb_seg_rec.p, d->mb_ent_row.p, d->mb_ent_val.p, n_seg);
-  FMWR_LAUNCH(ctx, mb_seg_len, ceil_div(n_seg, 256), 256, 0, d->mb_seg_ptr.p, d->mb_seg_rec.p, n_seg);
-  DBuf<uint32_t> bseg;
-  bseg.alloc(n_batches + 1);
-  // default every batch offset to n_seg (covers trailing empty batches), then fill real starts.  (A kernel, not a host ->
-  // device copy: a copy would queue behind every value chunk still waiting for the H2D engine.)
-  // a batch's entries are as many in sorted order as in row order and come in batch order: its first segment is the one that holds
-  // its first entry (a walk over all m keys took 1.5 ms for the 153 answers)
-  FMWR_LAUNCH(ctx, mb_batch_first_seg, ceil_div(n_batches + 1, 256), 256, 0, bp.p, e0, segid.p, (uint32_t)m, n_seg, n_batches + 1, bseg.p);
-  FMWR_LAUNCH(ctx, peek_u32, ceil_div(n_batches + 1, 256), 256, 0, bseg.p, n_batches + 1, hp);
-  FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
-  std::vector<uint32_t> hb(hp, hp + n_batches + 1);
-  // empty batches in the middle were filled by the next non-empty one; trailing ones keep n_seg
-  for (int64_t b = 0; b <= n_batches; ++b) d->mb_batch_seg[b] = hb[b];
-  d->mb_batch_seg[n_batches] = n_seg;
-  for (int64_t b = n_batches - 1; b >= 0; --b) if (d->mb_batch_seg[b] > d->mb_batch_seg[b + 1]) d->mb_batch_seg[b] = d->mb_batch_seg[b + 1];
-  d->mb_batch = batch; d->mb_row0 = row0;
-  d->mb_vals_pending = false;
-  if (deferred) { d->mb_e0 = e0; d->mb_vals_pending = true; }
-}
-
-// ---- the same structure built ROW GROUP BY ROW GROUP while the column ids are still uploading (one-shot training path).
-// A group is a run of whole batches (~32M entries); its entries are sorted on (batch inside the group, feature) -- fewer key bits,
-// one radix pass less than the whole-matrix sort -- and emitted into the global arrays at the group's entry / segment offsets.
-template <class K>
-__global__ void mbg_keys(const uint32_t* __restrict__ rowptr, const uint32_t* __restrict__ col, int64_t r0, int64_t r1, int64_t row0,
-                         uint32_t batch, uint32_t b0, int colbits, uint32_t eg0, K* __restrict__ keys, uint32_t* __restrict__ erow)
-{
-  const int64_t row = r0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-  if (row >= r1) return;
-  const uint32_t b = rowptr[row], e = rowptr[row + 1];
-  const uint64_t bid = (uint64_t)((row - row0) / batch) - b0;
-  for (uint32_t j = b + (threadIdx.x & 31); j < e; j += 32) {
-    keys[j - eg0] = (K)((bid << colbits) | (uint64_t)col[j]);
-    erow[j - eg0] = (uint32_t)row;
-  }
-}
-
-template <class K>
-__global__ void mbg_emit(const K* __restrict__ keys, const uint32_t* __restrict__ head, const uint32_t* __restrict__ segid,
-                         const uint32_t* __restrict__ perm_local, const uint32_t* __restrict__ erow, int64_t mg, int colbits, uint32_t eoff,
-                         uint32_t seg_base, uint32_t n_seg_g, uint32_t* __restrict__ seg_ptr, uint4* __restrict__ seg_rec,
-                         uint32_t* __restrict__ ent_row, uint32_t* __restrict__ perm_global)
-{
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= mg) return;
-  const uint32_t e = perm_local[i];
-  const uint32_t r = erow[e];
-  ent_row[eoff + i] = r;
-  perm_global[eoff + i] = e + eoff;                  // relative to the first entry of the whole structure, like the one-piece build
-  if (head[i]) {
-    const uint32_t s = seg_base + segid[i];
-    seg_ptr[s] = eoff + (uint32_t)i;
-    seg_rec[s] = make_uint4((uint32_t)((uint64_t)keys[i] & ((1ull << colbits) - 1ull)), 0u, r, 0u);      // value: mb_fill_values
-  }
-  if (i == mg - 1) seg_ptr[seg_base + n_seg_g] = eoff + (uint32_t)mg;
-}
-
+// host_dst[k] = segment of the first sorted entry of batch b0 + k (a batch's entries are as many in sorted order as in row order
+// and come in batch order); past the group's last entry: its end
 __global__ void mbg_batch_first_seg(const uint32_t* __restrict__ batch_ent, uint32_t eg0, const uint32_t* __restrict__ segid, uint32_t mg, uint32_t n_seg_g,
                                     uint32_t seg_base, int64_t b0, int64_t count, uint32_t* __restrict__ host_dst)
 {
@@ -856,9 +648,12 @@ template <class K>
 static void minibatch_build_grouped(fmwr_data* d, int64_t row0, int64_t batch, int64_t gb /* batches per group */, int gbits)
 {
   fmwr_ctx* ctx = d->ctx;
+  const bool streaming = d->cols_pending;              // column ids (and values) still crossing PCIe
   const int64_t rows = d->n - row0;
   const int64_t n_batches = ceil_div64(rows, batch);
   d->mb_batch_seg.assign(n_batches + 1, 0);
+  // small device -> host reads are zero-copy stores of a kernel into pinned memory: a cudaMemcpy of 4 bytes would queue behind
+  // the upload chunks on the copy engine (measured: the build then ends when the upload ends)
   ctx->h_u32.ensure(2 * (size_t)n_batches + 64);
   uint32_t* hp = ctx->h_u32.p;
   DBuf<uint32_t> bp;
@@ -869,20 +664,22 @@ static void minibatch_build_grouped(fmwr_data* d, int64_t row0, int64_t batch, i
   std::vector<uint32_t> ent(hp + 8, hp + 8 + n_batches + 1);       // absolute first entry of every batch
   const uint32_t e0 = ent[0], e1 = ent[n_batches];
   const int64_t m = (int64_t)e1 - e0;
+  // entries before each batch (rows of a batch are consecutive, so this is also the batch's offset in the sorted arrays)
   d->mb_batch_ent.resize(n_batches + 1);
   for (int64_t b = 0; b <= n_batches; ++b) d->mb_batch_ent[b] = (int64_t)ent[b] - (int64_t)e0;
   const int colbits = bits_for((uint64_t)(d->p > 0 ? d->p - 1 : 0));
   // segments: at most one per entry and at most one per (batch, feature)
-  const int64_t seg_cap = std::min<int64_t>(m, n_batches * d->p);
-  d->mb_ent_row.alloc(m + 8); d->mb_ent_val.alloc(m + 8); d->mb_perm.alloc(m);
-  d->mb_seg_ptr.alloc((size_t)seg_cap + 1 + 8); d->mb_seg_rec.alloc(seg_cap);
+  const int64_t seg_cap = (int64_t)std::min<uint64_t>(m, (uint64_t)n_batches * (uint64_t)d->p);
+  d->mb_ent_row.alloc(m + 8); d->mb_ent_val.alloc(m + 8);      // +8: the dense update kernel stages 16-byte-rounded ranges (update_tma.cuh)
+  if (streaming) d->mb_perm.alloc(m);
+  else data_wait_values(d);
   int64_t mg_max = 0;
   for (int64_t b0 = 0; b0 < n_batches; b0 += gb) mg_max = std::max<int64_t>(mg_max, (int64_t)ent[std::min(n_batches, b0 + gb)] - ent[b0]);
   DBuf<K> keys_in, keys_out;
   DBuf<uint32_t> perm, erow, head, segid;
   DBuf<int> flags;
-  keys_in.alloc(mg_max); keys_out.alloc(mg_max); perm.alloc(mg_max); erow.alloc(mg_max); head.alloc(mg_max); segid.alloc(mg_max);
-  flags.alloc(1); flags.zero(ctx->stream);
+  keys_in.alloc(mg_max); keys_out.alloc(mg_max); erow.alloc(mg_max); head.alloc(mg_max); segid.alloc(mg_max); perm.alloc(mg_max);
+  if (streaming) { flags.alloc(1); flags.zero(ctx->stream); }
   uint32_t seg_base = 0;
   int64_t next_ev = 0;                                 // column chunks already waited for
   for (int64_t b0 = 0; b0 < n_batches; b0 += gb) {
@@ -890,12 +687,15 @@ static void minibatch_build_grouped(fmwr_data* d, int64_t row0, int64_t batch, i
     const int64_t r0 = row0 + b0 * batch, r1 = std::min(d->n, row0 + b1 * batch);
     const uint32_t eg0 = ent[b0], eg1 = ent[b1];
     const int64_t mg = (int64_t)eg1 - eg0;
-    // the chunks that hold this group's column ids
-    const int64_t need = mg > 0 ? ((int64_t)eg1 - 1) / d->col_chunk + 1 : next_ev;
-    for (; next_ev < need && next_ev < (int64_t)d->col_ev.size(); ++next_ev) FMWR_CUDA(cudaStreamWaitEvent(ctx->stream, d->col_ev[next_ev], 0));
+    if (streaming) {
+      // the chunks that hold this group's column ids
+      const int64_t need = mg > 0 ? ((int64_t)eg1 - 1) / d->col_chunk + 1 : next_ev;
+      for (; next_ev < need && next_ev < (int64_t)d->col_ev.size(); ++next_ev) FMWR_CUDA(cudaStreamWaitEvent(ctx->stream, d->col_ev[next_ev], 0));
+    }
     uint32_t n_seg_g = 0;
     if (mg > 0) {
-      FMWR_LAUNCH(ctx, validate_csr, ceil_div(r1 - r0, 256), 256, 0, d->rowptr.p + r0, d->col.p, r1 - r0, (uint32_t)d->p, (uint32_t)d->nnz, flags.p);
+      // (resident data was validated when it was uploaded)
+      if (streaming) FMWR_LAUNCH(ctx, validate_csr, ceil_div(r1 - r0, 256), 256, 0, d->rowptr.p + r0, d->col.p, r1 - r0, (uint32_t)d->p, (uint32_t)d->nnz, flags.p);
       FMWR_LAUNCH(ctx, mbg_keys<K>, ceil_div((r1 - r0) * 32, 256), 256, 0, d->rowptr.p, d->col.p, r0, r1, row0, (uint32_t)batch, (uint32_t)b0, colbits, eg0,
                   keys_in.p, erow.p);
       if (sizeof(K) == 4) sort_pairs_u32(ctx, (const uint32_t*)keys_in.p, (uint32_t*)keys_out.p, nullptr, perm.p, mg, colbits + gbits);
@@ -903,10 +703,10 @@ static void minibatch_build_grouped(fmwr_data* d, int64_t row0, int64_t batch, i
       FMWR_LAUNCH(ctx, mb_heads<K>, ceil_div(mg, 256), 256, 0, keys_out.p, mg, head.p);
       exclusive_scan_u32(ctx, head.p, segid.p, mg);
       FMWR_LAUNCH(ctx, peek2_u32, 1, 32, 0, segid.p + (mg - 1), head.p + (mg - 1), hp);
-      FMWR_LAUNCH(ctx, peek_u32, 1, 32, 0, reinterpret_cast<const uint32_t*>(flags.p), (int64_t)1, hp + 4);
+      if (streaming) FMWR_LAUNCH(ctx, peek_u32, 1, 32, 0, reinterpret_cast<const uint32_t*>(flags.p), (int64_t)1, hp + 4);
     }
     FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (mg > 0) {
+    if (streaming && mg > 0) {
       // a bad group stops the build here, with the reference's message, before its keys are taken for segments
       const uint32_t hf = hp[4];
       if (hf) d->cols_pending = false;
@@ -916,9 +716,14 @@ static void minibatch_build_grouped(fmwr_data* d, int64_t row0, int64_t batch, i
     }
     if (mg > 0) n_seg_g = hp[0] + hp[1];
     FMWR_REQUIRE((int64_t)seg_base + n_seg_g <= seg_cap, FMWR_ERR_SHAPE, "segment count exceeds its bound");
+    if (b0 == 0) {
+      // one group: exactly its segments; several: the bound (the later groups are not counted yet)
+      const int64_t cap = gb == n_batches ? n_seg_g : seg_cap;
+      d->mb_seg_ptr.alloc((size_t)cap + 1 + 8); d->mb_seg_rec.alloc(cap);
+    }
     if (mg > 0) {
-      FMWR_LAUNCH(ctx, mbg_emit<K>, ceil_div(mg, 256), 256, 0, keys_out.p, head.p, segid.p, perm.p, erow.p, mg, colbits, eg0 - e0, seg_base, n_seg_g,
-                  d->mb_seg_ptr.p, d->mb_seg_rec.p, d->mb_ent_row.p, d->mb_perm.p);
+      FMWR_LAUNCH(ctx, mbg_emit<K>, ceil_div(mg, 256), 256, 0, keys_out.p, head.p, segid.p, perm.p, erow.p, streaming ? (const float*)nullptr : d->val.p,
+                  mg, colbits, eg0, eg0 - e0, seg_base, n_seg_g, d->mb_seg_ptr.p, d->mb_seg_rec.p, d->mb_ent_row.p, d->mb_ent_val.p, d->mb_perm.p);
       FMWR_LAUNCH(ctx, mb_seg_len, ceil_div(n_seg_g, 256), 256, 0, d->mb_seg_ptr.p + seg_base, d->mb_seg_rec.p + seg_base, n_seg_g);
     }
     FMWR_LAUNCH(ctx, mbg_batch_first_seg, ceil_div(b1 - b0, 256), 256, 0, bp.p, eg0, segid.p, (uint32_t)mg, n_seg_g, seg_base, b0, b1 - b0, hp + 16);
@@ -927,48 +732,85 @@ static void minibatch_build_grouped(fmwr_data* d, int64_t row0, int64_t batch, i
     seg_base += n_seg_g;
   }
   const uint32_t n_seg = seg_base;
+  // empty batches in the middle share the next non-empty one's first segment; trailing ones start at n_seg
   d->mb_batch_seg[n_batches] = n_seg;
   for (int64_t b = n_batches - 1; b >= 0; --b) if (d->mb_batch_seg[b] > d->mb_batch_seg[b + 1]) d->mb_batch_seg[b] = d->mb_batch_seg[b + 1];
   if (m == 0) FMWR_CUDA(cudaMemsetAsync(d->mb_seg_ptr.p, 0, 4, ctx->stream));
-  // rows before row0 (the skipped first row) were not part of any group: validate them with the rest of the checks
-  for (; next_ev < (int64_t)d->col_ev.size(); ++next_ev) FMWR_CUDA(cudaStreamWaitEvent(ctx->stream, d->col_ev[next_ev], 0));
-  if (row0 > 0) FMWR_LAUNCH(ctx, validate_csr, ceil_div(row0, 256), 256, 0, d->rowptr.p, d->col.p, row0, (uint32_t)d->p, (uint32_t)d->nnz, flags.p);
-  int h = 0;
-  FMWR_CUDA(cudaMemcpyAsync(&h, flags.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
-  d->cols_pending = false;
-  FMWR_REQUIRE(!(h & 4), FMWR_ERR_SHAPE, "the length of input's row_size is not correct...");
-  FMWR_REQUIRE(!(h & 1), FMWR_ERR_SHAPE, "col_idx out of range (>= number of features)");
-  FMWR_REQUIRE(!(h & 2), FMWR_ERR_SHAPE, "col_idx must be strictly ascending within each row");
+  if (streaming) {
+    // rows before row0 (the skipped first row) were not part of any group: validate them with the rest of the checks
+    for (; next_ev < (int64_t)d->col_ev.size(); ++next_ev) FMWR_CUDA(cudaStreamWaitEvent(ctx->stream, d->col_ev[next_ev], 0));
+    if (row0 > 0) FMWR_LAUNCH(ctx, validate_csr, ceil_div(row0, 256), 256, 0, d->rowptr.p, d->col.p, row0, (uint32_t)d->p, (uint32_t)d->nnz, flags.p);
+    int h = 0;
+    FMWR_CUDA(cudaMemcpyAsync(&h, flags.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
+    d->cols_pending = false;
+    FMWR_REQUIRE(!(h & 4), FMWR_ERR_SHAPE, "the length of input's row_size is not correct...");
+    FMWR_REQUIRE(!(h & 1), FMWR_ERR_SHAPE, "col_idx out of range (>= number of features)");
+    FMWR_REQUIRE(!(h & 2), FMWR_ERR_SHAPE, "col_idx must be strictly ascending within each row");
+  }
   d->mb_batch = batch; d->mb_row0 = row0;
-  d->mb_e0 = e0; d->mb_vals_pending = true;
+  d->mb_e0 = e0; d->mb_vals_pending = streaming;
 }
 
 void minibatch_build(fmwr_data* d, int64_t row0, int64_t batch)
 {
   if (d->mb_batch == batch && d->mb_row0 == row0) return;
-  if (d->cols_pending && batch > 0 && d->n - row0 > 0 && d->up_chunks > 0 && d->nnz > 0) {
-    // one-shot path, columns and values still crossing PCIe: build group by group behind the upload
-    const int64_t rows = d->n - row0;
-    const int64_t n_batches = ceil_div64(rows, batch);
-    const double per_batch = (double)d->nnz / (double)n_batches;
-    const double group_entries = getenv("FMWR_GROUP_ENTRIES") ? atof(getenv("FMWR_GROUP_ENTRIES")) : (double)(32ll << 20);
-    int64_t gb = (int64_t)std::max(1.0, std::floor(group_entries / std::max(1.0, per_batch)));
-    if (gb > n_batches) gb = n_batches;
-    const int gbits = bits_for((uint64_t)(gb > 0 ? gb - 1 : 0));
-    const int bits = bits_for((uint64_t)(d->p > 0 ? d->p - 1 : 0)) + gbits;
-    if (bits <= 32) minibatch_build_grouped<uint32_t>(d, row0, batch, gb, gbits);
-    else minibatch_build_grouped<uint64_t>(d, row0, batch, gb, gbits);
+  const int64_t rows = d->n - row0;
+  if (rows <= 0 || batch <= 0) {
+    data_wait_cols(d);
+    FMWR_REQUIRE(batch > 0, FMWR_ERR_ARG, "batch_size must be positive");
+    d->mb_batch_seg.assign(1, 0); d->mb_batch_ent.assign(1, 0);
+    d->mb_batch = batch; d->mb_row0 = row0;
     return;
   }
-  data_wait_cols(d);
-  FMWR_REQUIRE(batch > 0, FMWR_ERR_ARG, "batch_size must be positive");
-  const int64_t rows = d->n - row0;
-  const int64_t n_batches = rows > 0 ? ceil_div64(rows, batch) : 0;
-  const int bits = bits_for((uint64_t)(d->p > 0 ? d->p - 1 : 0)) + bits_for((uint64_t)(n_batches > 0 ? n_batches - 1 : 0));
-  if (bits <= 32) minibatch_build_t<uint32_t>(d, row0, batch);     // (batch, feature) fits one word: half the sort traffic
-  else minibatch_build_t<uint64_t>(d, row0, batch);
+  const int64_t n_batches = ceil_div64(rows, batch);
+  int64_t gb = n_batches;                              // resident data: one group
+  if (d->cols_pending) {
+    // one-shot path, columns and values still crossing PCIe: build group by group behind the upload
+    const double per_batch = (double)d->nnz / (double)n_batches;
+    const double group_entries = getenv("FMWR_GROUP_ENTRIES") ? atof(getenv("FMWR_GROUP_ENTRIES")) : (double)(32ll << 20);
+    gb = std::min(n_batches, (int64_t)std::max(1.0, std::floor(group_entries / std::max(1.0, per_batch))));
+  }
+  const int gbits = bits_for((uint64_t)(gb - 1));
+  const int bits = bits_for((uint64_t)(d->p > 0 ? d->p - 1 : 0)) + gbits;
+  if (bits <= 32) minibatch_build_grouped<uint32_t>(d, row0, batch, gb, gbits);     // (batch, feature) fits one word: half the sort traffic
+  else minibatch_build_grouped<uint64_t>(d, row0, batch, gb, gbits);
 }
+
+static void minibatch_fill_values(fmwr_data* d, uint32_t seg_lo, uint32_t seg_hi)
+{
+  if (seg_hi <= seg_lo) return;
+  FMWR_LAUNCH(d->ctx, mb_fill_values, ceil_div((int64_t)seg_hi - seg_lo, 256), 256, 0, d->mb_seg_ptr.p, d->mb_seg_rec.p, d->mb_perm.p, d->val.p,
+              d->mb_e0, seg_lo, seg_hi, d->mb_ent_val.p);
+}
+
+// the values of batch b of the per-batch CSC ready on the compute stream: it waits for the value chunks that hold the batch's
+// entries, narrows the raw ones and fills the batch's segments (nothing to do once every value is in place)
+void minibatch_batch_values(fmwr_data* d, int64_t b)
+{
+  if (!d->mb_vals_pending) return;
+  const int64_t lo = b == 0 ? 0 : (int64_t)d->mb_e0 + d->mb_batch_ent[b], hi = (int64_t)d->mb_e0 + d->mb_batch_ent[b + 1];
+  if (hi > 0) {
+    const int64_t ci = std::min<int64_t>((int64_t)d->val_ev.size() - 1, (hi - 1) / d->val_chunk);
+    data_wait_chunk_issued(d, ci);          // the event exists once the uploader has queued the chunk
+    // every chunk up to ci (a mixed upload queues a raw chunk before the two narrowed ones in front of it)
+    for (; d->val_waited <= ci; ++d->val_waited) FMWR_CUDA(cudaStreamWaitEvent(d->ctx->stream, d->val_ev[d->val_waited], 0));
+  }
+  data_narrow_values(d, lo, hi);
+  minibatch_fill_values(d, (uint32_t)d->mb_batch_seg[b], (uint32_t)d->mb_batch_seg[b + 1]);
+  if (b + 2 == (int64_t)d->mb_batch_seg.size()) { d->mb_vals_pending = false; d->val_all_narrowed = true; }     // the last batch
+}
+
+// every value of the per-batch CSC in place (a first epoch that stopped before its last batch)
+void minibatch_all_values(fmwr_data* d)
+{
+  if (!d->mb_vals_pending) return;
+  data_wait_values(d);
+  minibatch_fill_values(d, 0u, (uint32_t)d->mb_batch_seg.back());
+  d->mb_vals_pending = false;
+}
+
+int64_t minibatch_entries(const fmwr_data* d) { return d->mb_batch_ent.empty() ? 0 : d->mb_batch_ent.back(); }
 
 // ------------------------------------------------------------------------------------------ scales / normalize
 __global__ void col_moments(const uint32_t* __restrict__ col, const float* __restrict__ val, int64_t nnz,
@@ -1302,6 +1144,8 @@ __global__ void gather_row_entries(const uint32_t* __restrict__ rowptr, const ui
 fmwr_data* data_gather_rows(fmwr_data* src, const uint32_t* order_dev, int64_t m)
 {
   fmwr_ctx* ctx = src->ctx;
+  data_wait_cols(src);
+  data_wait_values(src);
   fmwr_data* d = new fmwr_data();
   try {
     d->ctx = ctx; d->n = m; d->p = src->p;
@@ -1342,6 +1186,7 @@ fmwr_data* data_concat_rows(fmwr_data* const* parts, int n_parts)
                  "parts must share context, feature count and label presence");
     n += parts[i]->n; nnz += parts[i]->nnz;
   }
+  for (int i = 0; i < n_parts; ++i) { data_wait_cols(parts[i]); data_wait_values(parts[i]); }
   FMWR_REQUIRE(nnz < (int64_t)0xffffffffll && n < (int64_t)0xffffffffll, FMWR_ERR_UNSUPPORTED, "dimensions must fit 32-bit indices per device shard");
   fmwr_data* d = new fmwr_data();
   try {

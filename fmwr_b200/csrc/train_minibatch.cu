@@ -26,10 +26,6 @@ int solver_state_count(const SolverParams<double>& sp);
 double tracker_score(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s);
 void tracker_snapshot(fmwr_model* m, fmwr_trace* tr, int idx, int iter, double score);
 int tracker_step_size(int step_size, int max_iter);
-void minibatch_fill_values(fmwr_data* d, uint32_t seg_lo, uint32_t seg_hi);
-void data_wait_values(fmwr_data* d);
-void data_narrow_values(fmwr_data* d, int64_t lo, int64_t hi);
-void data_wait_chunk_issued(fmwr_data* d, int64_t ci);
 void comm_allreduce_sum(fmwr_ctx* ctx, void* buf, size_t count, bool f64);
 
 // ---- K1: forward + multiplier + S cache --------------------------------------------------------
@@ -808,6 +804,14 @@ static double tracker_score_sharded(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, 
   return evaluate_dev(ctx, d, m->cfg.task, s->metric);
 }
 
+// Data whose values are still uploading (fmwr_train) may go to this trainer when nothing reads them before their batch: no
+// tracker (its scoring pass reads every row) and no strided or explicit visit order (its rows are gathered up front).
+bool minibatch_streams_values(const fmwr_solver_cfg* s)
+{
+  return s->mode == FMWR_MODE_MINIBATCH && (s->solver == FMWR_SGD || s->solver == FMWR_FTRL || s->solver == FMWR_TDAP) &&
+         s->step_size <= 0 && s->random_step <= 1 && !(s->visit_order && s->n_visit > 0);
+}
+
 template <class T>
 static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, fmwr_data* eval_d = nullptr)
 {
@@ -936,18 +940,7 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
     for (int64_t b = 0; b < n_batches && iter < max_iter; ++b) {
       if (use_graph && captured == 0) { FMWR_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal)); bag.capturing = true; }
       const int64_t rb = row0 + b * B;
-      if (d->mb_vals_pending) {
-        const int64_t last_entry = (int64_t)d->mb_e0 + d->mb_batch_ent[b + 1] - 1;
-        if (last_entry >= 0 && d->val_chunk > 0) {
-          const size_t ci = std::min<size_t>(d->val_ev.size() - 1, (size_t)(last_entry / d->val_chunk));
-          data_wait_chunk_issued(d, (int64_t)ci);          // host-narrowed upload: the event exists once the uploader queued the chunk
-          // every chunk up to ci (a mixed upload queues a raw chunk before the two narrowed ones in front of it)
-          for (; d->val_waited <= (int64_t)ci; ++d->val_waited) FMWR_CUDA(cudaStreamWaitEvent(ctx->stream, d->val_ev[d->val_waited], 0));
-        }
-        data_narrow_values(d, b == 0 ? 0 : (int64_t)d->mb_e0 + d->mb_batch_ent[b], (int64_t)d->mb_e0 + d->mb_batch_ent[b + 1]);
-        minibatch_fill_values(d, (uint32_t)d->mb_batch_seg[b], (uint32_t)d->mb_batch_seg[b + 1]);
-        if (b == n_batches - 1) { d->mb_vals_pending = false; d->val_all_narrowed = true; }      // every batch has its values now
-      }
+      minibatch_batch_values(d, b);
       int64_t rows = std::min<int64_t>(B, d->n - rb);
       rows = std::min<int64_t>(rows, max_iter - iter);
       L.row_begin = rb; L.rows = (int)rows;
@@ -984,11 +977,7 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
       }
     }
   }
-  if (d->mb_vals_pending) {                      // a truncated first epoch: finish the value fill for later calls
-    data_wait_values(d);
-    minibatch_fill_values(d, 0u, (uint32_t)d->mb_batch_seg[n_batches]);
-    d->mb_vals_pending = false;
-  }
+  minibatch_all_values(d);                       // a truncated first epoch: finish the value fill for later calls
   flush_graph();
   if (sgd_l1) { const double h[2] = {u_w, u_v}; FMWR_CUDA(cudaMemcpyAsync((double*)m->scal.p + 1, h, 16, cudaMemcpyHostToDevice, ctx->stream)); }
   FMWR_CUDA(cudaStreamSynchronize(ctx->stream));

@@ -164,12 +164,14 @@ def test_warm_state_continues_the_optimizer(gpu_ctx, solver, regs, mode):
     d.close()
 
 
-@pytest.mark.parametrize("group_entries,pinned", [(None, False), ("1000000", False), ("250000", False), ("1000000", True), (None, True)])
+@pytest.mark.parametrize("group_entries,pinned,random_step",
+                         [(None, False, 1), ("1000000", False, 1), ("250000", False, 1), ("1000000", True, 1), (None, True, 1), ("1000000", True, 3)])
 @pytest.mark.parametrize("solver", [O.FTRL, O.SGD])
-def test_one_shot_train_equals_handle_path(gpu_ctx, monkeypatch, solver, group_entries, pinned):
+def test_one_shot_train_equals_handle_path(gpu_ctx, monkeypatch, solver, group_entries, pinned, random_step):
     """fmwr_train (host fm.matrix lists in, host model out; the values upload on the copy stream while the per-batch CSC is
     sorted, and every batch waits only for its own chunk) must give the parameters of the handle path bit for bit --
-    also over two epochs, when the second pass finds every value in place."""
+    also over two epochs, when the second pass finds every value in place.  random_step > 1 gathers the visited rows up front,
+    so there the one-shot call must upload every value before training."""
     import ctypes as C
     ctx = gpu_ctx
     lib = L.lib()
@@ -188,13 +190,17 @@ def test_one_shot_train_equals_handle_path(gpu_ctx, monkeypatch, solver, group_e
     w = rng.normal(0, 0.02, p); v = rng.normal(0, 0.02, (p, k)); w0 = 0.01
     mc = L.ModelCfg(task=L.CLASSIFICATION, keep_w0=1, keep_w1=1, k=k, l1_w1=1e-4, l2_w1=1e-3, l2_v=1e-3)
     for iters in (n - 1, 2 * (n - 1) - 12345):
-        sc = L.SolverCfg(solver=solver, max_iter=iters, random_step=1, learn_rate=0.01, alpha_w=0.1, alpha_v=0.1, beta_w=1.0, beta_v=1.0,
+        sc = L.SolverCfg(solver=solver, max_iter=iters, random_step=random_step, learn_rate=0.01, alpha_w=0.1, alpha_v=0.1, beta_w=1.0, beta_v=1.0,
                          min_target=-1.0, max_target=1.0, mode=L.MODE_MINIBATCH, batch_size=16384, precision=L.F32,
                          compat=L.COMPAT_REFERENCE, step_size=-1)
         d = L.Data.from_csr32(ctx, n, p, rowptr, col, val, y)
         m = L.Model(ctx, mc, p, L.F32); m.set(w0, w, v)
+        C.CDLL(None).srand(5)                              # random_step > 1: both calls draw the same visit sequence from rand()
         L.train_dev(ctx, m, d, sc)
         a = m.get(); m.close(); d.close()
+        # the library reuses freed device blocks: leave other values in the blocks of this size, so that a value the one-shot
+        # call never uploads shows up as a difference instead of as the handle path's leftover
+        L.Data.from_csr32(ctx, n, p, rowptr, col, val + 1.0, y).close()
         rs = np.diff(rowptr.astype(np.int64)).astype(np.int32)
         ci = col.astype(np.int32); v64 = val.astype(np.float64); y64 = y.astype(np.float64)
         bw0 = C.c_double(w0); bw = w.copy(); bv = v.copy()
@@ -202,6 +208,7 @@ def test_one_shot_train_equals_handle_path(gpu_ctx, monkeypatch, solver, group_e
             for arr in (ci, v64):
                 L.check(lib.fmwr_host_pin(L.ptr(arr), C.c_int64(arr.nbytes)))
         try:
+            C.CDLL(None).srand(5)
             L.check(lib.fmwr_train(C.byref(mc), C.byref(sc), C.c_int64(n), C.c_int64(p), C.c_int64(ci.size), L.ptr(rs), L.ptr(ci), L.ptr(v64),
                                    L.ptr(y64), C.byref(bw0), L.ptr(bw), L.ptr(bv), None))
         finally:
