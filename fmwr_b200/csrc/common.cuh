@@ -280,16 +280,8 @@ __device__ __forceinline__ char* peer_base(const PeerArgs& pa, int i)
 
 // __threadfence_system() is fence.sc.sys (MEMBAR.SC.SYS); the release / acquire patterns here need no sequential consistency
 // between fences, and the acq_rel form is the cheaper instruction (the cta-scope pair measured 3000-6000 vs < 1000 cycles in the
-// exact pipeline, profiles/r02_summary.md).  FMWR_PEER_SC_FENCE=1 at build time restores the old form for A/B.
-#ifdef FMWR_PEER_SC_FENCE
-__device__ __forceinline__ void peer_fence_sys() { __threadfence_system(); }
-#else
+// exact pipeline, profiles/r02_summary.md).
 __device__ __forceinline__ void peer_fence_sys() { asm volatile("fence.acq_rel.sys;" ::: "memory"); }
-#endif
-#ifndef FMWR_PEER_NAP
-#define FMWR_PEER_NAP 0          // ns between polls of a peer flag; 0 = plain spinning (__nanosleep wakes late)
-#endif
-__device__ __forceinline__ void peer_nap() { if (FMWR_PEER_NAP) __nanosleep(FMWR_PEER_NAP); }
 __device__ __forceinline__ void st_release_sys(uint32_t* p, uint32_t v) { asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
 // flag stores AFTER one __threadfence_system(): fence + relaxed stores is the release pattern, and it costs one system-scope
 // fence per publication instead of one per peer (st.release.sys in a loop over 8 ranks was 8 fences back to back)
@@ -326,9 +318,9 @@ __device__ __forceinline__ void peer_wait(const PeerArgs& pa, int flag_base, int
     const uint32_t ep = *reinterpret_cast<volatile uint32_t*>(ctl + epoch_word);
     const uint32_t* f = ctl + flag_base + 32 * threadIdx.x;
     const long long t0 = clock64();
+    // plain spinning between polls: __nanosleep wakes late
     while ((int32_t)(ld_acquire_sys(f) - ep) < 0) {
       if (clock64() - t0 > 40000000000ll) { ctl[PEER_ERR] = 1u; break; }   // ~20 s: a peer died; the host reports it
-      peer_nap();
     }
   }
   __syncthreads();
@@ -377,7 +369,6 @@ __device__ __forceinline__ void peer_wait_ep(const PeerArgs& pa, int flag_base, 
     // invalidates the SM's L1, and hundreds of CTAs polling that way slow down the CTAs that are still computing
     while ((int32_t)(*reinterpret_cast<const volatile uint32_t*>(f) - ep) < 0) {
       if (clock64() - t0 > 40000000000ll) { ctl[PEER_ERR] = 1u; break; }
-      peer_nap();
     }
     (void)ld_acquire_sys(f);
   }

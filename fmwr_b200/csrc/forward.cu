@@ -6,7 +6,7 @@
 namespace fmwr {
 
 template <class T, int LPR, int CH, int TEAM>
-__global__ void __launch_bounds__(256, FMWR_FWD_BLOCKS)
+__global__ void __launch_bounds__(256, FWD_BLOCKS)
 forward_kernel(const uint32_t* __restrict__ rowptr, const uint32_t* __restrict__ col, const float* __restrict__ val,
                const T* __restrict__ w, const T* __restrict__ v, const double* __restrict__ scal, int kp, int k0, int k1,
                int64_t n, int link, double lo, double hi, const double* __restrict__ pnY, double* __restrict__ out)
@@ -55,8 +55,7 @@ struct FwdLaunch {
   {
     const int block = 256, rpb = (block / 32) * (32 / TEAM);
     int64_t want = ceil_div64(d->n, rpb);
-    static const int fwd_ctas = getenv("FMWR_FWD_CTAS") ? atoi(getenv("FMWR_FWD_CTAS")) : 32;
-    int64_t cap = (int64_t)ctx->sm_count * fwd_ctas;   // CTAs per SM, grid-stride beyond that
+    int64_t cap = (int64_t)ctx->sm_count * 32;   // 32 CTAs per SM, grid-stride beyond that
     int grid = (int)(want < cap ? want : cap);
     if (grid < 1) grid = 1;
     // predictions are always kept in fp64 (8 of ~5.5 KB per row): the R side wants a NumericVector and the

@@ -178,14 +178,9 @@ __device__ __forceinline__ T team_sum(T x)
   return x;
 }
 
-#ifndef FMWR_FWD_U
-#define FMWR_FWD_U 4
-#endif
-#ifndef FMWR_FWD_BLOCKS
-#define FMWR_FWD_BLOCKS 4
-#endif
-// factor rows in flight per sub-group: long rows (warp team) take the experiment knobs, short rows 4
-template <int LPR, int TEAM = 32> struct GatherDepth { enum { U = TEAM != 32 ? 4 : (LPR >= 16 ? 8 : FMWR_FWD_U) }; };
+constexpr int FWD_BLOCKS = 4;      // resident CTAs per SM of the row-forward kernels
+// factor rows in flight per sub-group: 8 for warp teams over 16 or 32 lanes per row, otherwise 4
+template <int LPR, int TEAM = 32> struct GatherDepth { enum { U = (TEAM == 32 && LPR >= 16) ? 8 : 4 }; };
 
 // score (no link) of the team's row, identical in every lane of the team
 template <class T, int LPR, int CH, int TEAM>
@@ -211,13 +206,9 @@ __device__ __forceinline__ T team_forward_partial(const uint32_t* __restrict__ c
 // rows with at most this many non-zeros per LPR-lane group on average go one row per group
 __host__ __device__ inline bool short_rows(int64_t nnz, int64_t n, int lpr) { return lpr < 32 && n > 0 && nnz <= n * 4 * (32 / lpr); }
 // 1: one row per LPR-lane group; 2: one row per half warp (two sub-groups; the per-row fixed cost -- bounds, linear sweep,
-// combine, team sum, stores -- is shared by two rows per warp); 0: one row per warp.  FMWR_TEAM=8|16|32 forces a choice.
+// combine, team sum, stores -- is shared by two rows per warp); 0: one row per warp.
 inline int team_mode(int64_t nnz, int64_t n, int lpr)
 {
-  static const int forced = getenv("FMWR_TEAM") ? atoi(getenv("FMWR_TEAM")) : 0;
-  if (forced == 32) return 0;
-  if (forced == 16) return lpr <= 8 ? 2 : (lpr == 16 ? 1 : 0);
-  if (forced == 8) return lpr < 32 ? 1 : 0;
   if (short_rows(nnz, n, lpr)) return 1;
   // long rows: half-warp teams measured best for every k <= 32 (predict 8.4 -> 6.6 ms at k = 32, 4.8 -> 3.7 ms at k = 8); k = 64 is
   // DRAM-bound either way and keeps one row per 16-lane group

@@ -20,9 +20,7 @@
 
 namespace fmwr {
 
-#ifndef FMWR_SF_BLOCKS
-#define FMWR_SF_BLOCKS 3     // 78 registers, no spills; at 4 (64 registers) ptxas rematerialises every shared-memory address per step
-#endif
+constexpr int SF_BLOCKS = 3;     // 78 registers, no spills; at 4 (64 registers) ptxas rematerialises every shared-memory address per step
 __device__ __forceinline__ unsigned long long globaltimer_ns() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
 enum { SF_PREDICT = 0, SF_TRAIN = 1, SF_PARTIAL = 2, SF_PARTIAL_PEER = 3 };
 
@@ -40,7 +38,7 @@ struct SfArgs {
 };
 
 template <int MODE>
-__global__ void __launch_bounds__(256, FMWR_SF_BLOCKS) forward_stream_kernel(SfArgs a)
+__global__ void __launch_bounds__(256, SF_BLOCKS) forward_stream_kernel(SfArgs a)
 {
   constexpr int LPR = 8, U = 8;
   const int lane = threadIdx.x & 31, g = lane >> 3, l = lane & 7;
@@ -245,14 +243,12 @@ static __global__ void link_inplace_kernel(double* __restrict__ out, int64_t n, 
 // group idles while others walk one row more: rows per group from the resident group count, CTAs from the groups needed.
 inline int stream_grid(const fmwr_ctx* ctx, int64_t rows, int* rpg_out)
 {
-  const int sf_ctas = getenv("FMWR_SF_CTAS") ? atoi(getenv("FMWR_SF_CTAS")) : FMWR_SF_BLOCKS;
-  const int64_t max_groups = (int64_t)ctx->sm_count * sf_ctas * 32;
+  const int64_t max_groups = (int64_t)ctx->sm_count * SF_BLOCKS * 32;
   int64_t rpg = std::max<int64_t>(1, (rows + max_groups - 1) / max_groups);
   // Long launches: cap the rows per group and let the grid run in waves.  With one contiguous range per resident group the
   // groups of an SM stream from ~100 different 2 MB pages of the CSR arrays at once (on top of the 64 pages of V) and the
   // 128-entry TLB thrashes: predict over 10M rows took 8.9 ms with 704 rows per group, 5.8 ms with 64 (profiles/r02_summary.md)
-  const int64_t cap = getenv("FMWR_SF_RPG") ? atoll(getenv("FMWR_SF_RPG")) : 64;
-  if (cap > 0 && rpg > cap) rpg = cap;
+  rpg = std::min<int64_t>(rpg, 64);
   const int64_t groups = (rows + rpg - 1) / rpg;
   *rpg_out = (int)rpg;
   return (int)std::max<int64_t>(1, (groups + 31) / 32);
@@ -263,8 +259,7 @@ inline int stream_grid(const fmwr_ctx* ctx, int64_t rows, int* rpg_out)
 // stream kernel, which then also runs the exchange)
 inline bool stream_forward_ok(const fmwr_model* m, int64_t nnz, int64_t n, int min_nnz_per_row = 8)
 {
-  const bool off = getenv("FMWR_NO_STREAM") != nullptr;     // read per call: tests flip it
-  return !off && m->prec == FMWR_F32 && m->kp == 32 && n > 0 && n < (1ll << 31) && nnz >= (int64_t)min_nnz_per_row * n;
+  return m->prec == FMWR_F32 && m->kp == 32 && n > 0 && n < (1ll << 31) && nnz >= (int64_t)min_nnz_per_row * n;
 }
 
 }  // namespace fmwr

@@ -793,11 +793,8 @@ struct FusedArgs {
   int cur_sorted;      // the rows are sorted by the current field: equal features sit in consecutive rows
 };
 
-#ifndef FMWR_FUSED_BLOCKS
-#define FMWR_FUSED_BLOCKS 3
-#endif
 constexpr int FUSED_THREADS = 512;
-constexpr int FUSED_BLOCKS = FMWR_FUSED_BLOCKS;  // resident CTAs per SM
+constexpr int FUSED_BLOCKS = 3;             // resident CTAs per SM
 constexpr int FUSED_MAX_REP = 64;           // replicas of the per-feature (A, B) table
 constexpr size_t FUSED_AB_BYTES = 8u << 20; // ... as many as fit this budget (L2-resident)
 
@@ -1127,7 +1124,7 @@ static void run_steps_dense(fmwr_ctx* ctx, const std::vector<uint32_t>& pbeg, co
   uint32_t max_cols = 1;
   for (size_t j = 0; j + 1 < pbeg.size(); ++j) max_cols = std::max(max_cols, pbeg[j + 1] - pbeg[j]);
   const size_t slot_bytes = ((size_t)2 * max_cols * sizeof(T) + 255) & ~(size_t)255;
-  const bool use_peer = ctx->nccl_comm && ctx->world > 1 && ctx->peer.ready && getenv("FMWR_NO_PEER") == nullptr &&
+  const bool use_peer = ctx->nccl_comm && ctx->world > 1 && ctx->peer.ready &&
                         PEER_CTL_BYTES + 2 * (size_t)ctx->world * slot_bytes <= ctx->peer.bytes;
   if (use_peer) {
     pa.rank = ctx->rank; pa.world = ctx->world;
@@ -1578,7 +1575,6 @@ __global__ void repack_rows_kernel(const A* __restrict__ src, int kp_src, B* __r
 int als_effective_precision(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s)
 {
   if (m->prec == FMWR_F64) return FMWR_F64;
-  if (getenv("FMWR_ALS_F32_STRICT")) return FMWR_F32;       // diagnostics: measure what fp32 does on such data
   if (s->solver == FMWR_MCMC && m->cfg.task == FMWR_CLASSIFICATION) return FMWR_F64;
   return has_thin_columns(ctx, d) ? FMWR_F64 : FMWR_F32;
 }

@@ -50,7 +50,7 @@ struct ExactArgs {
   int skip_row0;             // F5: scan rows 1..n-1
   int64_t t_begin, t_end;    // sample counters of this launch
   int tdap_zw_index;         // F6
-  int prefetch;              // L2 run-ahead of parameter lines (FMWR_EXACT_PREFETCH=0 disables)
+  int nohazard;              // tests only (FMWR_EXACT_NOHAZARD=1): the pipeline does not wait for column hazards
   SolverParams<T> sp;
   double lo, hi;
 };
@@ -423,7 +423,7 @@ __global__ void __launch_bounds__(EX_THREADS, 1) exact_kernel(ExactArgs<T> a)
           if (idx < (uint32_t)RN && j < e2) { pc_col[q] = a.col[j]; pc_val[q] = a.val[j]; }
         }
       }
-      if (a.prefetch && t + 1 < a.t_end) {
+      if (t + 1 < a.t_end) {
         const uint32_t n1 = min(rE[(t + 1) & (RING - 1)] - rB[(t + 1) & (RING - 1)], (uint32_t)RN);
         for (uint32_t i = lane; i < n1; i += 32) {
           const uint32_t c = rCol[(t + 1) & (CRING - 1)][i];
@@ -639,8 +639,7 @@ static void train_exact_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr
   a.tdap_zw_index = (s->compat & FMWR_COMPAT_TDAP_ZW_INDEX) ? 1 : 0;
   a.sp = make_params<T>(m, s);
   a.lo = s->min_target; a.hi = s->max_target;
-  { const char* pf = std::getenv("FMWR_EXACT_PREFETCH"); a.prefetch = (pf && pf[0] == '0') ? 0 : 1; }
-  { const char* nh = std::getenv("FMWR_EXACT_NOHAZARD"); if (nh && nh[0] == '1') a.prefetch |= 2; }     // tests only: run the pipeline WITHOUT waiting for column hazards
+  { const char* nh = std::getenv("FMWR_EXACT_NOHAZARD"); a.nohazard = (nh && nh[0] == '1') ? 1 : 0; }
   bool pipelined = true;
   bool force_pipe = false;
   { const char* pp = std::getenv("FMWR_EXACT_PIPE"); if (pp && pp[0] == '0') pipelined = false; if (pp && pp[0] == '2') force_pipe = true; }

@@ -188,7 +188,6 @@ inline XpPlan xp_plan(int lc /* 16-byte vectors per factor row */, int spw, bool
   // 0.65 us per sample with 8, 0.69 with 12; configs[1] SGD: 0.93 with 8, 0.84 with 12)
   if (avg_nnz * lc < 128.0 && teams > 8) teams = 8;
   if (teams < 1) teams = 1;
-  if (getenv("FMWR_EXACT_TEAMS")) teams = std::max(1, std::min(XP_MAXT, atoi(getenv("FMWR_EXACT_TEAMS"))));
   int ecap = (int)(budget / teams / bpe) / spw * spw;
   if (ecap > XP_RN) ecap = XP_RN / spw * spw;
   pl.teams = teams; pl.ecap = ecap;
@@ -369,32 +368,30 @@ __global__ void __launch_bounds__((XP_MAXT + 3) * 32, 1) exact_pipe_kernel(Exact
 #endif
   } else if (warp == teams + 2) {
     // =========================== hint warp: L2 prefetch of every parameter / state line of the staged samples ===========================
-    if (a.prefetch & 1) {
-      for (uint32_t q = 0; q < total; ++q) {
-        const int slot = q & (XP_R - 1);
-        // a hint for a sample the workers already passed is useless: skip ahead instead of falling behind
-        if (xp_ld(&F.done[slot]) >= q + 1u || xp_ld(&F.loaded[slot]) > q + 1u) continue;
-        { XpSpin sp_; while (xp_ld(&F.fetched[slot]) < q + 1u) sp_.tick("the fetch warp (hints)", q); }
-        __syncwarp();
-        xp_order();
-        if (xp_ld(&F.fetched[slot]) != q + 1u) continue;         // the slot moved on
-        const uint32_t nr = min(F.mN[slot], (uint32_t)XP_RN);
-        for (uint32_t j = lane; j < nr; j += 32) {
-          const uint32_t c = F.rCol[slot][j];
-          const size_t off = (size_t)c * kp;
-          for (int x = 0; x < kp; x += LINE) {
-            prefetch_l2(a.v + off + x);
-            if (has_state) {
+    for (uint32_t q = 0; q < total; ++q) {
+      const int slot = q & (XP_R - 1);
+      // a hint for a sample the workers already passed is useless: skip ahead instead of falling behind
+      if (xp_ld(&F.done[slot]) >= q + 1u || xp_ld(&F.loaded[slot]) > q + 1u) continue;
+      { XpSpin sp_; while (xp_ld(&F.fetched[slot]) < q + 1u) sp_.tick("the fetch warp (hints)", q); }
+      __syncwarp();
+      xp_order();
+      if (xp_ld(&F.fetched[slot]) != q + 1u) continue;         // the slot moved on
+      const uint32_t nr = min(F.mN[slot], (uint32_t)XP_RN);
+      for (uint32_t j = lane; j < nr; j += 32) {
+        const uint32_t c = F.rCol[slot][j];
+        const size_t off = (size_t)c * kp;
+        for (int x = 0; x < kp; x += LINE) {
+          prefetch_l2(a.v + off + x);
+          if (has_state) {
 #pragma unroll
-              for (int s = 0; s < NS; ++s) prefetch_l2(a.sv[s] + off + x);
-            }
+            for (int s = 0; s < NS; ++s) prefetch_l2(a.sv[s] + off + x);
           }
-          if (a.k1) {
-            prefetch_l2(a.w + c);
-            if (has_state) {
+        }
+        if (a.k1) {
+          prefetch_l2(a.w + c);
+          if (has_state) {
 #pragma unroll
-              for (int s = 0; s < NS; ++s) prefetch_l2(a.sw[s] + c);
-            }
+            for (int s = 0; s < NS; ++s) prefetch_l2(a.sw[s] + c);
           }
         }
       }
@@ -442,7 +439,7 @@ __global__ void __launch_bounds__((XP_MAXT + 3) * 32, 1) exact_pipe_kernel(Exact
           if (dd) has_dep |= open_dep(dd & 0xffu) | open_dep((dd >> 8) & 0xffu) | open_dep((dd >> 16) & 0xffu) | open_dep(dd >> 24);
         }
       }
-      has_dep = __any_sync(0xffffffffu, has_dep) && !(a.prefetch & 2);      // bit 1: FMWR_EXACT_NOHAZARD=1, the tests' proof that the tracker matters
+      has_dep = __any_sync(0xffffffffu, has_dep) && !a.nohazard;      // FMWR_EXACT_NOHAZARD=1: the tests' proof that the tracker matters
       // this warp's previous sample publishes its write-back late (below, once its stores have had a forward pass to land);
       // a sample that is about to wait for others publishes it first: the sample it waits for may be that very one
       if (has_dep && pending != 0xffffffffu) {

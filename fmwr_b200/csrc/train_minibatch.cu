@@ -30,7 +30,7 @@ void comm_allreduce_sum(fmwr_ctx* ctx, void* buf, size_t count, bool f64);
 
 // ---- K1: forward + multiplier + S cache --------------------------------------------------------
 template <class T, int LPR, int CH, int TEAM, bool PEERK>
-__global__ void __launch_bounds__(256, FMWR_FWD_BLOCKS)
+__global__ void __launch_bounds__(256, FWD_BLOCKS)
 mb_forward_kernel(const uint32_t* __restrict__ rowptr, const uint32_t* __restrict__ col, const float* __restrict__ val,
                   const float* __restrict__ y, const T* __restrict__ w, const T* __restrict__ v,
                   const double* __restrict__ scal, int kp, int k0, int k1, int task, T lo, T hi,
@@ -212,13 +212,7 @@ struct MbUpdArgs {
   PeerArgs pa;
 };
 
-#ifndef FMWR_K2B
-#define FMWR_K2B 5
-#endif
-#ifndef FMWR_K2UE
-#define FMWR_K2UE 2
-#endif
-template <int SOLVER> struct K2Tune { enum { BLOCKS = SOLVER == FMWR_TDAP ? 3 : FMWR_K2B, UE = SOLVER == FMWR_TDAP ? 4 : FMWR_K2UE }; };
+template <int SOLVER> struct K2Tune { enum { BLOCKS = SOLVER == FMWR_TDAP ? 3 : 5, UE = SOLVER == FMWR_TDAP ? 4 : 2 }; };
 
 // the intercept (dense coordinate): fixed-order reduction of the batch's multipliers by ONE block.  It is block 0 so
 // that its serial chain of loads overlaps the rest of the grid instead of forming the kernel's tail.
@@ -477,7 +471,7 @@ __global__ void __launch_bounds__(256, (sizeof(T) == 4 && CH == 1) ? K2Tune<SOLV
   const int lane = threadIdx.x & 31;
   const int g = lane / LPR, l = lane % LPR;
   // grid-stride over the batch's segments: with a grid of (resident CTAs) the warps stay on the SM for the whole launch
-  // instead of being re-created every 4 segments (FMWR_K2_ONESHOT=1 launches one group per segment as before)
+  // instead of being re-created every 4 segments
   const uint32_t stride = (gridDim.x - 1) * (blockDim.x >> 5) * G;
   for (uint32_t seg = a.seg_begin + ((blockIdx.x - 1) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * G + g; seg < a.seg_end; seg += stride) {
     const uint4 rec = __ldg(a.seg_rec + seg);
@@ -494,7 +488,7 @@ namespace fmwr {
 
 // ---- K2, dense variant (update_tma.cuh): producer warp + 8 consumer warps over a ring of TMA-filled stages ----------------
 template <class T, int LPR, int CH, int SOLVER, bool L1, int TS, int NS, int MINB>
-__global__ void __launch_bounds__(TM_THREADS, MINB) mb_update_tma_kernel(MbUpdArgs<T> a, int hint)
+__global__ void __launch_bounds__(TM_THREADS, MINB) mb_update_tma_kernel(MbUpdArgs<T> a)
 {
   typedef TmGeom<T, LPR, CH, SOLVER, L1, TS, NS> G;
   constexpr int GRP = 32 / LPR;                         // lane groups (segments) per warp
@@ -519,8 +513,7 @@ __global__ void __launch_bounds__(TM_THREADS, MINB) mb_update_tma_kernel(MbUpdAr
   if (warp == TM_CONS_WARPS) {
     // ================================ producer: loads and write-backs, lane 0 only =================================
     if (lane != 0) return;
-    const uint64_t pol_th = l2_policy(hint ? 2 : 0);     // theta rows are re-read by the next batch's forward: keep
-    const uint64_t pol_st = l2_policy(hint ? 1 : 0);     // optimizer state and the batch's lists are touched once per batch: stream
+    const uint64_t pol = l2_policy();
     uint32_t wb_c0[NS], wb_rows[NS];                      // pending write-back of each stage (rows == 0: none)
 #pragma unroll
     for (int s = 0; s < NS; ++s) { wb_c0[s] = 0u; wb_rows[s] = 0u; }
@@ -529,11 +522,11 @@ __global__ void __launch_bounds__(TM_THREADS, MINB) mb_update_tma_kernel(MbUpdAr
       const uint32_t c0 = wb_c0[s], nr = wb_rows[s];
       if (nr) {
         const uint32_t bytes = nr * G::ROWB;
-        bulk_s2g(reinterpret_cast<unsigned char*>(a.v) + (size_t)c0 * G::ROWB, smem_u32(st + G::OFF_PAR), bytes, pol_th);
+        bulk_s2g(reinterpret_cast<unsigned char*>(a.v) + (size_t)c0 * G::ROWB, smem_u32(st + G::OFF_PAR), bytes, pol);
         if (G::USE_STATE) {
 #pragma unroll
           for (int i = 0; i < NSTW; ++i)
-            bulk_s2g(reinterpret_cast<unsigned char*>(a.sv[i]) + (size_t)c0 * G::ROWB, smem_u32(st + G::OFF_PAR + (i + 1) * G::RMAX * G::ROWB), bytes, pol_st);
+            bulk_s2g(reinterpret_cast<unsigned char*>(a.sv[i]) + (size_t)c0 * G::ROWB, smem_u32(st + G::OFF_PAR + (i + 1) * G::RMAX * G::ROWB), bytes, pol);
         }
         bulk_commit();
         bulk_wait_read0();                                 // the stage may be refilled once the stores have READ it
@@ -572,33 +565,33 @@ __global__ void __launch_bounds__(TM_THREADS, MINB) mb_update_tma_kernel(MbUpdAr
       hdr[0] = dense ? 1u : 0u; hdr[1] = c0; hdr[2] = nrows; hdr[3] = s0 - s0a; hdr[4] = e0; hdr[5] = e0 - e0a; hdr[6] = c0 - c0a; hdr[7] = ns;
       const uint32_t full = smem_u32(bars + s);
       uint32_t tx = ns * 16u + nsp * 4u;
-      bulk_g2s(smem_u32(st + G::OFF_REC), a.seg_rec + s0, ns * 16u, full, pol_st);
-      bulk_g2s(smem_u32(st + G::OFF_SEGP), a.seg_ptr + s0a, nsp * 4u, full, pol_st);
+      bulk_g2s(smem_u32(st + G::OFF_REC), a.seg_rec + s0, ns * 16u, full, pol);
+      bulk_g2s(smem_u32(st + G::OFF_SEGP), a.seg_ptr + s0a, nsp * 4u, full, pol);
       wb_rows[s] = 0u;
       if (dense) {
         if (nen) {
-          bulk_g2s(smem_u32(st + G::OFF_EROW), a.ent_row + e0a, nen * 4u, full, pol_st);
-          bulk_g2s(smem_u32(st + G::OFF_EVAL), a.ent_val + e0a, nen * 4u, full, pol_st);
+          bulk_g2s(smem_u32(st + G::OFF_EROW), a.ent_row + e0a, nen * 4u, full, pol);
+          bulk_g2s(smem_u32(st + G::OFF_EVAL), a.ent_val + e0a, nen * 4u, full, pol);
           tx += 2u * nen * 4u;
         }
         const uint32_t pbytes = nrows * G::ROWB;
-        bulk_g2s(smem_u32(st + G::OFF_PAR), reinterpret_cast<const unsigned char*>(a.v) + (size_t)c0 * G::ROWB, pbytes, full, pol_th);
+        bulk_g2s(smem_u32(st + G::OFF_PAR), reinterpret_cast<const unsigned char*>(a.v) + (size_t)c0 * G::ROWB, pbytes, full, pol);
         tx += pbytes;
         if (G::USE_STATE) {
 #pragma unroll
           for (int k = 0; k < NSTW; ++k) {
-            bulk_g2s(smem_u32(st + G::OFF_PAR + (k + 1) * G::RMAX * G::ROWB), reinterpret_cast<const unsigned char*>(a.sv[k]) + (size_t)c0 * G::ROWB, pbytes, full, pol_st);
+            bulk_g2s(smem_u32(st + G::OFF_PAR + (k + 1) * G::RMAX * G::ROWB), reinterpret_cast<const unsigned char*>(a.sv[k]) + (size_t)c0 * G::ROWB, pbytes, full, pol);
             tx += pbytes;
           }
         }
         if (a.k1) {
           const uint32_t wbytes = nw * (uint32_t)sizeof(T);
-          bulk_g2s(smem_u32(st + G::OFF_W), a.w + c0a, wbytes, full, pol_th);
+          bulk_g2s(smem_u32(st + G::OFF_W), a.w + c0a, wbytes, full, pol);
           tx += wbytes;
           if (G::USE_STATE) {
 #pragma unroll
             for (int k = 0; k < NSTW; ++k) {
-              bulk_g2s(smem_u32(st + G::OFF_W + (k + 1) * (G::RMAX + 8) * (int)sizeof(T)), a.sw[k] + c0a, wbytes, full, pol_st);
+              bulk_g2s(smem_u32(st + G::OFF_W + (k + 1) * (G::RMAX + 8) * (int)sizeof(T)), a.sw[k] + c0a, wbytes, full, pol);
               tx += wbytes;
             }
           }
@@ -676,11 +669,9 @@ struct MbLaunch {
       FMWR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, mb_update_tma_kernel<TT, LPR, CH, SOLVER, L1, TS, NS, MINB>, TM_THREADS, (size_t)G::SMEM_BYTES));
       occ = o < 1 ? 1 : o;
     }
-    const int hint = getenv("FMWR_K2_HINT") ? atoi(getenv("FMWR_K2_HINT")) : 0;
-    const int ctas = getenv("FMWR_K2_CTAS") ? atoi(getenv("FMWR_K2_CTAS")) : 0;
     const int64_t n_tiles = ceil_div64((int64_t)nseg, TS);
-    const int grid = (int)std::min<int64_t>(n_tiles, (int64_t)ctx->sm_count * (ctas > 0 ? std::min(ctas, occ) : occ)) + 1;     // +1: the intercept block
-    FMWR_LAUNCH(ctx, (mb_update_tma_kernel<TT, LPR, CH, SOLVER, L1, TS, NS, MINB>), grid, TM_THREADS, (size_t)G::SMEM_BYTES, ua, hint);
+    const int grid = (int)std::min<int64_t>(n_tiles, (int64_t)ctx->sm_count * occ) + 1;     // +1: the intercept block
+    FMWR_LAUNCH(ctx, (mb_update_tma_kernel<TT, LPR, CH, SOLVER, L1, TS, NS, MINB>), grid, TM_THREADS, (size_t)G::SMEM_BYTES, ua);
   }
   template <class TT, int LPR, int CH>
   void tma(uint32_t nseg)
@@ -690,15 +681,11 @@ struct MbLaunch {
         if (ua.sp.l1) tma_launch<TT, LPR, CH, FMWR_SGD, true, 32, 3, 3>(nseg);
         else tma_launch<TT, LPR, CH, FMWR_SGD, false, 32, 3, 3>(nseg);
         break;
-      case FMWR_FTRL: {
-        const int var = getenv("FMWR_K2_VAR") ? atoi(getenv("FMWR_K2_VAR")) : 0;
+      case FMWR_FTRL:
         // measured on configs[1] (profiles/r02_summary.md): 32-segment tiles, 3 stages, 3 CTAs/SM 168 us per batch; 2 stages 180;
         // 4 CTAs/SM (56 registers, spills) 204; 64-segment tiles x 2 stages x 2 CTAs 184; the gather kernel 178
-        if (var == 1) tma_launch<TT, LPR, CH, FMWR_FTRL, false, 32, 4, 2>(nseg);
-        else if (var == 2) tma_launch<TT, LPR, CH, FMWR_FTRL, false, 16, 4, 3>(nseg);
-        else tma_launch<TT, LPR, CH, FMWR_FTRL, false, 32, 3, 3>(nseg);
+        tma_launch<TT, LPR, CH, FMWR_FTRL, false, 32, 3, 3>(nseg);
         break;
-      }
       default: tma_launch<TT, LPR, CH, FMWR_TDAP, false, 32, 2, 2>(nseg); break;
     }
   }
@@ -720,16 +707,18 @@ struct MbLaunch {
       constexpr int G = 32 / LPR;
       const uint32_t nseg = ua.seg_end - ua.seg_begin;
       int grid = ceil_div((int64_t)nseg, 8 * G) + 1;       // +1: the intercept block
-      {
-        static const int persist = getenv("FMWR_K2_ONESHOT") ? 0 : (getenv("FMWR_K2_WAVES") ? atoi(getenv("FMWR_K2_WAVES")) : 1);
-        const int resident = (sizeof(TT) == 4 && CH == 1) ? (s->solver == FMWR_TDAP ? 3 : FMWR_K2B) : 2;
-        // feature-parallel ranks hold a fraction of the segments: there the one-shot grid measured faster (N = 2/4/8)
-        if (persist > 0 && !(ctx->nccl_comm && ctx->world > 1)) grid = std::min(grid, ctx->sm_count * resident * persist + 1);
+      // one wave of resident CTAs; feature-parallel ranks hold a fraction of the segments: there the one-shot grid measured
+      // faster (N = 2/4/8)
+      if (!(ctx->nccl_comm && ctx->world > 1)) {
+        const int resident = (sizeof(TT) == 4 && CH == 1) ? (s->solver == FMWR_TDAP ? K2Tune<FMWR_TDAP>::BLOCKS : K2Tune<FMWR_SGD>::BLOCKS) : 2;
+        grid = std::min(grid, ctx->sm_count * resident + 1);
       }
       // dense variant (update_tma.cuh): fp32, one 16-byte vector per lane, rows of at most 128 bytes; FMWR_K2_GATHER=1 keeps the
       // original gather kernel for every tile
-      const bool no_tma = getenv("FMWR_K2_GATHER") != nullptr;     // read per launch: tests flip it between calls
-      if (sizeof(TT) == 4 && CH == 1 && LPR <= 8 && !no_tma) { tma<TT, (LPR <= 8 ? LPR : 8), (CH == 1 ? CH : 1)>(nseg); return; }
+      if constexpr (sizeof(TT) == 4 && CH == 1 && LPR <= 8) {
+        const bool no_tma = getenv("FMWR_K2_GATHER") != nullptr;     // read per launch: tests flip it between calls
+        if (!no_tma) { tma<TT, LPR, CH>(nseg); return; }
+      }
       switch (s->solver) {
         case FMWR_SGD:
           if (ua.sp.l1) FMWR_LAUNCH(ctx, (mb_update_kernel<TT, LPR, CH, FMWR_SGD, true>), grid, 256, 0, ua);
@@ -747,9 +736,9 @@ template <class TT, int LPR, int CH, int TEAM>
 void MbLaunch<T>::k1()
 {
   const int rpb = 8 * (32 / TEAM);
-  // peer mode: one release fence per CTA at the end (it waits for the CTA's NVLink stores), so few fat CTAs
-  static const int k1_ctas = getenv("FMWR_K1_CTAS") ? atoi(getenv("FMWR_K1_CTAS")) : 4;      // resident CTAs per SM: measured best (persistent warps)
-  const int fgrid = (int)std::min<int64_t>(ceil_div(rows, rpb), (int64_t)ctx->sm_count * (partial == 2 ? 4 : k1_ctas));
+  // 4 resident CTAs per SM: measured best (persistent warps); peer mode wants few fat CTAs too, because each CTA ends with one
+  // release fence that waits for its NVLink stores
+  const int fgrid = (int)std::min<int64_t>(ceil_div(rows, rpb), (int64_t)ctx->sm_count * 4);
   // (the peer-window variant is a separate instantiation: indexing the window table by owner costs every thread a stack frame)
   if (partial == 2)
     FMWR_LAUNCH(ctx, (mb_forward_kernel<TT, LPR, CH, TEAM, true>), fgrid, 256, 0, d->rowptr.p, d->col.p, d->val.p, d->y.p,
@@ -850,7 +839,7 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
   const bool multi = ctx->nccl_comm != nullptr && ctx->world > 1;
   const int s_stride = multi ? m->kp + 4 : m->kp;
   // peer window open: the exchange runs inside our own kernels (NVLink stores + flags), no NCCL call per batch
-  const bool peer = multi && ctx->peer.ready && getenv("FMWR_NO_PEER") == nullptr;
+  const bool peer = multi && ctx->peer.ready;
   PeerArgs pa;
   memset(&pa, 0, sizeof pa);
   DBuf<T> mult, Scache;
@@ -882,7 +871,7 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
   ua.mult = mult_p; ua.Scache = sc_p;
   ua.peer = peer ? 1 : 0; ua.pa = pa; ua.mult_stride = peer ? s_stride : 1;
   // fp32 models with 32-float rows on long rows: the stream forward kernel runs the exchange itself
-  const bool fused_exchange = peer && sizeof(T) == 4 && stream_forward_ok(m, d->nnz, d->n, 2) && getenv("FMWR_NO_FUSED_EXCHANGE") == nullptr;
+  const bool fused_exchange = peer && sizeof(T) == 4 && stream_forward_ok(m, d->nnz, d->n, 2);
   if (fused_exchange) { ua.msum = reinterpret_cast<const double*>(pa.base[pa.rank] + pa.off_msum); ua.msum_n = ctx->world; }
   else if (peer) ua.mult_compact = reinterpret_cast<const T*>(pa.base[pa.rank] + pa.off_mult);
   L.fused_exchange = fused_exchange;
