@@ -401,3 +401,12 @@ def train_dev(ctx, model, data, scfg, trace=None, keep=()):
     """keep: numpy arrays referenced by pointer fields of scfg (kept alive for the call)"""
     check(lib().fmwr_train_dev(ctx.h, model.h, data.h, C.byref(scfg), C.byref(trace.c) if trace is not None else None))
     del keep
+
+
+def train_posterior_dev(ctx, model, data, scfg, burn_in, evals=(), trace=None, keep=()):
+    """train_dev plus the MCMC posterior mean of draws burn_in+1 .. max_iter: afterwards predict_fetch(ctx, data) and
+    predict_fetch(ctx, e) for every e in evals return the means (an entry of None passes a null handle)"""
+    arr = (C.c_void_p * max(len(evals), 1))(*[e.h if e is not None else None for e in evals])
+    check(lib().fmwr_train_posterior_dev(ctx.h, model.h, data.h, C.byref(scfg), C.byref(trace.c) if trace is not None else None,
+                                         C.c_int32(burn_in), arr if len(evals) else None, C.c_int32(len(evals))))
+    del keep

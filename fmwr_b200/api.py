@@ -268,14 +268,16 @@ def _model_cfg(mc):
                       l2_v=float(hp["L2.v"]))
 
 
-def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_list, streams=None):
-    """body of FM() (reference src/FM.cpp:7-174) on top of the C ABI"""
+def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_list, streams=None, posterior=None):
+    """body of FM() (reference src/FM.cpp:7-174) on top of the C ABI.  posterior (fm_posterior): dict(burn_in, newdata) in, and
+    the device means out as posterior["train"] and posterior["newdata_mean"]"""
     ctx = _ctx()
     feats = data["features"]
     n, p = feats["dim"]
     labels = data["labels"]
     normalize0 = np.atleast_1d(np.asarray(normalize0, np.int64))
     d, parked = _acquire(ctx, feats, labels, normalize0[0] > -1)
+    evals = []                                                            # (handle, parked) of posterior["newdata"]
     try:
         scales = {}
         if normalize0[0] > -1:                                            # FM.cpp:36-38
@@ -328,7 +330,16 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
                 from math import ceil
                 nrec = min(10001, int(ceil((sc.max_iter - 0.5) / sc.step_size)) + 2)
                 trace = L.TraceBuf(nrec, p, k, snapshots=True)
-            L.train_dev(ctx, m, d, sc, trace, keep=keep)
+            if posterior is None:
+                L.train_dev(ctx, m, d, sc, trace, keep=keep)
+            else:
+                for nd in posterior["newdata"]:                           # checked and z-scored as predict does it
+                    evals.append(_acquire(ctx, nd["features"], None, normalize0[0] > -1))
+                    if normalize0[0] > -1:
+                        evals[-1][0].normalize(scales["mean"], scales["std"])
+                L.train_posterior_dev(ctx, m, d, sc, posterior["burn_in"], [e for e, _ in evals], trace, keep=keep)
+                posterior["train"] = L.predict_fetch(ctx, d)
+                posterior["newdata_mean"] = [L.predict_fetch(ctx, e) for e, _ in evals]
             gw0, gw, gv = m.get()
             state = m.get_state() if (_OPTIONS["FM.keep_state"] and name in ("SGD", "FTRL", "TDAP")) else None
         finally:
@@ -336,6 +347,9 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
     finally:
         if not parked:
             d.close()
+        for e, e_parked in evals:
+            if not e_parked:
+                e.close()
     model = dict(w0=gw0, w=gw, v=gv.T.copy())                              # v returned k x p like Model::save_model
     model["model.control"] = fm_controls
     model["solver.control"] = solver_controls
@@ -356,6 +370,13 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
 
 def fm_train(data, normalize=True, control=None, _streams=None):
     """R/fm_train.R:70-127"""
+    data, norm, ctl = _train_setup(data, normalize, control)
+    return _FM(data, norm - 1, ctl["model"], ctl["solver"], ctl["track"], None, streams=_streams)
+
+
+def _train_setup(data, normalize, control):
+    """argument checks and controls of fm.train (R/fm_train.R:70-125): (data with recoded labels, 1-based columns to normalize
+    or [-1], controls)"""
     if data.get("labels") is None:
         raise ValueError("there are no labels in data")
     ncol = data.ncol()
@@ -387,7 +408,35 @@ def fm_train(data, normalize=True, control=None, _streams=None):
             data = FmMatrix(features=data["features"], labels=np.where(data["labels"] < 1, -1.0, 1.0))
         elif not np.array_equal(u, [-1, 1]):
             raise ValueError("target should be c(0, 1) or c(-1, 1)")
-    return _FM(data, norm - 1, ctl["model"], ctl["solver"], ctl["track"], None, streams=_streams)
+    return data, norm, ctl
+
+
+def fm_posterior(data, newdata=(), burn_in=0, normalize=True, control=None):
+    """Engine extension: the MCMC posterior mean libFM predicts with.  Trains exactly as fm_train(data, normalize, control) and
+    also averages, on the device, the predict.FM prediction of draws burn_in+1 .. max_iter (draw t = the model after sweep t)
+    on data and on every newdata (fm.matrix objects of the same width, z-scored with the training scales as predict does).
+    Returns dict(fit=<what fm_train returns>, train=<mean on data>, newdata=[<mean per newdata>])."""
+    if isinstance(newdata, FmMatrix):
+        newdata = [newdata]
+    newdata = list(newdata)
+    data, norm, ctl = _train_setup(data, normalize, control)
+    if ctl["solver"]["solver"].solver != "MCMC":
+        raise ValueError("posterior averaging needs the MCMC solver")
+    max_iter = int(ctl["solver"]["max_iter"])
+    if int(burn_in) != burn_in or not 0 <= burn_in < max_iter:
+        raise ValueError("burn_in must be an integer in [0, max_iter) = [0, %d)" % max_iter)
+    for i, nd in enumerate(newdata):
+        if not isinstance(nd, FmMatrix):
+            raise ValueError("newdata must be fm.matrix objects")
+        if np.isnan(nd["features"]["value"]).any():
+            raise ValueError("there are NAs in newdata")
+        if nd["features"] is data["features"]:
+            raise ValueError("newdata is the training data: its mean is returned as train")
+        if any(nd["features"] is o["features"] for o in newdata[:i]):
+            raise ValueError("the same newdata appears twice")
+    post = dict(burn_in=int(burn_in), newdata=newdata)
+    fit = _FM(data, norm - 1, ctl["model"], ctl["solver"], ctl["track"], None, posterior=post)
+    return dict(fit=fit, train=post["train"], newdata=post["newdata_mean"])
 
 
 def _link_for(model):

@@ -284,7 +284,8 @@ static void fetch_pred(fmwr_ctx* ctx, fmwr_data* d, double* out)
   }
 }
 
-static void train_dispatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr)
+static void train_dispatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr,
+                           const Posterior* post = nullptr)
 {
   FMWR_REQUIRE(d->has_labels, FMWR_ERR_ARG, "target's length is not equal the number of cases...");
   FMWR_REQUIRE(d->p == m->p, FMWR_ERR_SHAPE, "there's no the same number of features between train and fm object...");
@@ -295,7 +296,7 @@ static void train_dispatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmw
       else train_exact(ctx, m, d, s, tr);
       break;
     case FMWR_ALS: case FMWR_MCMC:
-      train_als_mcmc(ctx, m, d, s, tr);
+      train_als_mcmc(ctx, m, d, s, tr, post);
       break;
     default: throw Error(FMWR_ERR_ARG, "Unknown solver...");   // reference src/FM.cpp:85
   }
@@ -763,6 +764,27 @@ int fmwr_train_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver
     FMWR_REQUIRE(ctx && m && d && s, FMWR_ERR_ARG, "null argument");
     FMWR_CUDA(cudaSetDevice(ctx->device));
     train_dispatch(ctx, m, d, s, trace);
+  });
+}
+
+int fmwr_train_posterior_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* trace,
+                             int32_t burn_in, fmwr_data* const* eval, int32_t n_eval)
+{
+  return guarded([&] {
+    FMWR_REQUIRE(ctx && m && d && s, FMWR_ERR_ARG, "null argument");
+    FMWR_REQUIRE(n_eval >= 0 && (n_eval == 0 || eval), FMWR_ERR_ARG, "null eval list");
+    FMWR_REQUIRE(s->solver == FMWR_MCMC, FMWR_ERR_ARG, "posterior averaging needs the MCMC solver");
+    FMWR_REQUIRE(burn_in >= 0 && burn_in < s->max_iter, FMWR_ERR_ARG, "burn_in must be at least 0 and less than max_iter");
+    for (int i = 0; i < n_eval; ++i) {
+      FMWR_REQUIRE(eval[i], FMWR_ERR_ARG, "null eval data");
+      FMWR_REQUIRE(eval[i] != d, FMWR_ERR_ARG, "an eval set is the training data (its mean is the training rows' result)");
+      for (int j = 0; j < i; ++j) FMWR_REQUIRE(eval[j] != eval[i], FMWR_ERR_ARG, "an eval set appears twice");
+    }
+    for (int i = 0; i < n_eval; ++i) require_same_features(m, eval[i]);
+    FMWR_REQUIRE(!(ctx->nccl_comm && ctx->world > 1), FMWR_ERR_UNSUPPORTED, "posterior averaging runs on one GPU (row-sharded data is not supported)");
+    FMWR_CUDA(cudaSetDevice(ctx->device));
+    const Posterior post{burn_in, eval, n_eval};
+    train_dispatch(ctx, m, d, s, trace, &post);
   });
 }
 

@@ -427,7 +427,18 @@ int64_t minibatch_entries(const fmwr_data* d);          // entries of the per-ba
 bool minibatch_streams_values(const fmwr_solver_cfg* s);   // train_minibatch may start on data whose values are still uploading
 void train_exact(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr);
 void train_minibatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr);
-void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr);
+// MCMC posterior mean (fmwr_train_posterior_dev): average the predict.FM prediction of draws burn_in+1 .. max_iter on the
+// training rows and on every eval set (validated by the caller: distinct, not the training data, same feature count)
+struct Posterior {
+  int burn_in;
+  fmwr_data* const* eval; int n_eval;
+};
+void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Posterior* post = nullptr);
+// shape check of Model::predict_batch (reference src/core/Model.h:112-113)
+inline void require_same_features(const fmwr_model* m, const fmwr_data* d)
+{
+  FMWR_REQUIRE(d->p == m->p, FMWR_ERR_SHAPE, "number of input's features is not correct...");
+}
 double evaluate_dev(fmwr_ctx* ctx, fmwr_data* d, int task, int metric);
 bool model_alloc_state(fmwr_model* m, int n_state, int solver, bool warm);
 void model_get_host(fmwr_model* m, double* w0, double* w, double* v);

@@ -71,8 +71,7 @@ struct FwdLaunch {
 
 void forward_launch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, int link, double lo, double hi)
 {
-  // shape checks of Model::predict_batch (reference src/core/Model.h:112-113)
-  FMWR_REQUIRE(d->p == m->p, FMWR_ERR_SHAPE, "number of input's features is not correct...");
+  require_same_features(m, d);
   if (d->n == 0) return;
   if (stream_forward_ok(m, d->nnz, d->n)) {
     // fp32, 32-float factor rows, long rows: the software-pipelined stream kernel (forward_stream.cuh) + elementwise link

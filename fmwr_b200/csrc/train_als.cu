@@ -216,6 +216,28 @@ __global__ void als_error_stream_kernel(T* __restrict__ e, const float* __restri
   }
 }
 
+// ---- posterior mean (fmwr_train_posterior_dev) -------------------------------------------------------------------------
+// One draw: acc[i] += link(score[i]) in f64, launched once per draw in draw order.  A kernel of its own rather than an
+// accumulating variant of the error kernels: the eval sets need the same step on their forward results, and the kernels
+// that drive the chain stay exactly as they are.  On the training rows it costs 4 bytes more per row (the score is read
+// again) than a fused variant would, against ~146 GB of coordinate-pass traffic per sweep on the benchmark shape.
+template <class S>
+__global__ void posterior_accum_kernel(const S* __restrict__ score, int64_t n, int link, double lo, double hi,
+                                       const double* __restrict__ pnY, double* __restrict__ acc)
+{
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) acc[i] += apply_link(link, (double)score[i], lo, hi, pnY);
+}
+
+// out[perm[i]] = acc[i] / draws (perm == nullptr: out[i]); a division, so that a host summing the same predictions in the
+// same order gets the same bits
+__global__ void posterior_mean_kernel(const double* __restrict__ acc, int64_t n, double draws, const uint32_t* __restrict__ perm,
+                                      double* __restrict__ out)
+{
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[perm ? (int64_t)perm[i] : i] = acc[i] / draws;
+}
+
 // ---- reductions ------------------------------------------------------------------------------------------
 // mode 0: sum x, 1: sum x^2, 2: sum (x - c)^2
 template <class T>
@@ -949,6 +971,7 @@ struct DenseLayout {
   DBuf<uint32_t> pcol;   // [n][np] CSR columns of the permuted rows (global ids) for the forward pass
   DBuf<float> pval;      // [n][np]
   DBuf<float> py;        // [n] labels of the permuted rows
+  DBuf<uint32_t> perm;   // [n] original row of permuted row i (the posterior mean un-permutes its row sums with it)
 };
 
 __global__ void dense_check_kernel(const uint32_t* __restrict__ rowptr, const uint32_t* __restrict__ col, int64_t n, int np,
@@ -1020,7 +1043,7 @@ static void build_dense(fmwr_data* d, const std::vector<uint32_t>& pbeg_host, De
   // widest phase: if it does not fit the shared-memory table, sort the rows by its feature
   int jstar = 0;
   for (int j = 1; j < np; ++j) if (pbeg_host[j + 1] - pbeg_host[j] > pbeg_host[jstar + 1] - pbeg_host[jstar]) jstar = j;
-  DBuf<uint32_t> perm;
+  DBuf<uint32_t>& perm = dl.perm;
   dl.permuted = false; dl.sorted_phase = -1;
   if (allow_perm && pbeg_host[jstar + 1] - pbeg_host[jstar] > (uint32_t)RM_SMEM_COLS && d->has_labels) {
     DBuf<uint32_t> key_in, key_out, idx_in;
@@ -1281,7 +1304,7 @@ struct HostStreams {
 static inline bool hbad(double x) { return std::isnan(x) || std::isinf(x); }
 
 template <class T>
-static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr)
+static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Posterior* post)
 {
   const int64_t n = d->n, p = d->p;
   const int k = m->k, kp = m->kp;
@@ -1379,6 +1402,31 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
   double alpha = 1.0, w_mu = 0.0, w_lambda = 0.0;
   std::vector<double> v_mu(std::max(k, 1), 0.0), v_lambda(std::max(k, 1), 0.0);
 
+  // posterior mean: f64 sums of the predict.FM prediction of every averaged draw (the MCMC link of tracker_score) -- the
+  // training rows in the order e has, then each eval set.  Draw t is the model after t sweeps: at sweep t, right after the
+  // forward, e holds its raw score; the eval sets get a predict of their own.  None of it feeds back into the chain.
+  const int post_link = cls ? FMWR_LINK_PROBIT_TABLE : FMWR_LINK_CLAMP;
+  DBuf<double> post_acc;
+  std::vector<int64_t> post_off;           // [n_eval + 2] offsets into post_acc
+  if (post) {
+    post_off = {0, n};
+    for (int i = 0; i < post->n_eval; ++i) post_off.push_back(post_off.back() + post->eval[i]->n);
+    post_acc.alloc(post_off.back());
+    post_acc.zero(ctx->stream);
+  }
+  auto post_draw = [&]() {
+    if (n > 0)
+      FMWR_LAUNCH(ctx, posterior_accum_kernel<T>, ceil_div(n, 256), 256, 0, e.p, n, post_link, s->min_target, s->max_target,
+                  ctx->pn_table.p, post_acc.p);
+    for (int i = 0; i < post->n_eval; ++i) {
+      fmwr_data* ev = post->eval[i];
+      if (ev->n == 0) continue;
+      forward_launch(ctx, m, ev, FMWR_LINK_NONE, 0.0, 0.0);
+      FMWR_LAUNCH(ctx, posterior_accum_kernel<double>, ceil_div(ev->n, 256), 256, 0, ev->pred64.p, ev->n, post_link, s->min_target,
+                  s->max_target, ctx->pn_table.p, post_acc.p + post_off[i + 1]);
+    }
+  };
+
   T* wp = (T*)m->w.p;
   T* vp = (T*)m->v.p;
   double* scal = (double*)m->scal.p;
@@ -1401,6 +1449,7 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
     const float* yp = perm_rows ? dl.py.p : d->y.p;
     AlsFwd<T> fw{ctx, m, d, e.p, enable_v ? q.p : nullptr, perm_rows ? dl.pcol.p : d->col.p, perm_rows ? dl.pval.p : d->val.p};
     dispatch_layout<T>(kp, fw);
+    if (post && sweep > post->burn_in) post_draw();
     // calculate_error (:520-562)
     if (!cls) {
       FMWR_LAUNCH(ctx, als_error_kernel<T>, ceil_div(n, 256), 256, 0, e.p, yp, n, 0, ctx->dp_table.p, s->seed, (uint64_t)sweep, (uint64_t)row_off);
@@ -1516,6 +1565,22 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
       }
     }
   }
+  if (post) {
+    // the last draw is the returned model: one more forward (scores only) for the training rows
+    const bool perm_rows = use_rm && dl.ok && dl.permuted;
+    AlsFwd<T> fw{ctx, m, d, e.p, nullptr, perm_rows ? dl.pcol.p : d->col.p, perm_rows ? dl.pval.p : d->val.p};
+    dispatch_layout<T>(kp, fw);
+    post_draw();
+    const double draws = (double)(s->max_iter - post->burn_in);
+    for (int i = -1; i < post->n_eval; ++i) {
+      fmwr_data* dd = i < 0 ? d : post->eval[i];
+      if (dd->n == 0) continue;
+      dd->pred64.ensure(dd->n);
+      FMWR_LAUNCH(ctx, posterior_mean_kernel, ceil_div(dd->n, 256), 256, 0, post_acc.p + post_off[i + 1], dd->n, draws,
+                  (i < 0 && perm_rows) ? dl.perm.p : nullptr, dd->pred64.p);
+      dd->pred_prec = FMWR_F64;
+    }
+  }
   FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
   if (ctx->world > 1) peer_check_error(ctx);      // a timed-out exchange means partial (A,B) sums: the replicas have diverged
   if (tr) { tr->n_rec = std::min(n_rec, (int)tr->max_rec); tr->convergent = 0; tr->iters_done = sweep; }
@@ -1579,11 +1644,11 @@ int als_effective_precision(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fm
   return has_thin_columns(ctx, d) ? FMWR_F64 : FMWR_F32;
 }
 
-void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr)
+void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Posterior* post)
 {
-  if (m->prec == FMWR_F64) { train_als_t<double>(ctx, m, d, s, tr); return; }
-  if (als_effective_precision(ctx, m, d, s) == FMWR_F32) { train_als_t<float>(ctx, m, d, s, tr); return; }
-  // fp64 shadow of the fp32 handle
+  if (m->prec == FMWR_F64) { train_als_t<double>(ctx, m, d, s, tr, post); return; }
+  if (als_effective_precision(ctx, m, d, s) == FMWR_F32) { train_als_t<float>(ctx, m, d, s, tr, post); return; }
+  // fp64 shadow of the fp32 handle (a posterior mean averages the shadow's draws)
   fmwr_model* sh = nullptr;
   FMWR_REQUIRE(fmwr_model_create(ctx, &m->cfg, m->p, FMWR_F64, &sh) == 0, FMWR_ERR_CUDA, fmwr_last_error());
   try {
@@ -1593,7 +1658,7 @@ void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solve
       FMWR_LAUNCH(ctx, (repack_rows_kernel<float, double>), ceil_div(p, 256), 256, 0, (const float*)m->w.p, 1, (double*)sh->w.p, 1, p, 1);
       FMWR_LAUNCH(ctx, (repack_rows_kernel<float, double>), ceil_div(p * sh->kp, 256), 256, 0, (const float*)m->v.p, m->kp, (double*)sh->v.p, sh->kp, p, m->k);
     }
-    train_als_t<double>(ctx, sh, d, s, tr);
+    train_als_t<double>(ctx, sh, d, s, tr, post);
     FMWR_CUDA(cudaMemcpyAsync(m->scal.p, sh->scal.p, 8 * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
     if (p > 0) {
       FMWR_LAUNCH(ctx, (repack_rows_kernel<double, float>), ceil_div(p, 256), 256, 0, (const double*)sh->w.p, 1, (float*)m->w.p, 1, p, 1);

@@ -221,6 +221,17 @@ int fmwr_evaluate_dev(fmwr_ctx* ctx, fmwr_data* d, int32_t task, int32_t metric,
 
 /* ---- training: replaces Learner::init + learn (src/core/Learner.h:49-51 and src/solver/*_Learner.h) ---- */
 int fmwr_train_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* trace /* nullable */);
+/* MCMC posterior mean (extension: the reference returns the last draw only, MCMC_ALS_Learner.h:98-127).  Runs exactly the
+ * sweeps fmwr_train_dev(ctx, m, d, s, trace) runs and, in addition, averages the predict.FM prediction of draws
+ * burn_in+1 .. s->max_iter on d and on every eval[i].  On return each of those handles holds the mean as its forward result
+ * (fmwr_predict_fetch / fmwr_evaluate_dev read it).  eval sets need no labels.
+ * Draw t is the model after sweep t; the prediction is the one tracker scores use (regression: clamped to
+ * [s->min_target, s->max_target]; classification: the fast_pnorm table).  Sums are f64 in draw order, divided by the draw count
+ * at the end.  The model, the trace and every draw are bit-identical to fmwr_train_dev's.  Fails without touching the model
+ * with FMWR_ERR_ARG (solver not MCMC, burn_in outside [0, max_iter), an eval set null, equal to d or listed twice),
+ * FMWR_ERR_SHAPE (an eval set of another feature count) or FMWR_ERR_UNSUPPORTED (row-sharded context: one GPU only). */
+int fmwr_train_posterior_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* trace /* nullable */,
+                             int32_t burn_in, fmwr_data* const* eval /* [n_eval] */, int32_t n_eval);
 
 /* ---- one-shot host-buffer entry points: what the rewritten src/FM.cpp calls ---- */
 /* FMPredict body (src/FM.cpp:177-214) */
