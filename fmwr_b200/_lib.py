@@ -410,3 +410,15 @@ def train_posterior_dev(ctx, model, data, scfg, burn_in, evals=(), trace=None, k
     check(lib().fmwr_train_posterior_dev(ctx.h, model.h, data.h, C.byref(scfg), C.byref(trace.c) if trace is not None else None,
                                          C.c_int32(burn_in), arr if len(evals) else None, C.c_int32(len(evals))))
     del keep
+
+
+def train_holdout_dev(ctx, model, data, scfg, trace, evals, select_best=0, patience=0, keep=()):
+    """train_dev plus held-out tracking: every eval set (labelled Data handles; an entry of None passes a null handle) is
+    scored at every tracker record.  Returns (scores [n_eval][n_rec stored], best_rec)."""
+    arr = (C.c_void_p * max(len(evals), 1))(*[e.h if e is not None else None for e in evals])
+    scores = np.full((max(len(evals), 1), max(trace.max_rec, 1)), np.nan)
+    best = C.c_int32(-1)
+    check(lib().fmwr_train_holdout_dev(ctx.h, model.h, data.h, C.byref(scfg), C.byref(trace.c), arr if len(evals) else None,
+                                       C.c_int32(len(evals)), ptr(scores), C.c_int32(select_best), C.c_int32(patience), C.byref(best)))
+    del keep
+    return scores[:len(evals), :min(trace.c.n_rec, trace.max_rec)].copy(), best.value

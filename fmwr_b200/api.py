@@ -268,16 +268,17 @@ def _model_cfg(mc):
                       l2_v=float(hp["L2.v"]))
 
 
-def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_list, streams=None, posterior=None):
+def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_list, streams=None, posterior=None, holdout=None):
     """body of FM() (reference src/FM.cpp:7-174) on top of the C ABI.  posterior (fm_posterior): dict(burn_in, newdata) in, and
-    the device means out as posterior["train"] and posterior["newdata_mean"]"""
+    the device means out as posterior["train"] and posterior["newdata_mean"].  holdout (fm_train_holdout): dict(newdata, labels,
+    select_best, patience, snapshots) in; the trace gains "evaluation.test" and "best.index"."""
     ctx = _ctx()
     feats = data["features"]
     n, p = feats["dim"]
     labels = data["labels"]
     normalize0 = np.atleast_1d(np.asarray(normalize0, np.int64))
     d, parked = _acquire(ctx, feats, labels, normalize0[0] > -1)
-    evals = []                                                            # (handle, parked) of posterior["newdata"]
+    evals = []                                                            # (handle, parked) of posterior / holdout["newdata"]
     try:
         scales = {}
         if normalize0[0] > -1:                                            # FM.cpp:36-38
@@ -329,8 +330,15 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
             if sc.step_size > 0:
                 from math import ceil
                 nrec = min(10001, int(ceil((sc.max_iter - 0.5) / sc.step_size)) + 2)
-                trace = L.TraceBuf(nrec, p, k, snapshots=True)
-            if posterior is None:
+                trace = L.TraceBuf(nrec, p, k, snapshots=holdout is None or holdout["snapshots"])
+            if holdout is not None:
+                for nd, nd_labels in zip(holdout["newdata"], holdout["labels"]):   # z-scored with the training scales as fm.track does
+                    evals.append(_acquire(ctx, nd["features"], nd_labels, normalize0[0] > -1))
+                    if normalize0[0] > -1:
+                        evals[-1][0].normalize(scales["mean"], scales["std"])
+                test, best = L.train_holdout_dev(ctx, m, d, sc, trace, [e for e, _ in evals], holdout["select_best"],
+                                                 holdout["patience"], keep=keep)
+            elif posterior is None:
                 L.train_dev(ctx, m, d, sc, trace, keep=keep)
             else:
                 for nd in posterior["newdata"]:                           # checked and z-scored as predict does it
@@ -360,8 +368,12 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
     if trace is not None:
         t = trace.result()
         model["convergence"] = t["convergent"]
-        snaps = [dict(w0=t["snap_w0"][i], w=t["snap_w"][i], v=t["snap_v"][i].T.copy()) for i in range(len(t["rec_index"]))]
+        snaps = ([dict(w0=t["snap_w0"][i], w=t["snap_w"][i], v=t["snap_v"][i].T.copy()) for i in range(len(t["rec_index"]))]
+                 if "snap_w0" in t else [])
         res["Trace"] = {"trace": [t["rec_index"].astype(np.float64)] + snaps, "evaluation.train": t["eval_train"]}
+        if holdout is not None:
+            res["Trace"]["evaluation.test"] = [row for row in test]
+            res["Trace"]["best.index"] = best
     else:
         model["convergence"] = False
     scales["target.range"] = (lo, hi)
@@ -437,6 +449,55 @@ def fm_posterior(data, newdata=(), burn_in=0, normalize=True, control=None):
     post = dict(burn_in=int(burn_in), newdata=newdata)
     fit = _FM(data, norm - 1, ctl["model"], ctl["solver"], ctl["track"], None, posterior=post)
     return dict(fit=fit, train=post["train"], newdata=post["newdata_mean"])
+
+
+def fm_train_holdout(data, newdata, normalize=True, control=None, select="last", patience=0, snapshots=True):
+    """Engine extension of the fm.train -> fm.track -> fm.select workflow: trains exactly as fm_train(data, normalize, control)
+    and, at every tracker record (step_size > 0 in track.control), also scores every newdata (labelled fm.matrix objects of the
+    same width, labels 0/1 recoded and values z-scored with the training scales as fm_track does) on the device.
+    Trace gains "evaluation.test" (one array per newdata, what fm_track would return as "test") and "best.index" (the first
+    record with the best score on newdata[0]: highest for classification, lowest for regression; -1 if all were NaN).
+    select="best" puts that record's model in Model (fm_select(fit, best_iter=best.index)); patience > 0 also stops training
+    after that many records in a row without an improvement on newdata[0].  snapshots=False keeps no per-record model on the
+    host (the trace is then the index, the train and test curves and best.index; fm_track and fm_select refuse such a fit)."""
+    if isinstance(newdata, FmMatrix):
+        newdata = [newdata]
+    if not isinstance(newdata, (list, tuple)) or not newdata:
+        raise ValueError("newdata must be a fm.matrix object or a non-empty list of them")
+    newdata = list(newdata)
+    if select not in ("last", "best"):
+        raise ValueError("select must be \"last\" or \"best\"")
+    if int(patience) != patience or patience < 0:
+        raise ValueError("patience must be an integer >= 0")
+    data, norm, ctl = _train_setup(data, normalize, control)
+    if ctl["track"]["step_size"] <= 0:
+        raise ValueError("held-out tracking needs step_size > 0 in track.control")
+    cls = ctl["model"]["task"] == "CLASSIFICATION"
+    labels = []
+    for i, nd in enumerate(newdata):
+        if not isinstance(nd, FmMatrix):
+            raise ValueError("newdata must be fm.matrix objects")
+        if nd.get("labels") is None:
+            raise ValueError("there are no labels in newdata")
+        if np.isnan(nd["features"]["value"]).any():
+            raise ValueError("there are NAs in newdata")
+        if nd["features"] is data["features"]:
+            raise ValueError("newdata is the training data: its score is Trace$evaluation.train")
+        if any(nd["features"] is o["features"] for o in newdata[:i]):
+            raise ValueError("the same newdata appears twice")
+        y = np.asarray(nd["labels"], np.float64)
+        if cls and np.array_equal(np.unique(y), [0, 1]):                 # as fm_track recodes them
+            y = np.where(y < 1, -1.0, 1.0)
+        labels.append(y)
+    ho = dict(newdata=newdata, labels=labels, select_best=int(select == "best"), patience=int(patience), snapshots=bool(snapshots))
+    return _FM(data, norm - 1, ctl["model"], ctl["solver"], ctl["track"], None, holdout=ho)
+
+
+def _require_snapshots(obj):
+    t = obj["Trace"]["trace"]
+    if len(t) - 1 != len(t[0]):
+        raise ValueError("the trace keeps no model snapshots (fm_train_holdout(..., snapshots=False)): "
+                         "its held-out scores are Trace$evaluation.test and its best record Trace$best.index")
 
 
 def _link_for(model):
@@ -522,6 +583,7 @@ def fm_track(obj, newdata, normalize=True, evaluate_metric=None):
     score every recorded snapshot on new data"""
     if "Trace" not in obj:
         raise ValueError("there is no trace in FM model, please set step_size > 0 in track.control")
+    _require_snapshots(obj)
     if newdata.get("labels") is None:
         raise ValueError("there are no labels in newdata")
     model = obj["Model"]
@@ -560,6 +622,7 @@ def fm_select(obj, best_iter=None, track=None, higher_is_better=None):
     """R/fm_select.R:58-61: swap a recorded snapshot in as the model"""
     if "Trace" not in obj:
         raise ValueError("there is no trace in FM model")
+    _require_snapshots(obj)
     if best_iter is None:
         if track is None:
             raise ValueError("either best_iter or the result of fm.track is needed")

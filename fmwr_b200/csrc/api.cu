@@ -285,18 +285,18 @@ static void fetch_pred(fmwr_ctx* ctx, fmwr_data* d, double* out)
 }
 
 static void train_dispatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr,
-                           const Posterior* post = nullptr)
+                           const Posterior* post = nullptr, const Holdout* holdout = nullptr)
 {
   FMWR_REQUIRE(d->has_labels, FMWR_ERR_ARG, "target's length is not equal the number of cases...");
   FMWR_REQUIRE(d->p == m->p, FMWR_ERR_SHAPE, "there's no the same number of features between train and fm object...");
   if (tr) { tr->n_rec = 0; tr->convergent = 0; tr->iters_done = 0; }
   switch (s->solver) {
     case FMWR_SGD: case FMWR_FTRL: case FMWR_TDAP:
-      if (s->mode == FMWR_MODE_MINIBATCH) train_minibatch(ctx, m, d, s, tr);
-      else train_exact(ctx, m, d, s, tr);
+      if (s->mode == FMWR_MODE_MINIBATCH) train_minibatch(ctx, m, d, s, tr, holdout);
+      else train_exact(ctx, m, d, s, tr, holdout);
       break;
     case FMWR_ALS: case FMWR_MCMC:
-      train_als_mcmc(ctx, m, d, s, tr, post);
+      train_als_mcmc(ctx, m, d, s, tr, post, holdout);
       break;
     default: throw Error(FMWR_ERR_ARG, "Unknown solver...");   // reference src/FM.cpp:85
   }
@@ -785,6 +785,33 @@ int fmwr_train_posterior_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const f
     FMWR_CUDA(cudaSetDevice(ctx->device));
     const Posterior post{burn_in, eval, n_eval};
     train_dispatch(ctx, m, d, s, trace, &post);
+  });
+}
+
+int fmwr_train_holdout_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* trace,
+                           fmwr_data* const* eval, int32_t n_eval, double* eval_scores,
+                           int32_t select_best, int32_t patience, int32_t* best_rec)
+{
+  return guarded([&] {
+    FMWR_REQUIRE(ctx && m && d && s, FMWR_ERR_ARG, "null argument");
+    FMWR_REQUIRE(trace, FMWR_ERR_ARG, "held-out tracking needs a trace (its max_rec bounds the stored scores)");
+    FMWR_REQUIRE(s->step_size > 0, FMWR_ERR_ARG, "held-out tracking needs step_size > 0 (the held-out sets are scored at the tracker's records)");
+    FMWR_REQUIRE(n_eval >= 1 && eval, FMWR_ERR_ARG, "held-out tracking needs at least one eval set");
+    FMWR_REQUIRE(eval_scores, FMWR_ERR_ARG, "null eval_scores");
+    FMWR_REQUIRE(patience >= 0, FMWR_ERR_ARG, "patience must be at least 0");
+    for (int i = 0; i < n_eval; ++i) {
+      FMWR_REQUIRE(eval[i], FMWR_ERR_ARG, "null eval data");
+      FMWR_REQUIRE(eval[i]->has_labels, FMWR_ERR_ARG, "an eval set has no labels");
+      FMWR_REQUIRE(eval[i] != d, FMWR_ERR_ARG, "an eval set is the training data (its score is the trace's eval_train)");
+      for (int j = 0; j < i; ++j) FMWR_REQUIRE(eval[j] != eval[i], FMWR_ERR_ARG, "an eval set appears twice");
+    }
+    for (int i = 0; i < n_eval; ++i) require_same_features(m, eval[i]);
+    FMWR_REQUIRE(!(ctx->nccl_comm && ctx->world > 1), FMWR_ERR_UNSUPPORTED, "held-out tracking runs on one GPU (sharded models are not supported)");
+    FMWR_CUDA(cudaSetDevice(ctx->device));
+    int32_t best = -1;
+    const Holdout ho{eval, n_eval, eval_scores, trace->max_rec, select_best != 0, patience, &best};
+    train_dispatch(ctx, m, d, s, trace, nullptr, &ho);
+    if (best_rec) *best_rec = best;
   });
 }
 

@@ -425,15 +425,37 @@ void minibatch_batch_values(fmwr_data* d, int64_t b);   // batch b's values read
 void minibatch_all_values(fmwr_data* d);                // every value ready (a first epoch that stopped early)
 int64_t minibatch_entries(const fmwr_data* d);          // entries of the per-batch CSC
 bool minibatch_streams_values(const fmwr_solver_cfg* s);   // train_minibatch may start on data whose values are still uploading
-void train_exact(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr);
-void train_minibatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr);
+// Held-out tracking (fmwr_train_holdout_dev): at every tracker record, score each eval set (validated by the caller: labelled,
+// distinct, not the training data, same feature count) with the record's model; select the best record on eval[0]
+struct Holdout {
+  fmwr_data* const* eval; int n_eval;
+  double* scores; int max_rec;        // scores[i * max_rec + r] for records r < max_rec
+  bool select_best;                   // restore the best record's (w0, w, V) into the model at the end
+  int patience;                       // > 0: stop after this many records in a row without an improvement on eval[0]
+  int32_t* best_rec;                  // out: the first record with the best eval[0] score, -1 if every score was NaN
+};
+// One training call's held-out state.  The trainers call record() right after tracker_snapshot and finish() after their
+// loop (before the final synchronise); with h == nullptr both do nothing.
+struct HoldoutRun {
+  const Holdout* h;
+  double best = 0.0;
+  int best_rec = -1, since = 0;       // since: records after best_rec
+  DBuf<char> w, v;                    // device copy of the best record's w [p] and V [p][kp], the model's own type
+  DBuf<double> w0;
+  explicit HoldoutRun(const Holdout* h_) : h(h_) {}
+  bool record(fmwr_ctx* ctx, fmwr_model* m, const fmwr_solver_cfg* s, int rec);   // true: patience says stop
+  void finish(fmwr_ctx* ctx, fmwr_model* m);
+};
+void train_exact(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* holdout = nullptr);
+void train_minibatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* holdout = nullptr);
 // MCMC posterior mean (fmwr_train_posterior_dev): average the predict.FM prediction of draws burn_in+1 .. max_iter on the
 // training rows and on every eval set (validated by the caller: distinct, not the training data, same feature count)
 struct Posterior {
   int burn_in;
   fmwr_data* const* eval; int n_eval;
 };
-void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Posterior* post = nullptr);
+void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Posterior* post = nullptr,
+                    const Holdout* holdout = nullptr);
 // shape check of Model::predict_batch (reference src/core/Model.h:112-113)
 inline void require_same_features(const fmwr_model* m, const fmwr_data* d)
 {

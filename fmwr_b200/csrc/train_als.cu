@@ -1304,7 +1304,8 @@ struct HostStreams {
 static inline bool hbad(double x) { return std::isnan(x) || std::isinf(x); }
 
 template <class T>
-static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Posterior* post)
+static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Posterior* post,
+                        const Holdout* holdout)
 {
   const int64_t n = d->n, p = d->p;
   const int k = m->k, kp = m->kp;
@@ -1433,6 +1434,7 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
   const int step = tracker_step_size(s->step_size, s->max_iter);
   int ii = -1, n_rec = 0;
   int sweep = 0;
+  HoldoutRun ho(holdout);
   for (; sweep < s->max_iter; ++sweep) {
     // tracker (:101-124): train metric of the model at the start of the sweep
     if (step > 0) {
@@ -1441,7 +1443,9 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
       if (ii == 0 || sweep == s->max_iter - 1) {
         const double score = tracker_score(ctx, m, d, s);
         tracker_snapshot(m, tr, n_rec, sweep, score);
+        const bool patience_stop = ho.record(ctx, m, s, n_rec);
         n_rec++;
+        if (patience_stop) break;            // decided at the start of the sweep: this sweep does not run
       }
     }
     // e <- predict_batch (:100), q[r][f] <- S_f
@@ -1581,6 +1585,7 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
       dd->pred_prec = FMWR_F64;
     }
   }
+  ho.finish(ctx, m);
   FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
   if (ctx->world > 1) peer_check_error(ctx);      // a timed-out exchange means partial (A,B) sums: the replicas have diverged
   if (tr) { tr->n_rec = std::min(n_rec, (int)tr->max_rec); tr->convergent = 0; tr->iters_done = sweep; }
@@ -1644,11 +1649,13 @@ int als_effective_precision(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fm
   return has_thin_columns(ctx, d) ? FMWR_F64 : FMWR_F32;
 }
 
-void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Posterior* post)
+void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Posterior* post,
+                    const Holdout* holdout)
 {
-  if (m->prec == FMWR_F64) { train_als_t<double>(ctx, m, d, s, tr, post); return; }
-  if (als_effective_precision(ctx, m, d, s) == FMWR_F32) { train_als_t<float>(ctx, m, d, s, tr, post); return; }
-  // fp64 shadow of the fp32 handle (a posterior mean averages the shadow's draws)
+  if (m->prec == FMWR_F64) { train_als_t<double>(ctx, m, d, s, tr, post, holdout); return; }
+  if (als_effective_precision(ctx, m, d, s) == FMWR_F32) { train_als_t<float>(ctx, m, d, s, tr, post, holdout); return; }
+  // fp64 shadow of the fp32 handle (a posterior mean averages the shadow's draws; held-out tracking scores the shadow and
+  // restores its best copy into the shadow, before the handback below narrows it into the fp32 handle)
   fmwr_model* sh = nullptr;
   FMWR_REQUIRE(fmwr_model_create(ctx, &m->cfg, m->p, FMWR_F64, &sh) == 0, FMWR_ERR_CUDA, fmwr_last_error());
   try {
@@ -1658,7 +1665,7 @@ void train_als_mcmc(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solve
       FMWR_LAUNCH(ctx, (repack_rows_kernel<float, double>), ceil_div(p, 256), 256, 0, (const float*)m->w.p, 1, (double*)sh->w.p, 1, p, 1);
       FMWR_LAUNCH(ctx, (repack_rows_kernel<float, double>), ceil_div(p * sh->kp, 256), 256, 0, (const float*)m->v.p, m->kp, (double*)sh->v.p, sh->kp, p, m->k);
     }
-    train_als_t<double>(ctx, sh, d, s, tr, post);
+    train_als_t<double>(ctx, sh, d, s, tr, post, holdout);
     FMWR_CUDA(cudaMemcpyAsync(m->scal.p, sh->scal.p, 8 * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
     if (p > 0) {
       FMWR_LAUNCH(ctx, (repack_rows_kernel<double, float>), ceil_div(p, 256), 256, 0, (const double*)sh->w.p, 1, (float*)m->w.p, 1, p, 1);

@@ -592,6 +592,46 @@ void tracker_snapshot(fmwr_model* m, fmwr_trace* tr, int idx, int iter, double s
   }
 }
 
+// Held-out sets are scored exactly as tracker_score scores the training data: same model, link and metric.  Better on eval[0]
+// is strictly greater for classification (LL, AUC, ACC) and strictly smaller for regression (evaluate_dev returns RMSE or MAE
+// there), so ties keep the earlier record and NaN never wins.  Every record counts, stored or not.
+bool HoldoutRun::record(fmwr_ctx* ctx, fmwr_model* m, const fmwr_solver_cfg* s, int rec)
+{
+  if (!h) return false;
+  double score0 = 0.0;
+  for (int i = 0; i < h->n_eval; ++i) {
+    const double sc = tracker_score(ctx, m, h->eval[i], s);
+    if (i == 0) score0 = sc;
+    if (rec < h->max_rec) h->scores[(size_t)i * h->max_rec + rec] = sc;
+  }
+  const bool cls = m->cfg.task == FMWR_CLASSIFICATION;
+  if (!std::isnan(score0) && (best_rec < 0 || (cls ? score0 > best : score0 < best))) {
+    best = score0; best_rec = rec; since = 0;
+    if (h->select_best) {
+      const size_t wb = (size_t)m->p * m->esz(), vb = (size_t)m->p * m->kp * m->esz();
+      w.alloc(wb); v.alloc(vb); w0.alloc(1);
+      if (wb) FMWR_CUDA(cudaMemcpyAsync(w.p, m->w.p, wb, cudaMemcpyDeviceToDevice, ctx->stream));
+      if (vb) FMWR_CUDA(cudaMemcpyAsync(v.p, m->v.p, vb, cudaMemcpyDeviceToDevice, ctx->stream));
+      FMWR_CUDA(cudaMemcpyAsync(w0.p, m->scal.p, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+  } else {
+    since++;
+  }
+  return h->patience > 0 && since >= h->patience;
+}
+
+// the best copy goes back over (w0, w, V) only: scal[1..] and the optimizer state stay as training left them
+void HoldoutRun::finish(fmwr_ctx* ctx, fmwr_model* m)
+{
+  if (!h) return;
+  *h->best_rec = best_rec;
+  if (!h->select_best || best_rec < 0) return;
+  const size_t wb = (size_t)m->p * m->esz(), vb = (size_t)m->p * m->kp * m->esz();
+  if (wb) FMWR_CUDA(cudaMemcpyAsync(m->w.p, w.p, wb, cudaMemcpyDeviceToDevice, ctx->stream));
+  if (vb) FMWR_CUDA(cudaMemcpyAsync(m->v.p, v.p, vb, cudaMemcpyDeviceToDevice, ctx->stream));
+  FMWR_CUDA(cudaMemcpyAsync(m->scal.p, w0.p, sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+}
+
 // Tracker::init step-size rule (reference src/core/Tracker.h:41-52, MAX_REC = 10000)
 int tracker_step_size(int step_size, int max_iter)
 {
@@ -623,7 +663,8 @@ std::vector<uint32_t> visit_order_host(const fmwr_data* d, const fmwr_solver_cfg
 }
 
 template <class T>
-static void train_exact_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr)
+static void train_exact_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr,
+                          const Holdout* holdout)
 {
   const SolverParams<double> spd = make_params<double>(m, s);
   model_alloc_state(m, solver_state_count(spd), s->solver, s->warm_state != 0);   // Learner::init(): the state restarts at zero unless warm
@@ -664,6 +705,7 @@ static void train_exact_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr
   int64_t iter = 0;
   int n_rec = 0, conv_times = 0, convergent = 0;
   double old_score = 0.0;
+  HoldoutRun ho(holdout);
   while (iter < max_iter) {
     // run up to the next tracker point: the reference evaluates after the update of samples
     // 0, step, 2*step, ... and of sample max_iter-1 (SGD_Learner.h:140-143)
@@ -694,19 +736,22 @@ static void train_exact_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr
         else conv_times = 0;
         old_score = score;
         tracker_snapshot(m, tr, n_rec, (int)last, score);
+        const bool patience_stop = ho.record(ctx, m, s, n_rec);
         n_rec++;
         if (conv_times >= 3) { convergent = 1; break; }
+        if (patience_stop) break;
       }
     }
   }
+  ho.finish(ctx, m);
   FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
   if (tr) { tr->n_rec = std::min(n_rec, (int)tr->max_rec); tr->convergent = convergent; tr->iters_done = (int)iter; }   // records WRITTEN (tracker_snapshot drops what does not fit)
 }
 
-void train_exact(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr)
+void train_exact(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* holdout)
 {
-  if (m->prec == FMWR_F64) train_exact_t<double>(ctx, m, d, s, tr);
-  else train_exact_t<float>(ctx, m, d, s, tr);
+  if (m->prec == FMWR_F64) train_exact_t<double>(ctx, m, d, s, tr, holdout);
+  else train_exact_t<float>(ctx, m, d, s, tr, holdout);
 }
 
 }  // namespace fmwr

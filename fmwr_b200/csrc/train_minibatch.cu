@@ -801,8 +801,10 @@ bool minibatch_streams_values(const fmwr_solver_cfg* s)
          s->step_size <= 0 && s->random_step <= 1 && !(s->visit_order && s->n_visit > 0);
 }
 
+// eval_d: the training data the tracker scores (the full data when d holds the gathered visits); holdout: the held-out sets
 template <class T>
-static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, fmwr_data* eval_d = nullptr)
+static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* holdout,
+                              fmwr_data* eval_d = nullptr)
 {
   FMWR_REQUIRE(s->batch_size > 0, FMWR_ERR_ARG, "batch_size must be positive in minibatch mode");
   if (!eval_d) eval_d = d;
@@ -822,7 +824,7 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
     s2.random_step = 1; s2.visit_order = nullptr; s2.n_visit = 0;
     s2.compat &= ~FMWR_COMPAT_SKIP_ROW0;                   // the sequence already says which rows are visited
     s2.max_iter = (int32_t)order.size();
-    train_minibatch_t<T>(ctx, m, visited.get(), &s2, tr, eval_d);
+    train_minibatch_t<T>(ctx, m, visited.get(), &s2, tr, holdout, eval_d);
     return;
   }
   const SolverParams<double> spd = make_params_f64(m, s);
@@ -884,7 +886,9 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
   const int step = tracker_step_size(s->step_size, s->max_iter);   // Tracker::init's MAX_REC rule (src/core/Tracker.h:41-52)
   int64_t iter = 0, next_track = 0;
   int n_rec = 0, conv_times = 0, convergent = 0;
+  bool patience_stop = false;
   double old_score = 0.0, u_w = 0.0, u_v = 0.0;
+  HoldoutRun ho(holdout);
   const bool sgd_l1 = spd.solver == FMWR_SGD && spd.l1;
   if (sgd_l1 && kept_state) {                // cumulative-L1 totals live in the scalar block ([1], [2]) like in the exact mode
     double h[2] = {0, 0};
@@ -925,7 +929,7 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
     FMWR_CUDA(cudaGraphLaunch(ge, ctx->stream));
     captured = 0;
   };
-  while (iter < max_iter && !convergent) {
+  while (iter < max_iter && !convergent && !patience_stop) {
     for (int64_t b = 0; b < n_batches && iter < max_iter; ++b) {
       if (use_graph && captured == 0) { FMWR_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal)); bag.capturing = true; }
       const int64_t rb = row0 + b * B;
@@ -960,15 +964,18 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
         else conv_times = 0;
         old_score = score;
         tracker_snapshot(m, tr, n_rec, (int)(iter - 1), score);
+        patience_stop = ho.record(ctx, m, s, n_rec);
         n_rec++;
         next_track = (iter / step + 1) * (int64_t)step;
         if (conv_times >= 3) { convergent = 1; break; }
+        if (patience_stop) break;
       }
     }
   }
   minibatch_all_values(d);                       // a truncated first epoch: finish the value fill for later calls
   flush_graph();
   if (sgd_l1) { const double h[2] = {u_w, u_v}; FMWR_CUDA(cudaMemcpyAsync((double*)m->scal.p + 1, h, 16, cudaMemcpyHostToDevice, ctx->stream)); }
+  ho.finish(ctx, m);
   FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
   if (peer) peer_check_error(ctx);
   if (peer && getenv("FMWR_PEER_DEBUG")) {
@@ -984,10 +991,10 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
   if (tr) { tr->n_rec = std::min(n_rec, (int)tr->max_rec); tr->convergent = convergent; tr->iters_done = (int)iter; }
 }
 
-void train_minibatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr)
+void train_minibatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* holdout)
 {
-  if (m->prec == FMWR_F64) train_minibatch_t<double>(ctx, m, d, s, tr);
-  else train_minibatch_t<float>(ctx, m, d, s, tr);
+  if (m->prec == FMWR_F64) train_minibatch_t<double>(ctx, m, d, s, tr, holdout);
+  else train_minibatch_t<float>(ctx, m, d, s, tr, holdout);
 }
 
 }  // namespace fmwr

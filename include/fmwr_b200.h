@@ -232,6 +232,27 @@ int fmwr_train_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver
  * FMWR_ERR_SHAPE (an eval set of another feature count) or FMWR_ERR_UNSUPPORTED (row-sharded context: one GPU only). */
 int fmwr_train_posterior_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* trace /* nullable */,
                              int32_t burn_in, fmwr_data* const* eval /* [n_eval] */, int32_t n_eval);
+/* Held-out tracking (extension of Tracker / fm.track, src/core/Tracker.h:70-94).  Runs exactly the training
+ * fmwr_train_dev(ctx, m, d, s, trace) runs and, at every tracker record, also scores each eval[i] (labels required) with the
+ * record's model: the forward with the tracker's link (regression: clamped to [s->min_target, s->max_target]; classification:
+ * the fast_pnorm table for ALS/MCMC, logistic otherwise) and the metric s->metric, as fmwr_predict_dev + fmwr_evaluate_dev
+ * would.  Records are the tracker's: SGD/FTRL/TDAP after samples 0, step, 2 step, ... and max_iter-1 (minibatch mode: at
+ * batch granularity), ALS/MCMC at the start of a sweep.  eval_scores[i * trace->max_rec + r] gets set i's score of record r;
+ * records past max_rec are scored and count below, but are not stored (as tracker_snapshot drops them).
+ * Better on eval[0] is strictly greater for classification and strictly smaller for regression (RMSE or MAE there); NaN is
+ * never better, ties keep the earlier record, the first non-NaN record is the initial best.  *best_rec (nullable) gets the
+ * best record's number, -1 when every score was NaN.  select_best != 0: on return the model holds (w0, w, V) of that record
+ * (the optimizer state stays as training left it, as fm.select).  patience > 0: training also stops after `patience`
+ * consecutive records without an improvement on eval[0] -- trace->iters_done < max_iter with trace->convergent == 0; ALS/MCMC
+ * decide it at the start of a sweep, which then does not run.  The train-score convergence rule is unchanged.  Each eval
+ * handle ends up holding the forward result of the last record (fmwr_predict_fetch reads it).  The fp64 shadow of an fp32
+ * ALS/MCMC handle is what is scored, selected and then narrowed into the handle.  Fails without touching the model with
+ * FMWR_ERR_ARG (trace null, s->step_size <= 0, n_eval < 1, eval or eval_scores null, an eval set null, without labels,
+ * equal to d or listed twice, patience < 0), FMWR_ERR_SHAPE (an eval set of another feature count) or FMWR_ERR_UNSUPPORTED
+ * (a communicator with world > 1: one GPU only). */
+int fmwr_train_holdout_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* trace,
+                           fmwr_data* const* eval /* [n_eval] */, int32_t n_eval, double* eval_scores /* [n_eval][trace->max_rec] */,
+                           int32_t select_best, int32_t patience, int32_t* best_rec /* nullable */);
 
 /* ---- one-shot host-buffer entry points: what the rewritten src/FM.cpp calls ---- */
 /* FMPredict body (src/FM.cpp:177-214) */
