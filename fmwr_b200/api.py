@@ -423,6 +423,22 @@ def _train_setup(data, normalize, control):
     return data, norm, ctl
 
 
+def _check_newdata(newdata, data, need_labels):
+    """the newdata list of fm_posterior / fm_train_holdout: fm.matrix objects (labelled where they are scored) without NAs,
+    none of them the training data, each listed once"""
+    for i, nd in enumerate(newdata):
+        if not isinstance(nd, FmMatrix):
+            raise ValueError("newdata must be fm.matrix objects")
+        if need_labels and nd.get("labels") is None:
+            raise ValueError("there are no labels in newdata")
+        if np.isnan(nd["features"]["value"]).any():
+            raise ValueError("there are NAs in newdata")
+        if nd["features"] is data["features"]:
+            raise ValueError("newdata is the training data")
+        if any(nd["features"] is o["features"] for o in newdata[:i]):
+            raise ValueError("the same newdata appears twice")
+
+
 def fm_posterior(data, newdata=(), burn_in=0, normalize=True, control=None):
     """Engine extension: the MCMC posterior mean libFM predicts with.  Trains exactly as fm_train(data, normalize, control) and
     also averages, on the device, the predict.FM prediction of draws burn_in+1 .. max_iter (draw t = the model after sweep t)
@@ -437,15 +453,7 @@ def fm_posterior(data, newdata=(), burn_in=0, normalize=True, control=None):
     max_iter = int(ctl["solver"]["max_iter"])
     if int(burn_in) != burn_in or not 0 <= burn_in < max_iter:
         raise ValueError("burn_in must be an integer in [0, max_iter) = [0, %d)" % max_iter)
-    for i, nd in enumerate(newdata):
-        if not isinstance(nd, FmMatrix):
-            raise ValueError("newdata must be fm.matrix objects")
-        if np.isnan(nd["features"]["value"]).any():
-            raise ValueError("there are NAs in newdata")
-        if nd["features"] is data["features"]:
-            raise ValueError("newdata is the training data: its mean is returned as train")
-        if any(nd["features"] is o["features"] for o in newdata[:i]):
-            raise ValueError("the same newdata appears twice")
+    _check_newdata(newdata, data, need_labels=False)
     post = dict(burn_in=int(burn_in), newdata=newdata)
     fit = _FM(data, norm - 1, ctl["model"], ctl["solver"], ctl["track"], None, posterior=post)
     return dict(fit=fit, train=post["train"], newdata=post["newdata_mean"])
@@ -472,19 +480,10 @@ def fm_train_holdout(data, newdata, normalize=True, control=None, select="last",
     data, norm, ctl = _train_setup(data, normalize, control)
     if ctl["track"]["step_size"] <= 0:
         raise ValueError("held-out tracking needs step_size > 0 in track.control")
+    _check_newdata(newdata, data, need_labels=True)
     cls = ctl["model"]["task"] == "CLASSIFICATION"
     labels = []
-    for i, nd in enumerate(newdata):
-        if not isinstance(nd, FmMatrix):
-            raise ValueError("newdata must be fm.matrix objects")
-        if nd.get("labels") is None:
-            raise ValueError("there are no labels in newdata")
-        if np.isnan(nd["features"]["value"]).any():
-            raise ValueError("there are NAs in newdata")
-        if nd["features"] is data["features"]:
-            raise ValueError("newdata is the training data: its score is Trace$evaluation.train")
-        if any(nd["features"] is o["features"] for o in newdata[:i]):
-            raise ValueError("the same newdata appears twice")
+    for nd in newdata:
         y = np.asarray(nd["labels"], np.float64)
         if cls and np.array_equal(np.unique(y), [0, 1]):                 # as fm_track recodes them
             y = np.where(y < 1, -1.0, 1.0)

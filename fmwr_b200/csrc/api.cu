@@ -284,6 +284,18 @@ static void fetch_pred(fmwr_ctx* ctx, fmwr_data* d, double* out)
   }
 }
 
+// eval sets of fmwr_train_posterior_dev / fmwr_train_holdout_dev: non-null, labelled if scored, not d, listed once, p features
+static void check_eval_list(const fmwr_model* m, const fmwr_data* d, fmwr_data* const* eval, int n_eval, bool need_labels)
+{
+  for (int i = 0; i < n_eval; ++i) {
+    FMWR_REQUIRE(eval[i], FMWR_ERR_ARG, "null eval data");
+    FMWR_REQUIRE(!need_labels || eval[i]->has_labels, FMWR_ERR_ARG, "an eval set has no labels");
+    FMWR_REQUIRE(eval[i] != d, FMWR_ERR_ARG, "an eval set is the training data");
+    for (int j = 0; j < i; ++j) FMWR_REQUIRE(eval[j] != eval[i], FMWR_ERR_ARG, "an eval set appears twice");
+  }
+  for (int i = 0; i < n_eval; ++i) require_same_features(m, eval[i]);
+}
+
 static void train_dispatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr,
                            const Posterior* post = nullptr, const Holdout* holdout = nullptr)
 {
@@ -775,12 +787,7 @@ int fmwr_train_posterior_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const f
     FMWR_REQUIRE(n_eval >= 0 && (n_eval == 0 || eval), FMWR_ERR_ARG, "null eval list");
     FMWR_REQUIRE(s->solver == FMWR_MCMC, FMWR_ERR_ARG, "posterior averaging needs the MCMC solver");
     FMWR_REQUIRE(burn_in >= 0 && burn_in < s->max_iter, FMWR_ERR_ARG, "burn_in must be at least 0 and less than max_iter");
-    for (int i = 0; i < n_eval; ++i) {
-      FMWR_REQUIRE(eval[i], FMWR_ERR_ARG, "null eval data");
-      FMWR_REQUIRE(eval[i] != d, FMWR_ERR_ARG, "an eval set is the training data (its mean is the training rows' result)");
-      for (int j = 0; j < i; ++j) FMWR_REQUIRE(eval[j] != eval[i], FMWR_ERR_ARG, "an eval set appears twice");
-    }
-    for (int i = 0; i < n_eval; ++i) require_same_features(m, eval[i]);
+    check_eval_list(m, d, eval, n_eval, false);
     FMWR_REQUIRE(!(ctx->nccl_comm && ctx->world > 1), FMWR_ERR_UNSUPPORTED, "posterior averaging runs on one GPU (row-sharded data is not supported)");
     FMWR_CUDA(cudaSetDevice(ctx->device));
     const Posterior post{burn_in, eval, n_eval};
@@ -799,13 +806,7 @@ int fmwr_train_holdout_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmw
     FMWR_REQUIRE(n_eval >= 1 && eval, FMWR_ERR_ARG, "held-out tracking needs at least one eval set");
     FMWR_REQUIRE(eval_scores, FMWR_ERR_ARG, "null eval_scores");
     FMWR_REQUIRE(patience >= 0, FMWR_ERR_ARG, "patience must be at least 0");
-    for (int i = 0; i < n_eval; ++i) {
-      FMWR_REQUIRE(eval[i], FMWR_ERR_ARG, "null eval data");
-      FMWR_REQUIRE(eval[i]->has_labels, FMWR_ERR_ARG, "an eval set has no labels");
-      FMWR_REQUIRE(eval[i] != d, FMWR_ERR_ARG, "an eval set is the training data (its score is the trace's eval_train)");
-      for (int j = 0; j < i; ++j) FMWR_REQUIRE(eval[j] != eval[i], FMWR_ERR_ARG, "an eval set appears twice");
-    }
-    for (int i = 0; i < n_eval; ++i) require_same_features(m, eval[i]);
+    check_eval_list(m, d, eval, n_eval, true);
     FMWR_REQUIRE(!(ctx->nccl_comm && ctx->world > 1), FMWR_ERR_UNSUPPORTED, "held-out tracking runs on one GPU (sharded models are not supported)");
     FMWR_CUDA(cudaSetDevice(ctx->device));
     int32_t best = -1;
@@ -924,9 +925,7 @@ int fmwr_track(const fmwr_model_cfg* cfg, int32_t solver, int32_t precision, int
     if (fmwr_data_create(ctx, n, p, nnz, row_size, col_idx, value, labels, &dg.d)) throw Error(FMWR_ERR_ARG, g_last_error);
     if (fmwr_model_create(ctx, cfg, p, precision, &mg.m)) throw Error(FMWR_ERR_ARG, g_last_error);
     // Tracker::report (reference src/core/Tracker.h:70-94): forward + metric per snapshot
-    int link;
-    if (cfg->task == FMWR_REGRESSION) link = FMWR_LINK_CLAMP;
-    else link = (solver == FMWR_MCMC || solver == FMWR_ALS) ? FMWR_LINK_PROBIT_TABLE : FMWR_LINK_LOGISTIC;
+    const int link = tracker_link(cfg->task, solver);
     std::vector<double> zw(p > 0 ? p : 1, 0.0), zv((size_t)(p > 0 ? p : 1) * (cfg->k > 0 ? cfg->k : 1), 0.0);
     for (int i = 0; i < n_snap; ++i) {
       const double* wi = snap_w ? snap_w + (size_t)i * p : zw.data();

@@ -434,17 +434,32 @@ struct Holdout {
   int patience;                       // > 0: stop after this many records in a row without an improvement on eval[0]
   int32_t* best_rec;                  // out: the first record with the best eval[0] score, -1 if every score was NaN
 };
-// One training call's held-out state.  The trainers call record() right after tracker_snapshot and finish() after their
-// loop (before the final synchronise); with h == nullptr both do nothing.
-struct HoldoutRun {
-  const Holdout* h;
-  double best = 0.0;
+// ---- tracker (tracker.cu): the reference's Tracker (src/core/Tracker.h), shared by the three trainers ----
+int tracker_link(int task, int solver);                                                      // the link of the tracker's scores
+double tracker_score(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s);   // train metric of m on d
+// One training call's records.  The trainer asks due() (after sample idx in exact mode, at the start of sweep idx in ALS/MCMC)
+// or due_after_batch() (minibatch mode: one record per step samples crossed, and at the end) and passes the train score to
+// record(): snapshot, convergence rule (SGD/FTRL/TDAP, from the third record on), held-out scores, best copy and patience; true
+// means stop.  After its loop it calls restore_best() before its final synchronise and write_trace() after it.  m is the model
+// the loop trains (the fp64 shadow of an fp32 ALS/MCMC handle), so snapshots, held-out scores and the best copy come from it.
+struct Tracker {
+  const int step;                     // step_size after Tracker::init's MAX_REC rule; <= 0: no records
+  Tracker(fmwr_ctx* ctx, fmwr_model* m, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* h);
+  bool due(int64_t idx) const { return step > 0 && (idx % step == 0 || idx == s->max_iter - 1); }
+  bool due_after_batch(int64_t iter);
+  bool record(int64_t idx, double score);
+  void restore_best();                // held-out tracking: best_rec out, and the best record's (w0, w, V) when select_best
+  void write_trace(int64_t iters_done);
+ private:
+  fmwr_ctx* ctx; fmwr_model* m; const fmwr_solver_cfg* s; fmwr_trace* tr; const Holdout* h;
+  int n_rec = 0, conv_times = 0, convergent = 0;
+  double old_score = 0.0;
+  int64_t next_track = 0;             // minibatch mode: the sample count a batch must pass for the next record
+  double best = 0.0;                  // held-out tracking: best eval[0] score so far
   int best_rec = -1, since = 0;       // since: records after best_rec
-  DBuf<char> w, v;                    // device copy of the best record's w [p] and V [p][kp], the model's own type
-  DBuf<double> w0;
-  explicit HoldoutRun(const Holdout* h_) : h(h_) {}
-  bool record(fmwr_ctx* ctx, fmwr_model* m, const fmwr_solver_cfg* s, int rec);   // true: patience says stop
-  void finish(fmwr_ctx* ctx, fmwr_model* m);
+  DBuf<char> best_w, best_v;          // device copy of the best record's w [p] and V [p][kp], the model's own type
+  DBuf<double> best_w0;
+  bool record_holdout();              // true: patience says stop
 };
 void train_exact(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* holdout = nullptr);
 void train_minibatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* holdout = nullptr);

@@ -21,10 +21,6 @@
 
 namespace fmwr {
 
-double tracker_score(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s);
-void tracker_snapshot(fmwr_model* m, fmwr_trace* tr, int idx, int iter, double score);
-int tracker_step_size(int step_size, int max_iter);
-
 template <class T> struct Vec2;
 template <> struct Vec2<float> { typedef float2 type; };
 template <> struct Vec2<double> { typedef double2 type; };
@@ -1406,7 +1402,7 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
   // posterior mean: f64 sums of the predict.FM prediction of every averaged draw (the MCMC link of tracker_score) -- the
   // training rows in the order e has, then each eval set.  Draw t is the model after t sweeps: at sweep t, right after the
   // forward, e holds its raw score; the eval sets get a predict of their own.  None of it feeds back into the chain.
-  const int post_link = cls ? FMWR_LINK_PROBIT_TABLE : FMWR_LINK_CLAMP;
+  const int post_link = tracker_link(m->cfg.task, s->solver);
   DBuf<double> post_acc;
   std::vector<int64_t> post_off;           // [n_eval + 2] offsets into post_acc
   if (post) {
@@ -1431,23 +1427,11 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
   T* wp = (T*)m->w.p;
   T* vp = (T*)m->v.p;
   double* scal = (double*)m->scal.p;
-  const int step = tracker_step_size(s->step_size, s->max_iter);
-  int ii = -1, n_rec = 0;
+  Tracker trk(ctx, m, s, tr, holdout);
   int sweep = 0;
-  HoldoutRun ho(holdout);
   for (; sweep < s->max_iter; ++sweep) {
-    // tracker (:101-124): train metric of the model at the start of the sweep
-    if (step > 0) {
-      ii++;
-      if (ii == step) ii = 0;
-      if (ii == 0 || sweep == s->max_iter - 1) {
-        const double score = tracker_score(ctx, m, d, s);
-        tracker_snapshot(m, tr, n_rec, sweep, score);
-        const bool patience_stop = ho.record(ctx, m, s, n_rec);
-        n_rec++;
-        if (patience_stop) break;            // decided at the start of the sweep: this sweep does not run
-      }
-    }
+    // tracker (:101-124): train metric of the model at the start of the sweep; a stop decided there skips the sweep
+    if (trk.due(sweep) && trk.record(sweep, tracker_score(ctx, m, d, s))) break;
     // e <- predict_batch (:100), q[r][f] <- S_f
     const bool perm_rows = use_rm && dl.ok && dl.permuted;     // e, q, labels in permuted row order (see DenseLayout)
     const float* yp = perm_rows ? dl.py.p : d->y.p;
@@ -1585,10 +1569,10 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
       dd->pred_prec = FMWR_F64;
     }
   }
-  ho.finish(ctx, m);
+  trk.restore_best();
   FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
   if (ctx->world > 1) peer_check_error(ctx);      // a timed-out exchange means partial (A,B) sums: the replicas have diverged
-  if (tr) { tr->n_rec = std::min(n_rec, (int)tr->max_rec); tr->convergent = 0; tr->iters_done = sweep; }
+  trk.write_trace(sweep);
 }
 
 // ---- precision policy ------------------------------------------------------------------------------------------------------
