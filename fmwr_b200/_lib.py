@@ -369,6 +369,19 @@ def predict_fetch(ctx, data):
     return out
 
 
+def contrib_dev(ctx, model, data):
+    """per-entry contributions of the raw score on the device; the raw score becomes data's forward result (predict_fetch)"""
+    check(lib().fmwr_contrib_dev(ctx.h, model.h, data.h))
+
+
+def contrib_fetch(ctx, data):
+    """the contributions of the last contrib_dev on data, f64[nnz] in CSR entry order"""
+    nnz = data.shape()[2]
+    out = np.zeros(nnz)
+    check(lib().fmwr_contrib_fetch(ctx.h, data.h, ptr(out)))
+    return out
+
+
 def evaluate_dev(ctx, data, task, metric):
     out = C.c_double()
     check(lib().fmwr_evaluate_dev(ctx.h, data.h, C.c_int32(task), C.c_int32(metric), C.byref(out)))

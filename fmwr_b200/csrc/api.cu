@@ -760,6 +760,29 @@ int fmwr_predict_fetch(fmwr_ctx* ctx, fmwr_data* d, double* out)
   });
 }
 
+int fmwr_contrib_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d)
+{
+  return guarded([&] {
+    FMWR_REQUIRE(ctx && m && d, FMWR_ERR_ARG, "null argument");
+    FMWR_REQUIRE(!(ctx->nccl_comm && ctx->world > 1), FMWR_ERR_UNSUPPORTED, "contributions run on one GPU (a column slice holds partial S_f)");
+    FMWR_CUDA(cudaSetDevice(ctx->device));
+    contrib_launch(ctx, m, d);
+  });
+}
+
+int fmwr_contrib_fetch(fmwr_ctx* ctx, fmwr_data* d, double* out)
+{
+  return guarded([&] {
+    FMWR_REQUIRE(ctx && d && (out || d->nnz == 0), FMWR_ERR_ARG, "null argument");
+    FMWR_REQUIRE(d->contrib64.p, FMWR_ERR_ARG, "no contributions on the device (fmwr_contrib_dev has not run on this data)");
+    FMWR_CUDA(cudaSetDevice(ctx->device));
+    if (d->nnz == 0) return;
+    ctx->d2h_bytes += 8 * d->nnz;
+    FMWR_CUDA(cudaMemcpyAsync(out, d->contrib64.p, 8 * d->nnz, cudaMemcpyDeviceToHost, ctx->stream));
+    FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
+  });
+}
+
 int fmwr_evaluate_dev(fmwr_ctx* ctx, fmwr_data* d, int32_t task, int32_t metric, double* out)
 {
   return guarded([&] {

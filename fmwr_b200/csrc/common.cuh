@@ -212,6 +212,7 @@ struct fmwr_data {
   int pred_prec = FMWR_F32;
   fmwr::DBuf<float> pred32;      // [n]
   fmwr::DBuf<double> pred64;     // [n]
+  fmwr::DBuf<double> contrib64;  // [nnz] per-entry contributions of the last fmwr_contrib_dev (allocated by its first call)
   double min_y = 0, max_y = 0;
   int64_t min_col_nnz = -1;      // smallest non-zero column count (-1: not computed yet); train_als.cu precision policy
 };
@@ -414,6 +415,7 @@ int padded_k(int k, int prec);
 // module entry points (implemented across the .cu files)
 void build_link_tables(fmwr_ctx* ctx);
 void forward_launch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, int link, double lo, double hi);
+void contrib_launch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d);   // raw score into pred64, per-entry contributions into contrib64
 void transpose_build(fmwr_data* d);
 void launch_iota(fmwr_ctx* ctx, uint32_t* a, int64_t n);
 // stable LSD radix sort of (key, value) pairs on the low `bits` key bits (sort.cu); val_in == nullptr: values are 0, 1, 2, ...

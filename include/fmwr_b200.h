@@ -216,6 +216,20 @@ int fmwr_model_set_state(fmwr_model* m, int32_t solver, int32_t n_state, const d
  * (src/util/Random.h:95-111); CLAMP to [lo, hi] (src/FM.cpp:204-210).  Result stays on the device. */
 int fmwr_predict_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, int32_t link, double lo, double hi);
 int fmwr_predict_fetch(fmwr_ctx* ctx, fmwr_data* d, double* out /*[n]*/);
+/* Per-feature contributions of the score (extension: xgboost's predcontrib / LightGBM's pred_contrib).  For entry j of a row
+ *   phi_j = [k1] w_j x_j + 1/2 x_j ( sum_f v_jf S_f - x_j sum_f v_jf^2 ),   S_f = sum_l v_lf x_l,   phi_0 = [k0] w0 (every row),
+ * the exact Shapley values of the game v(T) = score of the row with every entry outside T set to 0 (a pairwise term gives half of
+ * its interaction to each of its two features), so  phi_0 + sum_j phi_j = [k0] w0 + [k1] sum_j w_j x_j + sum_{j<l} <v_j,v_l> x_j x_l,
+ * the raw score.  They are on the raw-score (margin) scale: the logistic, probit-table and clamp links are not additive.  They are
+ * computed from the values the handle holds, which are z-scored when it was normalised; an explicitly stored zero gets phi = 0.
+ * fmwr_contrib_dev computes phi_j for every entry of d (arithmetic in the model's type, results f64) and leaves the raw score as
+ * d's forward result (fmwr_predict_fetch / fmwr_evaluate_dev read it; it equals fmwr_predict_dev(..., FMWR_LINK_NONE) up to
+ * summation order).  fmwr_contrib_fetch copies the contributions out in the handle's CSR entry order -- that of value / col_idx
+ * of the fm.matrix.  Errors leave the handle untouched: FMWR_ERR_ARG (a null argument; a fetch before any fmwr_contrib_dev on d),
+ * FMWR_ERR_SHAPE (d has another feature count, the predict message), FMWR_ERR_UNSUPPORTED (a communicator with world > 1: a
+ * column slice holds partial S_f). */
+int fmwr_contrib_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d);
+int fmwr_contrib_fetch(fmwr_ctx* ctx, fmwr_data* d, double* out /*[nnz]*/);
 /* train-set metric of the last fmwr_predict_dev result (src/core/Evaluation.h:20-115) */
 int fmwr_evaluate_dev(fmwr_ctx* ctx, fmwr_data* d, int32_t task, int32_t metric, double* out);
 
