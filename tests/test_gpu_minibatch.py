@@ -6,6 +6,7 @@ import pytest
 from oracle import oracle as O
 from fmwr_b200 import _lib as L
 from fmwr_b200 import synth
+from tests import minibatch_cases as MC
 from tests.util import relerr
 
 pytestmark = pytest.mark.gpu
@@ -98,9 +99,16 @@ def test_minibatch_deterministic_and_truncated_tail(gpu_ctx):
     b, pb, tb = mb_train(gpu_ctx, L.F32, ds, ds["y"], L.CLASSIFICATION, L.FTRL, k, 0.0, w, v, iters, 512)
     assert ta["iters_done"] == iters
     assert a[0] == b[0] and np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
-    # rows beyond the truncation point of the last batch were not applied: compare with a run whose data stops there
-    cut = 1 + (iters - 4999)                 # second epoch visits rows 1 .. cut-1... of which full batches + tail
     assert np.isfinite(a[2]).all() and np.isfinite(pa).all()
+    # the second epoch stops 210 rows into its third batch: only those rows are applied.  The fp64 reference of the batch step
+    # on the same inputs (tests/minibatch_cases.py: truncated_tail_case) holds the run to that; applying the whole third batch
+    # moves the result by > 1 (tests/test_minibatch_reference.py)
+    c = MC.truncated_tail_case()
+    assert c["max_iter"] == iters and c["B"] == 512 and np.array_equal(c["v"], v.astype(np.float32).astype(np.float64))
+    want = MC.reference(c)
+    err = max(relerr(a[0], want["w0"]), relerr(a[1], want["w"]), relerr(a[2], want["v"]))
+    print("truncated tail against the reference: max relerr %.3g (tolerance %.1g)" % (err, c["tol"]))
+    assert err <= c["tol"], err
 
 
 def test_minibatch_hot_feature_segments(gpu_ctx, port):
