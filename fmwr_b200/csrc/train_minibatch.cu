@@ -22,7 +22,6 @@
 
 namespace fmwr {
 
-int solver_state_count(const SolverParams<double>& sp);
 void comm_allreduce_sum(fmwr_ctx* ctx, void* buf, size_t count, bool f64);
 
 // ---- K1: forward + multiplier + S cache --------------------------------------------------------
@@ -242,38 +241,21 @@ __device__ __forceinline__ void mb_intercept(const MbUpdArgs<T>& a)
   if (threadIdx.x == 0) {
     double gsum = 0;
     for (int i = 0; i < (nt >> 5); ++i) gsum += red[i];
-    double* sc = a.scal;
-    if (SOLVER == FMWR_SGD) {
-      if (a.k0) sc[0] -= (double)sp.lr * (gsum / (double)a.rows + (double)sp.reg_w0 * sc[0]);
-    } else if (SOLVER == FMWR_FTRL) {
-      if (a.k0) {
-        const double old = sc[2];
-        sc[2] += gsum * gsum;
-        const double delta = (sqrt(sc[2]) - sqrt(old)) / (double)sp.alpha_w;
-        sc[1] += gsum - delta * sc[0];
-      }
-      sc[0] = -sc[1] * (double)sp.alpha_w / ((double)sp.beta_w + sqrt(sc[2]));
-    } else {
-      if (a.k0) {
-        const double old = sc[1];
-        sc[1] += gsum * gsum; sc[2] += gsum;
-        const double sigma = (sqrt(sc[1]) - sqrt(old)) / (double)sp.alpha_w;
-        sc[3] = (double)sp.egamma * (sc[3] + sigma);
-        sc[4] = (double)sp.egamma * (sc[4] + sigma * sc[0]);
-        sc[5] = sc[2] - sc[4];
-      }
-      sc[0] = -sc[5] / sc[3];
-    }
+    double s[6];
+    for (int i = 0; i < 6; ++i) s[i] = a.scal[i];
+    double sq = SOLVER == FMWR_SGD ? 0.0 : sqrt(SOLVER == FMWR_FTRL ? s[2] : s[1]);
+    intercept_step<T, SOLVER, false>(s, SOLVER == FMWR_SGD ? gsum / (double)a.rows : gsum, a.k0, sq, sp);
+    for (int i = 0; i < 6; ++i) a.scal[i] = s[i];
   }
 }
 
 // Everything a segment needs that depends only on its 16-byte record {feature, length, first row, first value}:
 // the parameter row, its optimizer state, the first row's S-cache line and multiplier, and the next LPR entries
 // of the segment (lane l fetches entry 1 + l).  seg_issue requests all of it in one go; seg_finish consumes it.
-template <class T, int CH, int NST>
+template <class T, int CH, int SOLVER>
 struct SegStage {
-  typename Vec<T>::type th[CH], s0[CH], st[NST][CH];
-  T m0, tw, stw[NST];
+  typename Vec<T>::type th[CH], s0[CH], st[solver_nst(SOLVER)][CH];
+  T m0, tw, stw[solver_nst(SOLVER)];
   uint32_t c, len, eb, r0, my_r;
   float x0, my_x;
   bool live;
@@ -281,11 +263,11 @@ struct SegStage {
 
 template <class T, int LPR, int CH, int SOLVER, bool L1>
 __device__ __forceinline__ void seg_issue(const MbUpdArgs<T>& a, const uint4 rec, const uint32_t eb, const int l, bool live,
-                                          SegStage<T, CH, (SOLVER == FMWR_SGD ? 1 : (SOLVER == FMWR_FTRL ? 2 : 4))>& sg)
+                                          SegStage<T, CH, SOLVER>& sg)
 {
   typedef typename Vec<T>::type V16;
   constexpr int VN = Vec<T>::N;
-  constexpr int NST = SOLVER == FMWR_SGD ? 1 : (SOLVER == FMWR_FTRL ? 2 : 4);
+  constexpr int NST = solver_nst(SOLVER);
   constexpr bool USE_STATE = SOLVER != FMWR_SGD || L1;
   sg.c = rec.x; sg.len = rec.y; sg.eb = eb; sg.x0 = __uint_as_float(rec.w);
   sg.r0 = rec.z - (uint32_t)a.row_begin;
@@ -320,19 +302,14 @@ __device__ __forceinline__ void seg_issue(const MbUpdArgs<T>& a, const uint4 rec
 }
 
 template <class T, int LPR, int CH, int SOLVER, bool L1>
-__device__ __forceinline__ void seg_finish(const MbUpdArgs<T>& a, const int g, const int l,
-                                           SegStage<T, CH, (SOLVER == FMWR_SGD ? 1 : (SOLVER == FMWR_FTRL ? 2 : 4))>& sg)
+__device__ __forceinline__ void seg_finish(const MbUpdArgs<T>& a, const int g, const int l, SegStage<T, CH, SOLVER>& sg)
 {
   typedef typename Vec<T>::type V16;
   constexpr int VN = Vec<T>::N;
-  constexpr int NST = SOLVER == FMWR_SGD ? 1 : (SOLVER == FMWR_FTRL ? 2 : 4);
+  constexpr int NST = solver_nst(SOLVER);
+  constexpr bool USE_STATE = SOLVER != FMWR_SGD || L1;
   constexpr bool FAST = sizeof(T) == 4;
-  // TDAP keeps the per-entry gradient form of the exact mode (see fm_grad: a rounding residue flips theta by +-alpha);
-  // SGD / FTRL sum  A_f = sum_r (m_r x_r) S_rf  and  b = sum_r m_r x_r^2  and form  G_f = A_f - v_f b  once (the same
-  // value up to rounding; at batch = 1 it differs from the exact mode's per-entry form by an ulp, not by a step)
-  constexpr bool ENTRY_FORM = SOLVER == FMWR_TDAP;
   if (!sg.live) return;
-  const SolverParams<T>& sp = a.sp;
   const uint32_t c = sg.c, len = sg.len, eb = sg.eb;
   const uint32_t rb32 = (uint32_t)a.row_begin, nrows = (uint32_t)a.rows;
   const size_t off = (size_t)c * a.kp + l * VN;
@@ -341,18 +318,10 @@ __device__ __forceinline__ void seg_finish(const MbUpdArgs<T>& a, const int g, c
   uint32_t my_r = sg.my_r;
   float my_x = sg.my_x;
 
-  T th[CH][VN], Gv[CH][VN];
-  const T x0 = T(sg.x0), m0 = sg.m0;
-  const T mx0 = m0 * x0;
-  T Gw = mx0, bsum = mx0 * x0;
+  T th[CH][VN], Gv[CH][VN], Gw, bsum;
 #pragma unroll
-  for (int ch = 0; ch < CH; ++ch) {
-    T s[VN];
-    vec_to_arr(sg.th[ch], th[ch]);
-    vec_to_arr(sg.s0[ch], s);
-#pragma unroll
-    for (int k2 = 0; k2 < VN; ++k2) Gv[ch][k2] = ENTRY_FORM ? m0 * fm_grad(s[k2], th[ch][k2], x0) : mx0 * s[k2];
-  }
+  for (int ch = 0; ch < CH; ++ch) vec_to_arr(sg.th[ch], th[ch]);
+  seg_grad_entry<SOLVER, true>(Gw, bsum, Gv, th, sg.m0, T(sg.x0), sg.s0);
   for (uint32_t base = 1; base < len; base += LPR) {
     if (base > 1) {
       my_r = 0xffffffffu; my_x = 0.f;
@@ -375,79 +344,31 @@ __device__ __forceinline__ void seg_finish(const MbUpdArgs<T>& a, const int g, c
         for (int ch = 0; ch < CH; ++ch) se[u][ch] = reinterpret_cast<const V16*>(sr)[ch * LPR];
       }
 #pragma unroll
-      for (int u = 0; u < UE; ++u) {
-        const T mxe = me[u] * xe[u];
-        Gw += mxe;
-        if (!ENTRY_FORM) bsum += mxe * xe[u];
-#pragma unroll
-        for (int ch = 0; ch < CH; ++ch) {
-          T s[VN];
-          vec_to_arr(se[u][ch], s);
-#pragma unroll
-          for (int k2 = 0; k2 < VN; ++k2) {
-            if (ENTRY_FORM) Gv[ch][k2] += me[u] * fm_grad(s[k2], th[ch][k2], xe[u]);
-            else Gv[ch][k2] += mxe * s[k2];
-          }
-        }
-      }
+      for (int u = 0; u < UE; ++u) seg_grad_entry<SOLVER>(Gw, bsum, Gv, th, me[u], xe[u], se[u]);
     }
   }
-  if (!ENTRY_FORM) {
-#pragma unroll
-    for (int ch = 0; ch < CH; ++ch)
-#pragma unroll
-      for (int k2 = 0; k2 < VN; ++k2) Gv[ch][k2] = Gv[ch][k2] - th[ch][k2] * bsum;
-  }
+  seg_grad_close<SOLVER>(Gv, th, bsum);
 
   // ---- linear weight (lane 0 of the group)
   if (a.k1 && l == 0) {
-    T tw = sg.tw;
-    if (SOLVER == FMWR_SGD) {
-      T q = sg.stw[0];
-      tw = sgd_step(tw, Gw, sp.lr, sp.reg_w, L1 ? 1 : 0, a.u_w, q);
-      if (L1) a.sw[0][c] = q;
-    } else if (SOLVER == FMWR_FTRL) {
-      tw = ftrl_step<T, FAST>(tw, Gw, sg.stw[0], sg.stw[1 % NST], sp.alpha_w, sp.beta_w, sp.l1_w, sp.l2_w);
-      a.sw[0][c] = sg.stw[0]; a.sw[1][c] = sg.stw[1 % NST];
-    } else {
-      const T z = tdap_state<T, FAST>(tw, Gw, sg.stw[0], sg.stw[1 % NST], sg.stw[2 % NST], sg.stw[3 % NST], sp.alpha_w, sp.egamma);
-      a.sw[0][c] = sg.stw[0]; a.sw[1][c] = sg.stw[1 % NST]; a.sw[2][c] = sg.stw[2 % NST]; a.sw[3][c] = sg.stw[3 % NST];
-      tw = tdap_refresh<T, FAST>(z, sg.stw[2 % NST], sp.l1_w, sp.l2_w);
+    a.w[c] = coord_step<T, SOLVER, true, FAST, false>(sg.tw, Gw, sg.stw, a.sp, L1, a.u_w);
+    if (USE_STATE) {
+#pragma unroll
+      for (int k = 0; k < NST; ++k) a.sw[k][c] = sg.stw[k];
     }
-    a.w[c] = tw;
   }
   // ---- factors
 #pragma unroll
   for (int ch = 0; ch < CH; ++ch) {
-    if (SOLVER == FMWR_SGD) {
-      T q[VN];
-      if (L1) vec_to_arr(sg.st[0][ch], q);
+    T st[NST][VN] = {};
+    if (USE_STATE) {
 #pragma unroll
-      for (int i = 0; i < VN; ++i) {
-        T qq = L1 ? q[i] : T(0);
-        th[ch][i] = sgd_step(th[ch][i], Gv[ch][i], sp.lr, sp.reg_v, L1 ? 1 : 0, a.u_v, qq);
-        if (L1) q[i] = qq;
-      }
-      if (L1) reinterpret_cast<V16*>(a.sv[0] + off)[ch * LPR] = arr_to_vec(q);
-    } else if (SOLVER == FMWR_FTRL) {
-      T z[VN], nn[VN];
-      vec_to_arr(sg.st[0][ch], z); vec_to_arr(sg.st[1 % NST][ch], nn);
+      for (int k = 0; k < NST; ++k) vec_to_arr(sg.st[k][ch], st[k]);
+    }
+    coord_step<T, SOLVER, false, FAST, false>(th[ch], Gv[ch], st, a.sp, L1, a.u_v);
+    if (USE_STATE) {
 #pragma unroll
-      for (int i = 0; i < VN; ++i) th[ch][i] = ftrl_step<T, FAST>(th[ch][i], Gv[ch][i], z[i], nn[i], sp.alpha_v, sp.beta_v, sp.l1_v, sp.l2_v);
-      reinterpret_cast<V16*>(a.sv[0] + off)[ch * LPR] = arr_to_vec(z);
-      reinterpret_cast<V16*>(a.sv[1] + off)[ch * LPR] = arr_to_vec(nn);
-    } else {
-      T u[VN], nu[VN], dl[VN], h[VN];
-      vec_to_arr(sg.st[0][ch], u); vec_to_arr(sg.st[1 % NST][ch], nu); vec_to_arr(sg.st[2 % NST][ch], dl); vec_to_arr(sg.st[3 % NST][ch], h);
-#pragma unroll
-      for (int i = 0; i < VN; ++i) {
-        const T z = tdap_state<T, FAST>(th[ch][i], Gv[ch][i], u[i], nu[i], dl[i], h[i], sp.alpha_v, sp.egamma);
-        th[ch][i] = tdap_refresh<T, FAST>(z, dl[i], sp.l1_v, sp.l2_v);
-      }
-      reinterpret_cast<V16*>(a.sv[0] + off)[ch * LPR] = arr_to_vec(u);
-      reinterpret_cast<V16*>(a.sv[1] + off)[ch * LPR] = arr_to_vec(nu);
-      reinterpret_cast<V16*>(a.sv[2] + off)[ch * LPR] = arr_to_vec(dl);
-      reinterpret_cast<V16*>(a.sv[3] + off)[ch * LPR] = arr_to_vec(h);
+      for (int k = 0; k < NST; ++k) reinterpret_cast<V16*>(a.sv[k] + off)[ch * LPR] = arr_to_vec(st[k]);
     }
     reinterpret_cast<V16*>(a.v + off)[ch * LPR] = arr_to_vec(th[ch]);
   }
@@ -462,7 +383,6 @@ template <class T, int LPR, int CH, int SOLVER, bool L1>
 __global__ void __launch_bounds__(256, (sizeof(T) == 4 && CH == 1) ? K2Tune<SOLVER>::BLOCKS : 1) mb_update_kernel(MbUpdArgs<T> a)
 {
   constexpr int G = 32 / LPR;
-  constexpr int NST = SOLVER == FMWR_SGD ? 1 : (SOLVER == FMWR_FTRL ? 2 : 4);
   if (a.peer) peer_wait(a.pa, PEER_FLAG2, PEER_EPOCH2);
   if (blockIdx.x == 0) { mb_intercept<T, SOLVER>(a); return; }
   const int lane = threadIdx.x & 31;
@@ -473,7 +393,7 @@ __global__ void __launch_bounds__(256, (sizeof(T) == 4 && CH == 1) ? K2Tune<SOLV
   for (uint32_t seg = a.seg_begin + ((blockIdx.x - 1) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * G + g; seg < a.seg_end; seg += stride) {
     const uint4 rec = __ldg(a.seg_rec + seg);
     const uint32_t eb = __ldg(a.seg_ptr + seg);
-    SegStage<T, CH, NST> sg;
+    SegStage<T, CH, SOLVER> sg;
     seg_issue<T, LPR, CH, SOLVER, L1>(a, rec, eb, l, true, sg);
     seg_finish<T, LPR, CH, SOLVER, L1>(a, g, l, sg);
   }
@@ -489,7 +409,7 @@ __global__ void __launch_bounds__(TM_THREADS, MINB) mb_update_tma_kernel(MbUpdAr
 {
   typedef TmGeom<T, LPR, CH, SOLVER, L1, TS, NS> G;
   constexpr int GRP = 32 / LPR;                         // lane groups (segments) per warp
-  constexpr int NSTW = G::NST;
+  constexpr int NSTW = solver_nst(SOLVER);
   extern __shared__ __align__(128) unsigned char tm_smem[];
   unsigned char* stages = tm_smem;
   uint32_t* hdr_all = reinterpret_cast<uint32_t*>(tm_smem + NS * G::STAGE_BYTES);
@@ -625,7 +545,7 @@ __global__ void __launch_bounds__(TM_THREADS, MINB) mb_update_tma_kernel(MbUpdAr
         const bool live = j < ns;
         const uint4 rec = live ? reinterpret_cast<const uint4*>(st + G::OFF_REC)[j] : make_uint4(0u, 0u, 0xffffffffu, 0u);
         const uint32_t eb = live ? reinterpret_cast<const uint32_t*>(st + G::OFF_SEGP)[hdr[3] + j] : 0u;
-        SegStage<T, CH, NSTW> sg;
+        SegStage<T, CH, SOLVER> sg;
         seg_issue<T, LPR, CH, SOLVER, L1>(a, rec, eb, l, live, sg);
         seg_finish<T, LPR, CH, SOLVER, L1>(a, g, l, sg);
       }
@@ -747,19 +667,6 @@ void MbLaunch<T>::k1()
                 m->cfg.task, TT(s->min_target), TT(s->max_target), row_begin, rows, mult, Scache, s_stride, partial, pa);
 }
 
-template <class T>
-static SolverParams<T> params_from(const SolverParams<double>& d)
-{
-  SolverParams<T> sp;
-  sp.solver = d.solver; sp.l1 = d.l1;
-  sp.lr = T(d.lr); sp.reg_w = T(d.reg_w); sp.reg_v = T(d.reg_v); sp.reg_w0 = T(d.reg_w0);
-  sp.alpha_w = T(d.alpha_w); sp.alpha_v = T(d.alpha_v); sp.beta_w = T(d.beta_w); sp.beta_v = T(d.beta_v);
-  sp.l1_w = T(d.l1_w); sp.l1_v = T(d.l1_v); sp.l2_w = T(d.l2_w); sp.l2_v = T(d.l2_v); sp.egamma = T(d.egamma);
-  return sp;
-}
-
-SolverParams<double> make_params_f64(const fmwr_model* m, const fmwr_solver_cfg* s);
-
 // Tracker on a feature-sharded model (reference: the full predict_batch + metric inside the epoch, src/solver/SGD_Learner.h:140-166).
 // Nothing is gathered: every rank forwards ITS column slice over all rows in chunks, the chunk's partials (S_f, additive scalar) are
 // summed over the ranks, and every rank finishes score -> link -> metric on the identical totals, so all ranks record the same value.
@@ -824,7 +731,7 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
     train_minibatch_t<T>(ctx, m, visited.get(), &s2, tr, holdout, eval_d);
     return;
   }
-  const SolverParams<double> spd = make_params_f64(m, s);
+  const SolverParams<double> spd = make_params<double>(m, s);
   const bool kept_state = model_alloc_state(m, solver_state_count(spd), s->solver, s->warm_state != 0);
 
   const int64_t row0 = (s->compat & FMWR_COMPAT_SKIP_ROW0) ? 1 : 0;     // F5: the reference scan starts at row 1
@@ -877,7 +784,7 @@ static void train_minibatch_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const 
   ua.w = (T*)m->w.p; ua.v = (T*)m->v.p; ua.scal = (double*)m->scal.p;
   for (int i = 0; i < 4; ++i) { ua.sw[i] = (T*)m->sw[i].p; ua.sv[i] = (T*)m->sv[i].p; }
   ua.kp = m->kp; ua.k0 = m->cfg.keep_w0; ua.k1 = m->cfg.keep_w1; ua.s_stride = s_stride;
-  ua.sp = params_from<T>(spd);
+  ua.sp = make_params<T>(m, s);
 
   const int64_t max_iter = s->max_iter;
   Tracker trk(ctx, m, s, tr, holdout);

@@ -6,8 +6,8 @@
 // array are ONE contiguous range each.  This kernel moves those ranges with 1-D bulk copies (cp.async.bulk, completion on an
 // mbarrier) into a shared-memory ring, lets the lane groups update them in place in shared memory, and writes the ranges back
 // with bulk stores: HBM sees full-line streams in both directions and no warp holds a DRAM round trip in registers.  A
-// producer warp runs the ring (loads, write-backs); eight consumer warps do the arithmetic of seg_finish (train_minibatch.cu)
-// on shared memory.  The only global gathers left in the consumers are the S-cache lines of the segment's rows (L2-resident).
+// producer warp runs the ring (loads, write-backs); eight consumer warps run the segment gradient and the coordinate steps of
+// coord.cuh on shared memory.  The only global gathers left in the consumers are the S-cache lines of the segment's rows (L2-resident).
 // Tiles whose row range is too wide for a stage (sparse batches, huge fields) fall back to the gather path of the original
 // kernel, segment by segment -- results are identical either way (same per-segment arithmetic, same order).
 #pragma once
@@ -63,9 +63,8 @@ template <class T, int LPR, int CH, int SOLVER, bool L1, int TS_, int NS_>
 struct TmGeom {
   enum {
     TS = TS_, NS = NS_,
-    NST = SOLVER == FMWR_SGD ? 1 : (SOLVER == FMWR_FTRL ? 2 : 4),
     USE_STATE = (SOLVER != FMWR_SGD || L1) ? 1 : 0,
-    NA = 1 + (USE_STATE ? NST : 0),                 // theta + state arrays
+    NA = 1 + (USE_STATE ? solver_nst(SOLVER) : 0),                 // theta + state arrays
     RMAX = TS + TS / 2 + TS / 4,                    // rows a stage can hold: the tile's feature range may be 1.75x its segment count
     EMAX = 6 * TS,                                  // entries a stage can hold (the first entry of a segment sits in its record too)
     ROWB = LPR * CH * 16,                           // bytes of one parameter row (kp elements)
@@ -81,17 +80,16 @@ struct TmGeom {
   };
 };
 
-// One segment of a dense tile: same arithmetic as seg_finish (train_minibatch.cu), operands from the stage.
+// One segment of a dense tile: the segment gradient and the steps of coord.cuh, as seg_finish (train_minibatch.cu), with the
+// entry lists and the parameter rows read from the stage.
 template <class T, int LPR, int CH, int SOLVER, bool L1, class G>
 __device__ __forceinline__ void seg_dense(const MbUpdArgs<T>& a, unsigned char* __restrict__ stage, const uint32_t* __restrict__ hdr, int j, int l)
 {
   typedef typename Vec<T>::type V16;
   constexpr int VN = Vec<T>::N;
-  constexpr int NST = G::NST;
+  constexpr int NST = solver_nst(SOLVER);
   constexpr bool USE_STATE = G::USE_STATE != 0;
   constexpr bool FAST = sizeof(T) == 4;
-  constexpr bool ENTRY_FORM = SOLVER == FMWR_TDAP;
-  const SolverParams<T>& sp = a.sp;
   const uint4 rec = reinterpret_cast<const uint4*>(stage + G::OFF_REC)[j];
   const uint32_t c = rec.x, len = rec.y;
   const uint32_t rb32 = (uint32_t)a.row_begin, nrows = (uint32_t)a.rows;
@@ -133,90 +131,38 @@ __device__ __forceinline__ void seg_dense(const MbUpdArgs<T>& a, unsigned char* 
       for (int ch = 0; ch < CH; ++ch) se[u][ch] = reinterpret_cast<const V16*>(sr)[ch * LPR];
     }
 #pragma unroll
-    for (int u = 0; u < UE; ++u) {
-      const T mxe = me[u] * xe[u];
-      Gw += mxe;
-      if (!ENTRY_FORM) bsum += mxe * xe[u];
-#pragma unroll
-      for (int ch = 0; ch < CH; ++ch) {
-        T s[VN];
-        vec_to_arr(se[u][ch], s);
-#pragma unroll
-        for (int k2 = 0; k2 < VN; ++k2) {
-          if (ENTRY_FORM) Gv[ch][k2] += me[u] * fm_grad(s[k2], th[ch][k2], xe[u]);
-          else Gv[ch][k2] += mxe * s[k2];
-        }
-      }
-    }
+    for (int u = 0; u < UE; ++u) seg_grad_entry<SOLVER>(Gw, bsum, Gv, th, me[u], xe[u], se[u]);
   };
   round(std::integral_constant<int, 3>(), 0u);
   for (uint32_t i0 = 3; i0 < len; i0 += 2) round(std::integral_constant<int, 2>(), i0);
-  if (!ENTRY_FORM) {
-#pragma unroll
-    for (int ch = 0; ch < CH; ++ch)
-#pragma unroll
-      for (int k2 = 0; k2 < VN; ++k2) Gv[ch][k2] = Gv[ch][k2] - th[ch][k2] * bsum;
-  }
+  seg_grad_close<SOLVER>(Gv, th, bsum);
 
   // ---- linear weight (lane 0 of the group): staged read, direct store
   if (a.k1 && l == 0) {
     const T* wst = reinterpret_cast<const T*>(stage + G::OFF_W) + hdr[6] + rl;
-    T tw = wst[0];
     T stw[NST];
 #pragma unroll
-    for (int st = 0; st < NST; ++st) stw[st] = USE_STATE ? wst[(st + 1) * (G::RMAX + 8)] : T(0);
-    if (SOLVER == FMWR_SGD) {
-      T q = stw[0];
-      tw = sgd_step(tw, Gw, sp.lr, sp.reg_w, L1 ? 1 : 0, a.u_w, q);
-      if (L1) a.sw[0][c] = q;
-    } else if (SOLVER == FMWR_FTRL) {
-      tw = ftrl_step<T, FAST>(tw, Gw, stw[0], stw[1 % NST], sp.alpha_w, sp.beta_w, sp.l1_w, sp.l2_w);
-      a.sw[0][c] = stw[0]; a.sw[1][c] = stw[1 % NST];
-    } else {
-      const T z = tdap_state<T, FAST>(tw, Gw, stw[0], stw[1 % NST], stw[2 % NST], stw[3 % NST], sp.alpha_w, sp.egamma);
-      a.sw[0][c] = stw[0]; a.sw[1][c] = stw[1 % NST]; a.sw[2][c] = stw[2 % NST]; a.sw[3][c] = stw[3 % NST];
-      tw = tdap_refresh<T, FAST>(z, stw[2 % NST], sp.l1_w, sp.l2_w);
+    for (int k = 0; k < NST; ++k) stw[k] = USE_STATE ? wst[(k + 1) * (G::RMAX + 8)] : T(0);
+    a.w[c] = coord_step<T, SOLVER, true, FAST, false>(wst[0], Gw, stw, a.sp, L1, a.u_w);
+    if (USE_STATE) {
+#pragma unroll
+      for (int k = 0; k < NST; ++k) a.sw[k][c] = stw[k];
     }
-    a.w[c] = tw;
   }
   // ---- factors: update the staged rows in place
   constexpr int ASTRIDE = G::RMAX * G::ROWB;       // bytes between the same row of two staged arrays
 #pragma unroll
   for (int ch = 0; ch < CH; ++ch) {
     unsigned char* pr = prow + ch * LPR * 16;
-    if (SOLVER == FMWR_SGD) {
-      T q[VN];
-      if (L1) vec_to_arr(*reinterpret_cast<const V16*>(pr + ASTRIDE), q);
+    T st[NST][VN] = {};
+    if (USE_STATE) {
 #pragma unroll
-      for (int i = 0; i < VN; ++i) {
-        T qq = L1 ? q[i] : T(0);
-        th[ch][i] = sgd_step(th[ch][i], Gv[ch][i], sp.lr, sp.reg_v, L1 ? 1 : 0, a.u_v, qq);
-        if (L1) q[i] = qq;
-      }
-      if (L1) *reinterpret_cast<V16*>(pr + ASTRIDE) = arr_to_vec(q);
-    } else if (SOLVER == FMWR_FTRL) {
-      T z[VN], nn[VN];
-      vec_to_arr(*reinterpret_cast<const V16*>(pr + ASTRIDE), z);
-      vec_to_arr(*reinterpret_cast<const V16*>(pr + 2 * ASTRIDE), nn);
+      for (int k = 0; k < NST; ++k) vec_to_arr(*reinterpret_cast<const V16*>(pr + (k + 1) * ASTRIDE), st[k]);
+    }
+    coord_step<T, SOLVER, false, FAST, false>(th[ch], Gv[ch], st, a.sp, L1, a.u_v);
+    if (USE_STATE) {
 #pragma unroll
-      for (int i = 0; i < VN; ++i) th[ch][i] = ftrl_step<T, FAST>(th[ch][i], Gv[ch][i], z[i], nn[i], sp.alpha_v, sp.beta_v, sp.l1_v, sp.l2_v);
-      *reinterpret_cast<V16*>(pr + ASTRIDE) = arr_to_vec(z);
-      *reinterpret_cast<V16*>(pr + 2 * ASTRIDE) = arr_to_vec(nn);
-    } else {
-      T u[VN], nu[VN], dl[VN], h[VN];
-      vec_to_arr(*reinterpret_cast<const V16*>(pr + ASTRIDE), u);
-      vec_to_arr(*reinterpret_cast<const V16*>(pr + 2 * ASTRIDE), nu);
-      vec_to_arr(*reinterpret_cast<const V16*>(pr + 3 * ASTRIDE), dl);
-      vec_to_arr(*reinterpret_cast<const V16*>(pr + 4 * ASTRIDE), h);
-#pragma unroll
-      for (int i = 0; i < VN; ++i) {
-        const T z = tdap_state<T, FAST>(th[ch][i], Gv[ch][i], u[i], nu[i], dl[i], h[i], sp.alpha_v, sp.egamma);
-        th[ch][i] = tdap_refresh<T, FAST>(z, dl[i], sp.l1_v, sp.l2_v);
-      }
-      *reinterpret_cast<V16*>(pr + ASTRIDE) = arr_to_vec(u);
-      *reinterpret_cast<V16*>(pr + 2 * ASTRIDE) = arr_to_vec(nu);
-      *reinterpret_cast<V16*>(pr + 3 * ASTRIDE) = arr_to_vec(dl);
-      *reinterpret_cast<V16*>(pr + 4 * ASTRIDE) = arr_to_vec(h);
+      for (int k = 0; k < NST; ++k) *reinterpret_cast<V16*>(pr + (k + 1) * ASTRIDE) = arr_to_vec(st[k]);
     }
     *reinterpret_cast<V16*>(pr) = arr_to_vec(th[ch]);
   }
