@@ -42,7 +42,8 @@ class SolverCfg(C.Structure):
                 ("normals", C.c_void_p), ("n_normals", C.c_int64),
                 ("gammas", C.c_void_p), ("n_gammas", C.c_int64),
                 ("rands", C.c_void_p), ("n_rands", C.c_int64),
-                ("seed", C.c_uint64), ("warm_state", C.c_int32)]
+                ("seed", C.c_uint64), ("warm_state", C.c_int32),
+                ("attr_group", C.c_void_p), ("n_groups", C.c_int32)]
 
 
 class Trace(C.Structure):

@@ -258,6 +258,21 @@ def _acquire(ctx, feats, labels, normalized):
     return d, False
 
 
+def _attr_group(g, p):
+    """the optional features$attr_group of an fm.matrix: 0-based group of every column (libFM's feature grouping), checked with
+    the messages of fmwr_solver_cfg's validation; returns (int32 map, number of groups = largest id + 1)"""
+    a = np.asarray(g)
+    if a.ndim != 1 or a.size != p or (a.size and not np.all(np.asarray(a, np.float64) == np.floor(np.asarray(a, np.float64)))):
+        raise ValueError("attr_group must be an integer vector with one entry per column")
+    a = np.ascontiguousarray(a, np.int64)
+    if a.size and a.min() < 0:
+        raise ValueError("attr_group entry out of range [0, n_groups)")
+    n_groups = int(a.max()) + 1 if a.size else 1
+    if n_groups > 65536 or n_groups > p:
+        raise ValueError("n_groups must be at least 1 and at most 65536 and the number of features")
+    return a.astype(np.int32), n_groups
+
+
 def _compat():
     return L.COMPAT_REFERENCE if _OPTIONS["FM.compat"] == "reference" else 0
 
@@ -321,6 +336,10 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
                              metric=L.METRICS[track_controls["evaluate.metric"]], convergence=float(track_controls["convergence"]),
                              seed=int(_OPTIONS["FM.seed"]), warm_state=warm)
             keep = []
+            if name == "MCMC" and feats.get("attr_group") is not None:
+                grp, n_groups = _attr_group(feats["attr_group"], p)
+                keep.append(grp)
+                sc.attr_group = L.ptr(grp); sc.n_groups = n_groups
             if streams:
                 for fld, cnt, dt in (("normals", "n_normals", np.float64), ("gammas", "n_gammas", np.float64), ("rands", "n_rands", np.int32)):
                     if streams.get(fld) is not None:

@@ -296,11 +296,26 @@ static void check_eval_list(const fmwr_model* m, const fmwr_data* d, fmwr_data* 
   for (int i = 0; i < n_eval; ++i) require_same_features(m, eval[i]);
 }
 
+// attribute groups of fmwr_solver_cfg (MCMC only; NULL map: one group)
+static void check_groups(const fmwr_model* m, const fmwr_solver_cfg* s)
+{
+  if (!s->attr_group) {
+    FMWR_REQUIRE(s->n_groups >= 0 && s->n_groups <= 1, FMWR_ERR_ARG, "n_groups > 1 needs an attr_group map");
+    return;
+  }
+  FMWR_REQUIRE(s->solver == FMWR_MCMC, FMWR_ERR_ARG, "attribute groups need the MCMC solver");
+  FMWR_REQUIRE(s->n_groups >= 1 && s->n_groups <= 65536 && s->n_groups <= m->p, FMWR_ERR_ARG,
+               "n_groups must be at least 1 and at most 65536 and the number of features");
+  for (int64_t i = 0; i < m->p; ++i)
+    FMWR_REQUIRE(s->attr_group[i] >= 0 && s->attr_group[i] < s->n_groups, FMWR_ERR_ARG, "attr_group entry out of range [0, n_groups)");
+}
+
 static void train_dispatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr,
                            const Posterior* post = nullptr, const Holdout* holdout = nullptr)
 {
   FMWR_REQUIRE(d->has_labels, FMWR_ERR_ARG, "target's length is not equal the number of cases...");
   FMWR_REQUIRE(d->p == m->p, FMWR_ERR_SHAPE, "there's no the same number of features between train and fm object...");
+  check_groups(m, s);
   if (tr) { tr->n_rec = 0; tr->convergent = 0; tr->iters_done = 0; }
   switch (s->solver) {
     case FMWR_SGD: case FMWR_FTRL: case FMWR_TDAP:

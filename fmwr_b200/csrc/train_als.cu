@@ -12,7 +12,7 @@
 // reference rebuilds per factor at :286-299) -> calculate_error -> alpha -> w0 -> lambda_w -> mu_w -> w
 // [-> lambda_v -> mu_v -> V when enable_v; the shipped code comments that block out, SURVEY F1].
 // Hyper-parameters are the ones MCMC_ALS_Learner::init forces (alpha_0 = gamma_0 = beta_0 = 1, mu_0 = 0,
-// alpha = 1, w0_mean_0 = 0; SURVEY F2), one attribute group (src/FM.cpp:75).
+// alpha = 1, w0_mean_0 = 0; SURVEY F2), one attribute group (src/FM.cpp:75) unless fmwr_solver_cfg::attr_group gives several.
 #include "forward.cuh"
 
 #include <algorithm>
@@ -313,6 +313,134 @@ static void reduce_v_all(fmwr_ctx* ctx, const T* v, int64_t p, int k, int kp, co
   for (int f = 0; f < k; ++f) row0[f] = (double)r0[f];
 }
 
+// ---- attribute groups (fmwr_solver_cfg::attr_group) -----------------------------------------------------------------------
+// The feature ids sorted by group (ascending inside a group) are cut into chunks of at most GRP_CHUNK features that never cross
+// a group boundary.  One CTA per chunk writes part[chunk][f] = sum x_if and part[chunk][kc + f] = sum (x_if - mu[f][g])^2 over
+// its features (w: kc = 1, ld = 1; V: kc = k, ld = kp); the host adds a group's chunk partials in chunk order.  No atomics and
+// a fixed order: row-sharded ranks derive bit-identical priors from their replicated models without an exchange.
+constexpr int GRP_CHUNK = 512;
+
+template <class T>
+__global__ void __launch_bounds__(256) grouped_reduce_kernel(const T* __restrict__ x, int64_t ld, int kc, int n_groups,
+                                                             const uint32_t* __restrict__ feat, const uint32_t* __restrict__ chunk_beg,
+                                                             const int32_t* __restrict__ chunk_grp, const double* __restrict__ mu,
+                                                             double* __restrict__ part)
+{
+  __shared__ double s1[256], s2[256];
+  const int lanes_f = kc < 256 ? kc : 256;
+  const int rows_par = 256 / lanes_f;
+  const int my_f0 = threadIdx.x % lanes_f, my_r = threadIdx.x / lanes_f;
+  const uint32_t c0 = chunk_beg[blockIdx.x], c1 = chunk_beg[blockIdx.x + 1];
+  const int g = chunk_grp[blockIdx.x];
+  for (int fo = 0; fo < kc; fo += lanes_f) {
+    const int f = fo + my_f0;
+    double a1 = 0.0, a2 = 0.0;
+    if (f < kc && my_r < rows_par) {
+      const double m = mu[(size_t)f * n_groups + g];
+      for (uint32_t c = c0 + my_r; c < c1; c += rows_par) {
+        const double v = (double)x[(size_t)feat[c] * ld + f];
+        a1 += v; a2 += (v - m) * (v - m);
+      }
+    }
+    s1[threadIdx.x] = a1; s2[threadIdx.x] = a2;
+    __syncthreads();
+    if (my_r == 0 && f < kc) {
+      for (int r = 1; r < rows_par; ++r) { a1 += s1[r * lanes_f + my_f0]; a2 += s2[r * lanes_f + my_f0]; }
+      part[(size_t)blockIdx.x * 2 * kc + f] = a1;
+      part[(size_t)blockIdx.x * 2 * kc + kc + f] = a2;
+    }
+    __syncthreads();
+  }
+}
+
+struct GroupPrior {
+  int G = 0;
+  std::vector<int64_t> count;                  // [G] p_g
+  std::vector<uint32_t> chunk_beg;             // [n_chunks + 1] offsets into feat
+  std::vector<int32_t> chunk_grp;              // [n_chunks]
+  DBuf<uint16_t> grp;                          // [p] group of every feature
+  DBuf<uint32_t> feat, chunk_beg_dev;          // feature ids sorted by group
+  DBuf<int32_t> chunk_grp_dev;
+  DBuf<double> mu, part;
+  DBuf<double2> prior;                         // [1 + k][G] (lambda, mu): row 0 for w, row 1 + f for factor f
+  std::vector<double> prior_host;              // its host image; outlives every copy out of it (the call does)
+};
+
+static void group_prior_build(fmwr_ctx* ctx, const int32_t* attr_group, int64_t p, int G, int k, GroupPrior& gp)
+{
+  gp.G = G;
+  gp.count.assign(G, 0);
+  for (int64_t i = 0; i < p; ++i) gp.count[attr_group[i]]++;
+  std::vector<int64_t> off(G + 1, 0);
+  for (int g = 0; g < G; ++g) off[g + 1] = off[g] + gp.count[g];
+  std::vector<uint32_t> feat(std::max<int64_t>(p, 1));
+  std::vector<uint16_t> grp(std::max<int64_t>(p, 1));
+  {
+    std::vector<int64_t> pos(off.begin(), off.end() - 1);
+    for (int64_t i = 0; i < p; ++i) { feat[pos[attr_group[i]]++] = (uint32_t)i; grp[i] = (uint16_t)attr_group[i]; }   // stable
+  }
+  gp.chunk_beg.clear(); gp.chunk_grp.clear();
+  for (int g = 0; g < G; ++g)
+    for (int64_t c = off[g]; c < off[g + 1]; c += GRP_CHUNK) { gp.chunk_beg.push_back((uint32_t)c); gp.chunk_grp.push_back(g); }
+  gp.chunk_beg.push_back((uint32_t)p);
+  const size_t nch = gp.chunk_grp.size();
+  gp.grp.alloc(grp.size()); gp.feat.alloc(feat.size()); gp.chunk_beg_dev.alloc(nch + 1); gp.chunk_grp_dev.alloc(std::max<size_t>(nch, 1));
+  gp.mu.alloc((size_t)G * std::max(k, 1)); gp.part.alloc(std::max<size_t>(nch, 1) * 2 * std::max(k, 1));
+  gp.prior.alloc((size_t)(1 + k) * G);
+  gp.prior_host.assign(2 * (size_t)(1 + k) * G, 0.0);
+  FMWR_CUDA(cudaMemcpyAsync(gp.grp.p, grp.data(), 2 * grp.size(), cudaMemcpyHostToDevice, ctx->stream));
+  FMWR_CUDA(cudaMemcpyAsync(gp.feat.p, feat.data(), 4 * feat.size(), cudaMemcpyHostToDevice, ctx->stream));
+  FMWR_CUDA(cudaMemcpyAsync(gp.chunk_beg_dev.p, gp.chunk_beg.data(), 4 * (nch + 1), cudaMemcpyHostToDevice, ctx->stream));
+  if (nch) FMWR_CUDA(cudaMemcpyAsync(gp.chunk_grp_dev.p, gp.chunk_grp.data(), 4 * nch, cudaMemcpyHostToDevice, ctx->stream));
+  FMWR_CUDA(cudaStreamSynchronize(ctx->stream));      // the host vectors above live on this stack frame
+}
+
+// sum[f][g] = sum_{i in I_g} x_if, sq[f][g] = sum_{i in I_g} (x_if - mu[f][g])^2, and (row != nullptr) row[f][g] = x_gf
+template <class T>
+static void group_sums(fmwr_ctx* ctx, GroupPrior& gp, const T* x, int64_t ld, int kc, const std::vector<double>& mu,
+                       std::vector<double>& sum, std::vector<double>& sq, std::vector<double>* row)
+{
+  const int G = gp.G;
+  const size_t nch = gp.chunk_grp.size();
+  sum.assign((size_t)kc * G, 0.0); sq.assign((size_t)kc * G, 0.0);
+  std::vector<double> h(nch * 2 * kc);
+  std::vector<T> r(row ? (size_t)G * ld : 0);
+  FMWR_CUDA(cudaMemcpyAsync(gp.mu.p, mu.data(), 8 * (size_t)kc * G, cudaMemcpyHostToDevice, ctx->stream));
+  if (nch) {
+    FMWR_LAUNCH(ctx, grouped_reduce_kernel<T>, (int)nch, 256, 0, x, ld, kc, G, gp.feat.p, gp.chunk_beg_dev.p, gp.chunk_grp_dev.p, gp.mu.p,
+                gp.part.p);
+    FMWR_CUDA(cudaMemcpyAsync(h.data(), gp.part.p, 8 * h.size(), cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  if (row) FMWR_CUDA(cudaMemcpyAsync(r.data(), x, sizeof(T) * r.size(), cudaMemcpyDeviceToHost, ctx->stream));
+  FMWR_CUDA(cudaStreamSynchronize(ctx->stream));
+  for (size_t b = 0; b < nch; ++b) {
+    const int g = gp.chunk_grp[b];
+    for (int f = 0; f < kc; ++f) { sum[(size_t)f * G + g] += h[b * 2 * kc + f]; sq[(size_t)f * G + g] += h[b * 2 * kc + kc + f]; }
+  }
+  if (row) {
+    row->assign((size_t)kc * G, 0.0);
+    for (int g = 0; g < G; ++g)
+      for (int f = 0; f < kc; ++f) (*row)[(size_t)f * G + g] = (double)r[(size_t)g * ld + f];
+  }
+}
+
+// out[f] = v[f] added `count` times in fp64, f < k (F7: the reference's v(f, attr_group[i]) reading of update_v_mu).  The
+// chains of 16 factors run side by side in registers: a factor-at-a-time loop, or one that keeps out[] in memory, leaves the
+// GPU idle for milliseconds per sweep on the configs[3] shape.
+static void repeated_sum(const double* v, int64_t count, int k, double* out)
+{
+  constexpr int B = 16;
+  for (int f0 = 0; f0 < k; f0 += B) {
+    const int nb = std::min(B, k - f0);
+    double x[B] = {}, acc[B] = {};
+    for (int j = 0; j < nb; ++j) x[j] = v[f0 + j];
+    for (int64_t i = 0; i < count; ++i)
+#pragma unroll
+      for (int j = 0; j < B; ++j) acc[j] += x[j];
+    for (int j = 0; j < nb; ++j) out[f0 + j] = acc[j];
+  }
+}
+
 template <class T>
 static double reduce(fmwr_ctx* ctx, const T* x, int64_t n, int64_t stride, int mode, double c)
 {
@@ -347,6 +475,7 @@ struct CoordArgs {
   int do_sample; int w_sd_is_var;    // F7: w drawn with the variance as s.d.
   const double* normals; long long n_normals; long long normal_base;   // draw for column c: normals[normal_base + c]
   uint64_t seed;
+  const uint16_t* grp; const double2* gprior;   // attribute groups: (lambda, mu) = gprior[grp[c]] (grp == nullptr: lambda, mu)
 };
 
 template <class T>
@@ -380,8 +509,10 @@ __device__ __forceinline__ void coord_update(const CoordArgs<T>& a, uint32_t c, 
   A = reduce(A);
   Bm = reduce(Bm);
   if (a.q != nullptr) Bm -= old * A;                                   // :322
-  const double var = 1.0 / (a.lambda + a.alpha * A);
-  const double mean = -var * (a.alpha * Bm - a.mu * a.lambda);
+  double lambda = a.lambda, mu = a.mu;
+  if (a.grp) { const double2 lm = a.gprior[a.grp[c]]; lambda = lm.x; mu = lm.y; }
+  const double var = 1.0 / (lambda + a.alpha * A);
+  const double mean = -var * (a.alpha * Bm - mu * lambda);
   double nv;
   bool upd = true;
   if (dev_bad(var)) nv = 0.0;                                           // :235-236, :326-327
@@ -523,6 +654,7 @@ struct RmArgs {
   double alpha, lambda, mu;
   int do_sample, w_sd_is_var;
   const double* normals; long long n_normals, normal_base; uint64_t seed;
+  const uint16_t* grp; const double2* gprior;   // attribute groups: (lambda, mu) = gprior[grp[cb + c]] (grp == nullptr: lambda, mu)
 };
 
 template <class T> __device__ __forceinline__ void rm_extract_one(const RmArgs<T>& a, uint32_t c);
@@ -673,8 +805,10 @@ __device__ __forceinline__ void rm_solve_finish(const RmArgs<T>& a, uint32_t c, 
 {
   const double old = (double)a.th[c];
   if (a.q != nullptr) Bm -= old * A;                                    // reference :322
-  const double var = 1.0 / (a.lambda + a.alpha * A);
-  const double mean = -var * (a.alpha * Bm - a.mu * a.lambda);
+  double lambda = a.lambda, mu = a.mu;
+  if (a.grp) { const double2 lm = a.gprior[a.grp[a.cb + c]]; lambda = lm.x; mu = lm.y; }
+  const double var = 1.0 / (lambda + a.alpha * A);
+  const double mean = -var * (a.alpha * Bm - mu * lambda);
   double nv;
   bool upd = true;
   if (isnan(var) || isinf(var)) nv = 0.0;
@@ -1127,7 +1261,8 @@ static double allreduce_scalar(fmwr_ctx* ctx, double x)
 
 // one coordinate step of a fused sequence
 template <class T>
-struct Step { int phase; T* q; int f; T* theta; int64_t stride; double lambda, mu; int w_sd_is_var; long long normal_base; };
+struct Step { int phase; T* q; int f; T* theta; int64_t stride; double lambda, mu; int w_sd_is_var; long long normal_base;
+              const uint16_t* grp; const double2* gprior; };
 
 template <class T>
 static void run_steps_dense(fmwr_ctx* ctx, const std::vector<uint32_t>& pbeg, const RowMajor& rm, const DenseLayout& dl, int64_t n,
@@ -1159,6 +1294,7 @@ static void run_steps_dense(fmwr_ctx* ctx, const std::vector<uint32_t>& pbeg, co
     ra.n_rep = fused_replicas<T>(ncols, grid);
     ra.alpha = alpha; ra.lambda = cs.lambda; ra.mu = cs.mu; ra.do_sample = do_sample; ra.w_sd_is_var = cs.w_sd_is_var;
     ra.normals = normals; ra.n_normals = n_normals; ra.normal_base = cs.normal_base; ra.seed = seed;
+    ra.grp = cs.grp; ra.gprior = cs.gprior;
     return ra;
   };
   RmArgs<T> ra, rnext;
@@ -1398,6 +1534,18 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
   const double alpha_0 = 1.0, gamma_0 = 1.0, beta_0 = 1.0, mu_0 = 0.0, w0_mean_0 = 0.0;
   double alpha = 1.0, w_mu = 0.0, w_lambda = 0.0;
   std::vector<double> v_mu(std::max(k, 1), 0.0), v_lambda(std::max(k, 1), 0.0);
+  // attribute groups (the one-group sampler above is untouched when there are none): per-group hyper-priors, [G] for w and
+  // [k][G] for V, and their device table read by the coordinate steps through the feature's group
+  const bool grouped = s->attr_group && s->n_groups > 1;
+  const int G = grouped ? s->n_groups : 0;
+  GroupPrior gp;
+  std::vector<double> gw_lambda(G, 0.0), gw_mu(G, 0.0), gv_lambda((size_t)k * G, 0.0), gv_mu((size_t)k * G, 0.0);
+  if (grouped) group_prior_build(ctx, s->attr_group, p, G, k, gp);
+  auto upload_prior = [&](int row0, int rows, const std::vector<double>& lam, const std::vector<double>& mu) {
+    double* hp = gp.prior_host.data() + 2 * (size_t)row0 * G;
+    for (size_t i = 0; i < (size_t)rows * G; ++i) { hp[2 * i] = lam[i]; hp[2 * i + 1] = mu[i]; }
+    FMWR_CUDA(cudaMemcpyAsync(gp.prior.p + (size_t)row0 * G, hp, 16 * (size_t)rows * G, cudaMemcpyHostToDevice, ctx->stream));
+  };
 
   // posterior mean: f64 sums of the predict.FM prediction of every averaged draw (the MCMC link of tracker_score) -- the
   // training rows in the order e has, then each eval set.  Draw t is the model after t sweeps: at sweep t, right after the
@@ -1470,7 +1618,22 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
     }
     if (m->cfg.keep_w1) {
       // update_w_lambda (:415-445), update_w_mu (:383-412)
-      if (do_multilevel) {
+      if (grouped) {
+        // lambda_w[0..G-1], then mu_w[0..G-1], each over the group's features (fmwr_solver_cfg::attr_group)
+        std::vector<double> sum, sq;
+        group_sums<T>(ctx, gp, wp, 1, 1, gw_mu, sum, sq, nullptr);
+        for (int g = 0; g < G; ++g) {
+          const double gg = sq[g] + (beta_0 * (gw_mu[g] - mu_0) * (gw_mu[g] - mu_0) + gamma_0);
+          const double nl = hs.gamma((alpha_0 + (double)gp.count[g] + 1) / 2.0, 2.0 / gg);
+          if (!hbad(nl)) gw_lambda[g] = nl;
+        }
+        for (int g = 0; g < G; ++g) {
+          const double pg = (double)gp.count[g];
+          const double nm = hs.normal((sum[g] + beta_0 * mu_0) / (pg + beta_0), std::sqrt(1.0 / ((pg + beta_0) * gw_lambda[g])));
+          if (!hbad(nm)) gw_mu[g] = nm;
+        }
+        upload_prior(0, 1, gw_lambda, gw_mu);
+      } else if (do_multilevel) {
         double g = reduce<T>(ctx, wp, p, 1, 2, w_mu);
         g += beta_0 * (w_mu - mu_0) * (w_mu - mu_0) + gamma_0;
         const double la = alpha_0 + (double)p + 1;
@@ -1490,18 +1653,49 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
       a.alpha = alpha; a.lambda = w_lambda; a.mu = w_mu; a.do_sample = do_sample;
       a.w_sd_is_var = (s->compat & FMWR_COMPAT_MCMC_W_SD) ? 1 : 0;
       a.normals = injected ? normals_dev.p : nullptr; a.n_normals = s->n_normals; a.normal_base = hs.i_normal; a.seed = s->seed;
+      a.grp = grouped ? gp.grp.p : nullptr; a.gprior = grouped ? gp.prior.p : nullptr;
       if (use_rm && dl.ok) {
         std::vector<Step<T>> steps;
-        for (int j = 0; j < n_phases; ++j) steps.push_back({j, nullptr, 0, wp, 1, w_lambda, w_mu, a.w_sd_is_var, a.normal_base});
+        for (int j = 0; j < n_phases; ++j) steps.push_back({j, nullptr, 0, wp, 1, w_lambda, w_mu, a.w_sd_is_var, a.normal_base, a.grp, a.gprior});
         run_steps_dense<T>(ctx, ph.begin, rm, dl, n, e.p, steps, scr, alpha, do_sample, a.normals, a.n_normals, a.seed);
-      } else if (use_rm) run_phases_rm<T>(ctx, ph.begin, rm, rm_args(e.p, nullptr, 0, wp, 1, alpha, w_lambda, w_mu, do_sample, a.w_sd_is_var,
-                                                               a.normals, a.n_normals, a.normal_base, a.seed));
-      else run_phases<T>(ctx, ph, a);
+      } else if (use_rm) {
+        RmArgs<T> ra = rm_args(e.p, nullptr, 0, wp, 1, alpha, w_lambda, w_mu, do_sample, a.w_sd_is_var, a.normals, a.n_normals, a.normal_base, a.seed);
+        ra.grp = a.grp; ra.gprior = a.gprior;
+        run_phases_rm<T>(ctx, ph.begin, rm, ra);
+      } else run_phases<T>(ctx, ph, a);
       if (do_sample) hs.i_normal += p;
     }
     if (enable_v) {
       // update_v_lambda (:486-517) for every factor, then update_v_mu (:448-483), then update_v (:272-354)
-      if (do_multilevel) {
+      if (grouped) {
+        // lambda_v[f][g] for f = 0..k-1 with g inside, then mu_v in the same order (fmwr_solver_cfg::attr_group)
+        std::vector<double> sum, sq, row;
+        group_sums<T>(ctx, gp, vp, kp, k, gv_mu, sum, sq, &row);
+        for (int f = 0; f < k; ++f)
+          for (int g = 0; g < G; ++g) {
+            const size_t i = (size_t)f * G + g;
+            const double gg = sq[i] + (beta_0 * (gv_mu[i] - mu_0) * (gv_mu[i] - mu_0) + gamma_0);
+            const double nl = hs.gamma((alpha_0 + (double)gp.count[g] + 1) / 2.0, 2.0 / gg);
+            if (!hbad(nl)) gv_lambda[i] = nl;
+          }
+        // F7: v(f, attr_group[i]) read for every i of group g is v_gf, added p_g times in fp64 as the one-group sampler does
+        if (s->compat & FMWR_COMPAT_MCMC_VMU_IDX) {
+          std::vector<double> vg(k), acc(k);
+          for (int g = 0; g < G; ++g) {
+            for (int f = 0; f < k; ++f) vg[f] = row[(size_t)f * G + g];
+            repeated_sum(vg.data(), gp.count[g], k, acc.data());
+            for (int f = 0; f < k; ++f) sum[(size_t)f * G + g] = acc[f];
+          }
+        }
+        for (int f = 0; f < k; ++f)
+          for (int g = 0; g < G; ++g) {
+            const size_t i = (size_t)f * G + g;
+            const double pg = (double)gp.count[g];
+            const double nm = hs.normal((sum[i] + beta_0 * mu_0) / (pg + beta_0), std::sqrt(1.0 / ((pg + beta_0) * gv_lambda[i])));
+            if (!hbad(nm)) gv_mu[i] = nm;
+          }
+        upload_prior(1, k, gv_lambda, gv_mu);
+      } else if (do_multilevel) {
         // V is not touched between these 2k draws and v_lambda[f] / v_mu[f] only depend on factor f's own sums, so all
         // the sums come from one batched reduction (the draw ORDER -- k lambdas, then k mus -- is the reference's)
         std::vector<double> vsum, vsq, vrow0;
@@ -1514,14 +1708,12 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
           if (!hbad(nl)) v_lambda[f] = nl;
         }
         // F7: the reference sums v(f, attr_group[i]) == v(f, 0), p times (:462).  The p-fold fp64 addition is reproduced
-        // exactly, but for all factors at once (k independent chains the CPU can pipeline) -- one factor at a time it
-        // was 3 ms of host time per sweep with the GPU idle.
+        // exactly (repeated_sum).
         std::vector<double> vrep(k, 0.0);
         if (s->compat & FMWR_COMPAT_MCMC_VMU_IDX) {
           std::vector<double> v0(k);
           for (int f = 0; f < k; ++f) v0[f] = (double)T(vrow0[f]);
-          for (int64_t i = 0; i < p; ++i)
-            for (int f = 0; f < k; ++f) vrep[f] += v0[f];
+          repeated_sum(v0.data(), p, k, vrep.data());
         }
         for (int f = 0; f < k; ++f) {
           double mm = (s->compat & FMWR_COMPAT_MCMC_VMU_IDX) ? vrep[f] : vsum[f];
@@ -1531,10 +1723,12 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
           if (!hbad(nm)) v_mu[f] = nm;
         }
       } else { for (int f = 0; f < k; ++f) v_mu[f] = mu_0; }
+      const uint16_t* vgrp = grouped ? gp.grp.p : nullptr;
+      auto vprior = [&](int f) { return grouped ? gp.prior.p + (size_t)(1 + f) * G : nullptr; };
       if (use_rm && dl.ok) {
         std::vector<Step<T>> steps;
         for (int f = 0; f < k; ++f) {
-          for (int j = 0; j < n_phases; ++j) steps.push_back({j, q.p, f, vp + f, (int64_t)kp, v_lambda[f], v_mu[f], 0, hs.i_normal});
+          for (int j = 0; j < n_phases; ++j) steps.push_back({j, q.p, f, vp + f, (int64_t)kp, v_lambda[f], v_mu[f], 0, hs.i_normal, vgrp, vprior(f)});
           if (do_sample) hs.i_normal += p;
         }
         run_steps_dense<T>(ctx, ph.begin, rm, dl, n, e.p, steps, scr, alpha, do_sample, injected ? normals_dev.p : nullptr, s->n_normals, s->seed);
@@ -1546,9 +1740,12 @@ static void train_als_t(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_s
         a.e = e.p; a.q = q.p; a.kp = kp; a.f = f; a.n = n; a.theta = vp + f; a.theta_stride = kp;
         a.alpha = alpha; a.lambda = v_lambda[f]; a.mu = v_mu[f]; a.do_sample = do_sample; a.w_sd_is_var = 0;
         a.normals = injected ? normals_dev.p : nullptr; a.n_normals = s->n_normals; a.normal_base = hs.i_normal; a.seed = s->seed;
-        if (use_rm) run_phases_rm<T>(ctx, ph.begin, rm, rm_args(e.p, q.p, f, vp + f, kp, alpha, v_lambda[f], v_mu[f], do_sample, 0,
-                                                                 a.normals, a.n_normals, a.normal_base, a.seed));
-        else run_phases<T>(ctx, ph, a);
+        a.grp = vgrp; a.gprior = vprior(f);
+        if (use_rm) {
+          RmArgs<T> ra = rm_args(e.p, q.p, f, vp + f, kp, alpha, v_lambda[f], v_mu[f], do_sample, 0, a.normals, a.n_normals, a.normal_base, a.seed);
+          ra.grp = a.grp; ra.gprior = a.gprior;
+          run_phases_rm<T>(ctx, ph.begin, rm, ra);
+        } else run_phases<T>(ctx, ph, a);
         if (do_sample) hs.i_normal += p;
       }
     }

@@ -91,6 +91,23 @@ typedef struct {
    * cumulative-L1 q and totals) instead of restarting it at zero.  The reference's fm.update drops the state
    * (FTRL_Learner.h:48-56, SURVEY 8f-4); 0 reproduces that. */
   int32_t warm_state;
+  /* MCMC attribute groups (libFM's feature grouping, its --meta file; extension: the reference hard-wires one group,
+   * src/FM.cpp:75).  attr_group[i] in [0, n_groups) is the group of feature i (host pointer to [p] entries, not retained);
+   * NULL means one group and n_groups must then be 0 or 1, so zero-initialised callers see no change.  Every group g has its
+   * own hyper-prior, drawn each sweep over the features I_g of the group (p_g = |I_g|, empty groups allowed; constants as F2):
+   *   lambda_w[g] ~ Gamma((alpha_0 + p_g + 1) / 2, scale 2 / (S2_g + beta_0 (mu_w[g] - mu_0)^2 + gamma_0))
+   *   mu_w[g]     ~ N((S1_g + beta_0 mu_0) / (p_g + beta_0), variance 1 / ((p_g + beta_0) lambda_w[g]))
+   * with S1_g the sum of w_i over i in I_g and S2_g the sum of (w_i - mu_w[g])^2 over i in I_g (ascending i),
+   * and lambda_v[g][f], mu_v[g][f] by the same formulas over the v_if of the group.  The coordinate step of w_i / v_if uses
+   * the lambda and mu of group attr_group[i]; nothing else of it changes.  Under FMWR_COMPAT_MCMC_VMU_IDX the sum in mu_v[g][f]
+   * is p_g times v_gf (the reference's v(f, attr_group[i]) reading), otherwise the sum of v_if over i in I_g.  Draw order of a sweep:
+   * the truncated normals, alpha, w0, lambda_w[0..G-1], mu_w[0..G-1], the p w-draws, lambda_v for f = 0..k-1 with g = 0..G-1
+   * inside each f, mu_v in the same order, the k p v-draws.  A NaN / Inf draw keeps that group's previous value; every group
+   * starts at lambda = mu = 0.  A map with n_groups = 1 runs the one-group sampler (bit-identical results).  Training fails
+   * with FMWR_ERR_ARG, before the model is touched, when an entry is outside [0, n_groups), when n_groups < 1, > 65536 or
+   * > p, when n_groups > 1 comes without a map, or when a map is given to a solver other than MCMC. */
+  const int32_t* attr_group;
+  int32_t n_groups;
 } fmwr_solver_cfg;
 
 /* train-metric trace (Tracker::save, src/core/Tracker.h:96-119) -- caller allocates */

@@ -198,6 +198,15 @@ List FM(List data_, IntegerVector normalize, List fm_controls, List solver_contr
   sc.metric = metric_id(as<std::string>(track_controls["evaluate.metric"]));
   sc.convergence = (double)track_controls["convergence"];
   sc.seed = (uint64_t)(R::unif_rand() * 4294967296.0);               // native MCMC RNG keyed off R's stream
+  // MCMC attribute groups (libFM's feature grouping): x$features$attr_group <- g, 0-based, one entry per column
+  IntegerVector attr_group;
+  if (sc.solver == FMWR_MCMC && X.containsElementNamed("attr_group") && !Rf_isNull(X["attr_group"])) {
+    attr_group = as<IntegerVector>(X["attr_group"]);
+    if (attr_group.size() != p) Rcpp::stop("attr_group must be an integer vector with one entry per column");
+    int mx = 0;
+    for (int i = 0; i < attr_group.size(); ++i) mx = std::max(mx, (int)attr_group[i]);
+    sc.attr_group = attr_group.begin(); sc.n_groups = mx + 1;            // range checks: fmwr_train_dev (FMWR_ERR_ARG)
+  }
 
   fmwr_trace tr; memset(&tr, 0, sizeof tr);
   std::vector<double> ev, sw0, sw, sv; std::vector<int> ri;
