@@ -426,6 +426,18 @@ def train_posterior_dev(ctx, model, data, scfg, burn_in, evals=(), trace=None, k
     del keep
 
 
+def train_sgda_dev(ctx, model, data, scfg, valid, lambda_w, lambda_v, trace=None, keep=()):
+    """SGDA (fmwr_train_sgda_dev): SGD in exact mode that learns per-group L2 rates on the labelled Data handle `valid`
+    (None passes a null handle).  lambda_w [G] and lambda_v [G, k] are C-contiguous float64 arrays updated in place
+    (None passes a null pointer)."""
+    for a in (lambda_w, lambda_v):
+        if a is not None and (a.dtype != np.float64 or not a.flags["C_CONTIGUOUS"]):
+            raise TypeError("lambda_w / lambda_v must be C-contiguous float64 arrays")
+    check(lib().fmwr_train_sgda_dev(ctx.h, model.h, data.h, C.byref(scfg), C.byref(trace.c) if trace is not None else None,
+                                    valid.h if valid is not None else None, ptr(lambda_w), ptr(lambda_v)))
+    del keep
+
+
 def train_holdout_dev(ctx, model, data, scfg, trace, evals, select_best=0, patience=0, keep=()):
     """train_dev plus held-out tracking: every eval set (labelled Data handles; an entry of None passes a null handle) is
     scored at every tracker record.  Returns (scores [n_eval][n_rec stored], best_rec)."""

@@ -284,10 +284,12 @@ def _model_cfg(mc):
                       l2_v=float(hp["L2.v"]))
 
 
-def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_list, streams=None, posterior=None, holdout=None):
+def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_list, streams=None, posterior=None, holdout=None,
+        sgda=None):
     """body of FM() (reference src/FM.cpp:7-174) on top of the C ABI.  posterior (fm_posterior): dict(burn_in, newdata) in, and
     the device means out as posterior["train"] and posterior["newdata_mean"].  holdout (fm_train_holdout): dict(newdata, labels,
-    select_best, patience, snapshots) in; the trace gains "evaluation.test" and "best.index"."""
+    select_best, patience, snapshots) in; the trace gains "evaluation.test" and "best.index".  sgda (fm_train_sgda): dict(newdata,
+    labels) in; Model gains "reg", the learned L2 rates."""
     ctx = _ctx()
     feats = data["features"]
     n, p = feats["dim"]
@@ -336,7 +338,8 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
                              metric=L.METRICS[track_controls["evaluate.metric"]], convergence=float(track_controls["convergence"]),
                              seed=int(_OPTIONS["FM.seed"]), warm_state=warm)
             keep = []
-            if name == "MCMC" and feats.get("attr_group") is not None:
+            n_groups = 1
+            if (name == "MCMC" or sgda is not None) and feats.get("attr_group") is not None:
                 grp, n_groups = _attr_group(feats["attr_group"], p)
                 keep.append(grp)
                 sc.attr_group = L.ptr(grp); sc.n_groups = n_groups
@@ -351,7 +354,14 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
                 from math import ceil
                 nrec = min(10001, int(ceil((sc.max_iter - 0.5) / sc.step_size)) + 2)
                 trace = L.TraceBuf(nrec, p, k, snapshots=holdout is None or holdout["snapshots"])
-            if holdout is not None:
+            if sgda is not None:                                          # z-scored with the training scales as fm_track does
+                evals.append(_acquire(ctx, sgda["newdata"]["features"], sgda["labels"], normalize0[0] > -1))
+                if normalize0[0] > -1:
+                    evals[-1][0].normalize(scales["mean"], scales["std"])
+                lam_w = np.full(n_groups, float(hp["L2.w1"]))
+                lam_v = np.full((n_groups, k), float(hp["L2.v"]))
+                L.train_sgda_dev(ctx, m, d, sc, evals[-1][0], lam_w, lam_v, trace, keep=keep)
+            elif holdout is not None:
                 for nd, nd_labels in zip(holdout["newdata"], holdout["labels"]):   # z-scored with the training scales as fm.track does
                     evals.append(_acquire(ctx, nd["features"], nd_labels, normalize0[0] > -1))
                     if normalize0[0] > -1:
@@ -369,7 +379,7 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
                 posterior["train"] = L.predict_fetch(ctx, d)
                 posterior["newdata_mean"] = [L.predict_fetch(ctx, e) for e, _ in evals]
             gw0, gw, gv = m.get()
-            state = m.get_state() if (_OPTIONS["FM.keep_state"] and name in ("SGD", "FTRL", "TDAP")) else None
+            state = m.get_state() if (_OPTIONS["FM.keep_state"] and name in ("SGD", "FTRL", "TDAP") and sgda is None) else None
         finally:
             m.close()
     finally:
@@ -379,6 +389,8 @@ def _FM(data, normalize0, fm_controls, solver_controls, track_controls, model_li
             if not e_parked:
                 e.close()
     model = dict(w0=gw0, w=gw, v=gv.T.copy())                              # v returned k x p like Model::save_model
+    if sgda is not None:
+        model["reg"] = dict(w=lam_w, v=lam_v.T.copy())                   # v: k x n_groups like the model's v
     model["model.control"] = fm_controls
     model["solver.control"] = solver_controls
     model["track.control"] = track_controls
@@ -510,6 +522,35 @@ def fm_train_holdout(data, newdata, normalize=True, control=None, select="last",
         labels.append(y)
     ho = dict(newdata=newdata, labels=labels, select_best=int(select == "best"), patience=int(patience), snapshots=bool(snapshots))
     return _FM(data, norm - 1, ctl["model"], ctl["solver"], ctl["track"], None, holdout=ho)
+
+
+def fm_train_sgda(data, validation, normalize=True, control=None):
+    """Engine extension: libFM's adaptive-regularization SGD (SGDA).  Trains as fm_train(data, normalize, control) with
+    SGD_solver() in exact mode (FM.mode = "exact") and, from the second pass over the training rows on, takes after every training
+    step a gradient step on the L2 rates themselves, on one row of `validation` (a labelled fm.matrix of the same width, labels
+    0/1 recoded and values z-scored with the training scales as fm_track does).  One rate per attribute group
+    (data$features$attr_group; none: one group) for w and one per group and factor for V, starting from L2.w1 / L2.v of
+    model.control; L1 must be 0.  The rules are those of fmwr_train_sgda_dev (include/fmwr_b200.h).  Returns the usual FM object
+    with Model$reg = dict(w=<rate per group>, v=<k x groups rates>)."""
+    if not isinstance(validation, FmMatrix):
+        raise ValueError("validation must be a fm.matrix object")
+    data, norm, ctl = _train_setup(data, normalize, control)
+    if ctl["solver"]["solver"].solver != "SGD":
+        raise ValueError("SGDA needs the SGD solver (SGD_solver())")
+    if _OPTIONS["FM.mode"] != "exact":
+        raise ValueError("SGDA runs in exact mode only (FM.mode = \"exact\")")
+    hp = ctl["model"]["hyper.params"]
+    if hp["L1.w1"] > 0 or hp["L1.v"] > 0:
+        raise ValueError("SGDA adapts L2 rates only: L1.w1 and L1.v must be 0")
+    _check_newdata([validation], data, need_labels=True)
+    if validation.ncol() != data.ncol():
+        raise ValueError("validation must have as many columns as data")
+    if data["features"].get("attr_group") is not None:
+        _attr_group(data["features"]["attr_group"], data.ncol())
+    y = np.asarray(validation["labels"], np.float64)
+    if ctl["model"]["task"] == "CLASSIFICATION" and np.array_equal(np.unique(y), [0, 1]):
+        y = np.where(y < 1, -1.0, 1.0)
+    return _FM(data, norm - 1, ctl["model"], ctl["solver"], ctl["track"], None, sgda=dict(newdata=validation, labels=y))
 
 
 def _require_snapshots(obj):

@@ -296,14 +296,14 @@ static void check_eval_list(const fmwr_model* m, const fmwr_data* d, fmwr_data* 
   for (int i = 0; i < n_eval; ++i) require_same_features(m, eval[i]);
 }
 
-// attribute groups of fmwr_solver_cfg (MCMC only; NULL map: one group)
-static void check_groups(const fmwr_model* m, const fmwr_solver_cfg* s)
+// attribute groups of fmwr_solver_cfg (MCMC, and SGD through fmwr_train_sgda_dev; NULL map: one group)
+static void check_groups(const fmwr_model* m, const fmwr_solver_cfg* s, bool grouped_solver)
 {
   if (!s->attr_group) {
     FMWR_REQUIRE(s->n_groups >= 0 && s->n_groups <= 1, FMWR_ERR_ARG, "n_groups > 1 needs an attr_group map");
     return;
   }
-  FMWR_REQUIRE(s->solver == FMWR_MCMC, FMWR_ERR_ARG, "attribute groups need the MCMC solver");
+  FMWR_REQUIRE(grouped_solver, FMWR_ERR_ARG, "attribute groups need the MCMC solver");
   FMWR_REQUIRE(s->n_groups >= 1 && s->n_groups <= 65536 && s->n_groups <= m->p, FMWR_ERR_ARG,
                "n_groups must be at least 1 and at most 65536 and the number of features");
   for (int64_t i = 0; i < m->p; ++i)
@@ -315,7 +315,7 @@ static void train_dispatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmw
 {
   FMWR_REQUIRE(d->has_labels, FMWR_ERR_ARG, "target's length is not equal the number of cases...");
   FMWR_REQUIRE(d->p == m->p, FMWR_ERR_SHAPE, "there's no the same number of features between train and fm object...");
-  check_groups(m, s);
+  check_groups(m, s, s->solver == FMWR_MCMC);
   if (tr) { tr->n_rec = 0; tr->convergent = 0; tr->iters_done = 0; }
   switch (s->solver) {
     case FMWR_SGD: case FMWR_FTRL: case FMWR_TDAP:
@@ -851,6 +851,35 @@ int fmwr_train_holdout_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmw
     const Holdout ho{eval, n_eval, eval_scores, trace->max_rec, select_best != 0, patience, &best};
     train_dispatch(ctx, m, d, s, trace, nullptr, &ho);
     if (best_rec) *best_rec = best;
+  });
+}
+
+int fmwr_train_sgda_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* trace,
+                        fmwr_data* valid, double* lambda_w, double* lambda_v)
+{
+  return guarded([&] {
+    FMWR_REQUIRE(ctx && m && d && s, FMWR_ERR_ARG, "null argument");
+    FMWR_REQUIRE(s->solver == FMWR_SGD, FMWR_ERR_ARG, "SGDA needs the SGD solver");
+    FMWR_REQUIRE(s->mode == FMWR_MODE_EXACT, FMWR_ERR_ARG, "SGDA runs in exact mode only");
+    FMWR_REQUIRE(!s->warm_state, FMWR_ERR_ARG, "SGDA starts from zero gradients: warm_state must be 0");
+    FMWR_REQUIRE(!(m->cfg.l1_w1 > 0 || m->cfg.l1_v > 0), FMWR_ERR_ARG, "SGDA adapts L2 rates only: L1.w1 and L1.v must be 0");
+    FMWR_REQUIRE(d->has_labels, FMWR_ERR_ARG, "target's length is not equal the number of cases...");
+    FMWR_REQUIRE(valid, FMWR_ERR_ARG, "null validation data");
+    FMWR_REQUIRE(valid != d, FMWR_ERR_ARG, "the validation data is the training data");
+    FMWR_REQUIRE(valid->has_labels, FMWR_ERR_ARG, "the validation data has no labels");
+    FMWR_REQUIRE(valid->n > 0, FMWR_ERR_ARG, "the validation data has no rows");
+    FMWR_REQUIRE(lambda_w && (lambda_v || m->k == 0), FMWR_ERR_ARG, "null lambda_w / lambda_v");
+    check_groups(m, s, true);
+    const int G = s->attr_group ? s->n_groups : 1;
+    for (int g = 0; g < G; ++g) FMWR_REQUIRE(std::isfinite(lambda_w[g]) && lambda_w[g] >= 0, FMWR_ERR_ARG, "lambda_w entries must be finite and >= 0");
+    for (int64_t i = 0; i < (int64_t)G * m->k; ++i)
+      FMWR_REQUIRE(std::isfinite(lambda_v[i]) && lambda_v[i] >= 0, FMWR_ERR_ARG, "lambda_v entries must be finite and >= 0");
+    FMWR_REQUIRE(d->p == m->p, FMWR_ERR_SHAPE, "there's no the same number of features between train and fm object...");
+    require_same_features(m, valid);
+    FMWR_REQUIRE(!(ctx->nccl_comm && ctx->world > 1), FMWR_ERR_UNSUPPORTED, "SGDA runs on one GPU (sharded models are not supported)");
+    FMWR_CUDA(cudaSetDevice(ctx->device));
+    if (trace) { trace->n_rec = 0; trace->convergent = 0; trace->iters_done = 0; }
+    train_sgda(ctx, m, d, s, trace, valid, lambda_w, lambda_v);
   });
 }
 

@@ -465,6 +465,10 @@ struct Tracker {
 };
 void train_exact(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* holdout = nullptr);
 void train_minibatch(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, const Holdout* holdout = nullptr);
+// SGDA (fmwr_train_sgda_dev, validated by the caller): SGD in exact mode that learns per-group L2 rates on `valid`; lambda_w [G] and
+// lambda_v [G][k] in/out
+void train_sgda(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* tr, fmwr_data* valid,
+                double* lambda_w, double* lambda_v);
 // MCMC posterior mean (fmwr_train_posterior_dev): average the predict.FM prediction of draws burn_in+1 .. max_iter on the
 // training rows and on every eval set (validated by the caller: distinct, not the training data, same feature count)
 struct Posterior {

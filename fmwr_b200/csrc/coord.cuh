@@ -84,6 +84,20 @@ __device__ __forceinline__ T sgd_step(T theta, T g, T lr, T reg, int l1, T u, T&
   return theta;
 }
 
+// SGDA (adaptive regularization, Rendle WSDM 2012; include/fmwr_b200.h, fmwr_train_sgda_dev).  The step with a learned L2 rate
+// lam, in the simultaneous form theta - lr (g + lam theta): it is linear in lam, so the validation step's look-ahead theta' is this
+// same expression on the current theta and its last gradient, and d theta' / d lam = -lr theta.
+template <class T>
+__device__ __forceinline__ T sgda_step(T theta, T g, T lr, T lam) { return theta - lr * (g + lam * theta); }
+
+// The look-ahead's per-entry term of d p' / d lam_v[g][f] = -lr * sum over the group's entries of x v (S'_f - x v'), the pairwise
+// gradient of p' at v' times d v' / d lam = -lr v  (for lam_w[g] the term is x w)
+template <class T>
+__device__ __forceinline__ T sgda_v_term(T S1, T v, T v1, T x) { return x * v * (S1 - x * v1); }
+
+// lam - lr m' d p' / d lam, clamped at 0; d is the group's sum of the terms above (d p' / d lam = -lr d)
+__device__ __forceinline__ double sgda_lambda_step(double lam, double lr, double mult, double d) { return fmax(0.0, lam + lr * mult * lr * d); }
+
 // Throughput-mode arithmetic: MUFU approximations (sqrt.approx / rcp.approx, <= 2 ulp) instead of the IEEE
 // sequences (~10 instructions each, and each ends a basic block) -- the minibatch update kernel is issue-bound on
 // them and the exact (batch = 1) kernel serialises a vector's elements behind them.  FAST is only ever set for

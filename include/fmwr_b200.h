@@ -285,6 +285,37 @@ int fmwr_train_holdout_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmw
                            fmwr_data* const* eval /* [n_eval] */, int32_t n_eval, double* eval_scores /* [n_eval][trace->max_rec] */,
                            int32_t select_best, int32_t patience, int32_t* best_rec /* nullable */);
 
+/* SGDA: SGD that learns its L2 rates on a validation set while it trains (extension: libFM's adaptive-regularization SGD,
+ * Rendle, "Learning recommender systems with adaptive regularization", WSDM 2012).  One rate per attribute group
+ * (s->attr_group / n_groups as for MCMC; NULL map: one group): lambda_w[G] and lambda_v[G][k], fp64, in/out -- they start from
+ * the caller's values and come back updated.  Notation: lr = s->learn_rate, g(i) the group of feature i, mult(p, y) the
+ * multiplier of SGD (regression: p clamped to [s->min_target, s->max_target]).  The training visit sequence is SGD's (the F5 scan,
+ * an explicit visit_order cycled, or the random_step sweeps) and T0 is the length of its first pass: n - skip_row0 for the scan,
+ * s->n_visit for an explicit order, and the first sweep for random_step > 1 (the sweeps are strictly ascending, so it ends where
+ * the row index first fails to increase; all max_iter samples when max_iter ends inside it).  Sample t of that sequence:
+ *   1. theta step on training row r: the forward, S_f and m = mult(p, y_r) as exact-mode SGD; for every entry (i, x), against
+ *      the pre-step theta:  gw_i = m x,  w_i <- w_i - lr (gw_i + lambda_w[g(i)] w_i)  (keep.w1 only);  for every f
+ *      gv_if = m (S_f x - v_if x^2),  v_if <- v_if - lr (gv_if + lambda_v[g(i)][f] v_if).  w0 takes SGD's step with the fixed
+ *      L2.w0 (its rate is not adapted).  gw / gv of a coordinate persist until the next training row that touches it and are 0
+ *      before the first one in this call.  The simultaneous penalty form (lambda = 2 reg of libFM) keeps the look-ahead linear.
+ *   2. only when t >= T0 (no lambda step in the first pass): lambda step on validation row u = (t - T0) mod n_val (plain order,
+ *      wrapping; F5 does not apply).  Look-ahead with theta after step 1:  w'_i = w_i - lr (gw_i + lambda_w[g(i)] w_i),
+ *      v'_if = v_if - lr (gv_if + lambda_v[g(i)][f] v_if),  S'_f = sum_i v'_if x_i,
+ *      p' = [k0] w0 + [k1] sum_i w'_i x_i + 1/2 sum_f (S'_f^2 - sum_i (v'_if x_i)^2),  m' = mult(p', y_u);  then for every group g
+ *      of the row:  lambda_w[g] <- max(0, lambda_w[g] + lr m' lr sum_{i in g} x_i w_i)  (keep.w1 only),
+ *      lambda_v[g][f] <- max(0, lambda_v[g][f] + lr m' lr (S'_f sum_{i in g} x_i v_if - sum_{i in g} x_i^2 v'_if v_if)),
+ *      i.e. lambda <- max(0, lambda - lr m' dp'/dlambda).  Group sums are taken in row order without atomics (bit-reproducible).
+ * Everything else is exact-mode SGD: the tracker records after samples 0, step, 2 step, ... and max_iter-1 with SGD's link and
+ * metric, snapshots and convergence stop.  The gradients are owned by the call: afterwards the handle holds no optimizer state
+ * (fmwr_model_state_info reports solver 0).  valid: a labelled handle of the same feature count, not d, z-scored by the caller
+ * like any eval set.  Both precisions; s->solver must be FMWR_SGD and s->mode FMWR_MODE_EXACT.  Fails before touching the model
+ * or the lambdas with FMWR_ERR_ARG (another solver or minibatch mode; warm_state = 1; L1.w1 or L1.v > 0; d unlabelled; valid
+ * null, unlabelled, equal to d or without rows; lambda_w null, or lambda_v null with k > 0; a lambda negative or not finite; a
+ * bad group map as for MCMC), FMWR_ERR_SHAPE (valid of another feature count) or FMWR_ERR_UNSUPPORTED (a communicator with
+ * world > 1).  fmwr_train_dev keeps refusing a group map for SGD. */
+int fmwr_train_sgda_dev(fmwr_ctx* ctx, fmwr_model* m, fmwr_data* d, const fmwr_solver_cfg* s, fmwr_trace* trace /* nullable */,
+                        fmwr_data* valid, double* lambda_w /* [n_groups] in/out */, double* lambda_v /* [n_groups][k] in/out */);
+
 /* ---- one-shot host-buffer entry points: what the rewritten src/FM.cpp calls ---- */
 /* FMPredict body (src/FM.cpp:177-214) */
 int fmwr_predict(const fmwr_model_cfg* cfg, int32_t precision, int64_t n, int64_t p, int64_t nnz,
